@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-frame radar perception path (cluster + track + pose) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one radar frame for every resident scene: Utils.normalize_data -> TrackBuffer.track ->
@@ -432,6 +432,39 @@ def other_configs(batches, weights3d, flush, local):
     return out
 
 
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(bt, offsets, out_dir):
+    """Writes what a caller of the timed path holds after its last step as out_dir/<name>.npy: every field of the track
+    records (mmw_get_tracks) and the track counts, the packed result records (mmw_pack_results), the per-scene status
+    flags and the association of every input point of the frame (with the frame's scene offsets).  Integers are stored
+    as float64, which holds them exactly.  Above DUMP_BYTES_MAX in all, a fixed seeded sample of the scenes is written;
+    scene_index lists the scenes written."""
+    import torch
+    from mmwave_msc_b200 import _lib
+    tr, nt = bt.tracks()
+    res = torch.empty(bt.S * bt.tcap * _lib.RESULT_FLOATS, dtype=torch.float32, device="cuda")
+    bt.pack_results(res.data_ptr())
+    bt.sync()
+    out = {"n_tracks": nt, "status": bt.status(), "results": res.cpu().numpy().reshape(bt.S, bt.tcap, -1)}
+    out.update(("track_" + k, tr[k]) for k in tr.dtype.names if not k.startswith("reserved"))
+    out = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in out.items()}
+    assoc = bt.point_assoc().astype(np.float64)
+    per_scene = sum(v.nbytes for v in out.values()) // bt.S + 8 * bt.ncap + 24
+    budget = DUMP_BYTES_MAX - (1 << 20)                  # room for the .npy headers
+    scenes = np.arange(bt.S)
+    if per_scene * bt.S > budget:
+        scenes = np.sort(np.random.default_rng(0).choice(bt.S, budget // per_scene, replace=False))
+    out = {k: v[scenes] for k, v in out.items()}
+    out["point_assoc"] = np.concatenate([assoc[offsets[s]:offsets[s + 1]] for s in scenes])
+    out["point_offsets"] = np.concatenate([[0], np.cumsum(offsets[scenes + 1] - offsets[scenes])]).astype(np.float64)
+    out["scene_index"] = scenes.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(v))
+
+
 def replay_check(world, S, n_frames_done, weights, gathered, per_scene, local, pose_calls):
     """SURVEY 8(e): a scene's results do not depend on which GPU ran it.  Rank 0 re-runs the first scenes of rank 1's
     shard from frame 0 through the same sequence of calls in a context of its own and compares the records with
@@ -473,7 +506,11 @@ def main():
     ap.add_argument("--e2e-full-records", action="store_true",
                     help="end-to-end pass downloads all S * max_tracks records per frame instead of the live ones")
     ap.add_argument("--e2e-reps", type=int, default=5, help="end-to-end windows of K steps (the median is reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed (rank 0's scenes) to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path, not of --impl reference")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -588,6 +625,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms_max = float(t.item())
     value = world * S * K / (total_ms_max / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(bt, batches[f - 1].offsets, args.dump_outputs)
 
     # ---- per-kernel durations (CUDA events on the library's stream around every launch), on the K frames that follow
     # the device-timed ones: the track count rises slowly over a sequence, and the roofline figures must describe the

@@ -44,6 +44,8 @@ CASES = [
     ("c1_s21_jitter", 21, 40, synth.SceneSpec(jitter_lattice=True), None),
     ("c3_s7_dense", 7, 16, synth.SceneSpec.dense(), 10),
 ]
+# feature maps are stored every 7th frame; the long trace keeps every 14th so that its file stays under 1 MB
+FEATURE_EVERY = {"c1_s100_long": 14}
 
 
 # Clouds built to sit on the edges of the grid screen that the CUDA tracker step puts in front of DBSCAN
@@ -229,9 +231,9 @@ def main():
     for name, sid, nf, spec, mt in CASES:
         sc = synth.gen_scene(sid, nf, spec)
         recs = rh.run_reference_scene(sc.frames, sc.dts(), pose_fn=lambda x: np.zeros((len(x), 57)), max_tracks=mt)
-        d = trace_io.pack(sc.frames, sc.dts(), recs)
+        d = trace_io.pack(sc.frames, sc.dts(), recs, feature_every=FEATURE_EVERY.get(name, 7))
         d["max_tracks"] = np.array(4 if mt is None else mt, np.int32)
-        np.savez_compressed(os.path.join(GOLDEN, name + ".npz"), **d)
+        trace_io.save_npz(os.path.join(GOLDEN, name + ".npz"), d)
         print(name, "frames", nf, "tracks at end", len(recs[-1]["tracks"]), "next id", recs[-1]["next_track_id"],
               "dbscan runs", int(d["labels_ran"].sum()))
     np.savez_compressed(os.path.join(GOLDEN, "track0_export.npz"), **track0_export_golden())

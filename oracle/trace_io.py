@@ -3,6 +3,7 @@ produced by ``ref_harness.run_reference_scene`` and ``mmw_oracle.SceneOracle.ste
 into flat arrays for ``tests/golden/*.npz``."""
 from __future__ import annotations
 
+import zipfile
 from typing import Dict, List
 
 import numpy as np
@@ -53,6 +54,15 @@ def pack(frames: List[np.ndarray], dts: np.ndarray, recs: List[dict], feature_ev
     d["feat_off"] = np.cumsum([0] + [len(x) for x in feats]).astype(np.int64)
     d["feats"] = np.concatenate(feats, axis=0) if feats else np.zeros((0, 3, 8, 8, 5))
     return d
+
+
+def save_npz(path: str, d: Dict[str, np.ndarray]) -> None:
+    """``np.savez`` with LZMA instead of deflate (``np.load`` reads either): the float64 states of a long trace take
+    about a seventh less room, which keeps every golden file under 1 MB."""
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for k, v in d.items():
+            with z.open(k + ".npy", "w") as fh:
+                np.lib.format.write_array(fh, np.asanyarray(v))
 
 
 def unpack(d) -> dict:
