@@ -76,12 +76,9 @@ struct mmw_ctx {
     // throughput mode (MMW_STEP_PIPELINE): pose network on its own stream, its inputs double-buffered
     cudaStream_t pose_stream = nullptr;
     cudaEvent_t feat_done[2] = {nullptr, nullptr}, packt_done[2] = {nullptr, nullptr}, pose_done[2] = {nullptr, nullptr};
-    cudaEvent_t conv_done[2] = {nullptr, nullptr};   // the convolutions of a pipelined frame have run (gate of the next tracker step)
-    int pipe_gate = 0;               // MMW_PIPE_GATE: 1 = the tracker of frame k+1 starts when the convolutions of frame k are done
     int32_t *d_row_scene2 = nullptr, *d_row_track2 = nullptr, *d_row_slot2 = nullptr;
     int* d_pose_total2 = nullptr;
     int32_t* d_pose_extra = nullptr; // [2] rows dbscan_big_kernel appended for the tracks it spawned (fused steps), by input buffer
-    bool feat_late = true;           // MMW_FEAT_LATE=0: the feature kernel waits for dbscan_big_kernel and lays out every row (round 1)
     int rows_buf = 0;                // row maps / pose_total of the last feature launch (0 / 1)
     unsigned pipe_idx = 0;           // pipelined steps so far
     int pipe_r = -1;                 // result buffer the last step filled itself (-1: the last step was serial)
@@ -236,7 +233,7 @@ int mmw_destroy(mmw_ctx* x) {
     }
     for (int i = 0; i < 2; ++i)
         for (cudaEvent_t e : {x->h2d_done[i], x->stage_free[i], x->packed[i], x->results_done[i], x->feat_done[i],
-                              x->packt_done[i], x->pose_done[i], x->conv_done[i]})
+                              x->packt_done[i], x->pose_done[i]})
             if (e) cudaEventDestroy(e);
     if (x->h2d_stream) cudaStreamDestroy(x->h2d_stream);
     if (x->d2h_stream) cudaStreamDestroy(x->d2h_stream);
@@ -408,13 +405,11 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
             cudaEventCreateWithFlags(&x->results_done[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->feat_done[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->packt_done[i], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&x->conv_done[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->pose_done[i], cudaEventDisableTiming) != cudaSuccess) {
             mmw_destroy(x);
             return fail(MMW_ERR_CUDA, "cudaEventCreate failed");
         }
     }
-    { const char* env = getenv("MMW_PIPE_GATE"); x->pipe_gate = env ? atoi(env) : 0; }
     // the pose network is the critical path of the throughput mode: its CTAs are scheduled ahead of the tracker's
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
@@ -426,7 +421,6 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
     }
     ALLOC(x->d_pose_total, sizeof(int));
     ALLOC(x->d_pose_extra, 2 * sizeof(int32_t));
-    { const char* env = getenv("MMW_FEAT_LATE"); x->feat_late = !(env && atoi(env) == 0); }
     x->pose_cap = n_scenes * max_tracks;
     ALLOC(x->d_row_scene, sizeof(int32_t) * x->pose_cap);
     ALLOC(x->d_row_track, sizeof(int32_t) * x->pose_cap);
@@ -523,26 +517,32 @@ int mmw_load_pose_weights(mmw_ctx* x, int variant, const float* blob, size_t n) 
     return MMW_OK;
 }
 
+// Tensor-core path: conv1 -> conv2 -> dense1 -> dense2 on stream st, input buffer b, operands handed over as split
+// bf16 (pose_tc.cu).  before_fc2: an event dense 2 waits for (throughput mode: the frame's result records are packed).
+static int run_pose_tc(mmw_ctx* x, const PoseTcRun& r, int max_rows, int b, cudaStream_t st,
+                       cudaEvent_t before_fc2 = nullptr) {
+    const bool marks = st == x->stream;       // the per-kernel events are recorded on the context's stream
+    int nl = 0;
+    if (marks) prof_mark(x, MMW_K_CONV);
+    if (pose_tc_conv(&x->tc, r, st, &nl, b) != 0) return fail(MMW_ERR_CUDA, std::string("tensor-core conv: ") + pose_tc_error());
+    x->launches += nl;
+    if (marks) prof_mark(x, MMW_K_FC1);
+    if (pose_tc_fc1(&x->tc, r, max_rows, st, &nl, x->h_rows_hint ? *(volatile int32_t*)x->h_rows_hint : 0) != 0)
+        return fail(MMW_ERR_CUDA, std::string("tensor-core dense 1: ") + pose_tc_error());
+    x->launches += nl;
+    if (before_fc2) CK(cudaStreamWaitEvent(st, before_fc2, 0));
+    if (marks) prof_mark(x, MMW_K_FC2);
+    if (pose_tc_fc2(&x->tc, r, max_rows, st, &nl) != 0) return fail(MMW_ERR_CUDA, std::string("tensor-core dense 2: ") + pose_tc_error());
+    x->launches += nl;
+    if (marks) prof_mark(x, -1);
+    return MMW_OK;
+}
+
 static int run_pose_net(mmw_ctx* x, float* keypoints_by_slot, int max_rows) {
     if (x->use_tc && x->tc.ready) {
-        // tensor-core path: conv1 -> conv2 -> dense1 -> dense2, operands handed over as split bf16 (pose_tc.cu)
         PoseTcRun r{x->d_pose_total, x->b1, x->b2, x->d_bn1s, x->d_bn1t, x->bd1, x->d_bn2s, x->d_bn2t, x->bd2,
                     x->d_pose_out, keypoints_by_slot, x->d_row_scene, x->d_row_slot, x->tcap};
-        int nl = 0;
-        prof_mark(x, MMW_K_CONV);
-        if (pose_tc_conv(&x->tc, r, x->stream, &nl) != 0)
-            return fail(MMW_ERR_CUDA, std::string("tensor-core conv: ") + pose_tc_error());
-        x->launches += nl;
-        prof_mark(x, MMW_K_FC1);
-        if (pose_tc_fc1(&x->tc, r, max_rows, x->stream, &nl, x->h_rows_hint ? *(volatile int32_t*)x->h_rows_hint : 0) != 0)
-            return fail(MMW_ERR_CUDA, std::string("tensor-core dense 1: ") + pose_tc_error());
-        x->launches += nl;
-        prof_mark(x, MMW_K_FC2);
-        if (pose_tc_fc2(&x->tc, r, max_rows, x->stream, &nl) != 0)
-            return fail(MMW_ERR_CUDA, std::string("tensor-core dense 2: ") + pose_tc_error());
-        x->launches += nl;
-        prof_mark(x, -1);
-        return MMW_OK;
+        return run_pose_tc(x, r, max_rows, 0, x->stream);
     }
     // CUDA-core fp32 path (kept for numerics comparison)
     ConvArgs ca{x->d_feats, x->w1, x->b1, x->w2, x->b2, x->d_bn1s, x->d_bn1t, x->d_act2, x->d_pose_total};
@@ -570,9 +570,32 @@ static int run_pose_net(mmw_ctx* x, float* keypoints_by_slot, int max_rows) {
 //   pose stream : wait feat[b]  [conv1][conv2][dense 1]  wait packt[b]  [dense 2 -> keypoints, results b]  ev pose[b]
 // so the tracker of frame k+1 runs under the convolutions / dense 1 of frame k.  The pose stream is serial, hence
 // "pose(k-1) done" implies every earlier frame's pose work is done (its activations are single-buffered).
-static int pipeline_pose(mmw_ctx* x, bool late);
+static int pipeline_pose(mmw_ctx* x);
 static int estimate_posture_impl(mmw_ctx* x, bool late);
 static int launch_pack_tracks(mmw_ctx* x, float* results);
+
+// The feature stage on stream st: the pose-row scan (unless pose_feature_kernel folds it in), then the feature maps,
+// the packed tensor-core input of buffer b and the row maps of buffer b.  late: the feature kernel lays out the rows of
+// the tracks step_kernel left and does not wait for dbscan_big_kernel, which appends the rows of the tracks it spawns.
+static int launch_feature_stage(mmw_ctx* x, int b, bool late, cudaStream_t st) {
+    int* pose_total = b ? x->d_pose_total2 : x->d_pose_total;
+    if (!x->fold_pose_index) {
+        prof_mark(x, MMW_K_POSE_INDEX);
+        CK(launch_pose_index(x->d_scenes, x->S, pose_total, x->d_counters, st));
+        x->launches++;
+    }
+    PoseFeatArgs fa{x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats,
+                    (x->use_tc && x->tc.ready) ? pose_tc_input(&x->tc, b) : nullptr, b ? x->d_row_scene2 : x->d_row_scene,
+                    b ? x->d_row_track2 : x->d_row_track, b ? x->d_row_slot2 : x->d_row_slot,
+                    x->fold_pose_index ? x->d_defer + 1 + x->S : nullptr, pose_total, x->d_counters, x->S};
+    fa.rows_hint = x->d_rows_hint;
+    fa.late_extra = late ? x->d_pose_extra + b : nullptr;
+    x->rows_buf = b;
+    prof_mark(x, MMW_K_POSE_FEATURES);
+    CK(launch_pose_features(fa, x->S, st));
+    x->launches++;
+    return MMW_OK;
+}
 
 int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double* dt, uint32_t flags) {
     if (!x || !offsets || !dt) return fail(MMW_ERR_INVALID, "ctx/offsets/dt is NULL");
@@ -630,28 +653,23 @@ int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double*
     a.defer_hint = x->d_defer_hint;
     a.ring_hist = x->d_ring_hist;
     const bool pipelined = (flags & MMW_STEP_PIPELINE) != 0;
-    // fused steps on the tensor-core pose path: the feature kernel does not wait for dbscan_big_kernel, which appends
-    // the rows of the tracks it spawns itself (StepArgs::nr_*)
-    // (serial mode only: in throughput mode, where the pose network of the previous frame holds most SMs, it measured 2 %
-    // slower -- 0.2324 against 0.2274 ms per step -- and 1.7 % faster in serial mode, 0.2419 against 0.2461)
-    const bool late = x->feat_late && !pipelined && (flags & MMW_STEP_POSE) && x->fold_pose_index && x->use_tc && x->tc.ready;
+    // fused serial steps on the tensor-core pose path: the feature kernel does not wait for dbscan_big_kernel, which
+    // appends the rows of the tracks it spawns itself (StepArgs::nr_*, buffer 0).  In throughput mode, where the pose
+    // network of the previous frame holds most SMs, this measured 2 % slower -- 0.2324 against 0.2274 ms per step --
+    // and 1.7 % faster in serial mode, 0.2419 against 0.2461.
+    const bool late = !pipelined && (flags & MMW_STEP_POSE) && x->fold_pose_index && x->use_tc && x->tc.ready;
     if (late) {
-        const int b = pipelined ? (int)(x->pipe_idx & 1u) : 0;
         a.nr_feats = x->d_feats;
-        a.nr_packed = pose_tc_input(&x->tc, b);
-        a.nr_row_scene = b ? x->d_row_scene2 : x->d_row_scene;
-        a.nr_row_track = b ? x->d_row_track2 : x->d_row_track;
-        a.nr_row_slot = b ? x->d_row_slot2 : x->d_row_slot;
-        a.nr_extra = x->d_pose_extra + b;
+        a.nr_packed = pose_tc_input(&x->tc);
+        a.nr_row_scene = x->d_row_scene;
+        a.nr_row_track = x->d_row_track;
+        a.nr_row_slot = x->d_row_slot;
+        a.nr_extra = x->d_pose_extra;
     }
     if (pipelined) {
         if (!(flags & MMW_STEP_POSE) || !(x->use_tc && x->tc.ready))
             return fail(MMW_ERR_STATE, "MMW_STEP_PIPELINE needs MMW_STEP_POSE and the tensor-core pose path");
         if (flags & MMW_STEP_RECORD_LABELS) return fail(MMW_ERR_INVALID, "MMW_STEP_PIPELINE cannot record labels");
-        // The persistent convolution kernels need (almost) whole SMs: tracker CTAs that are resident when one of them
-        // starts delay its slowest CTA by up to a tracker CTA's lifetime.  With the gate the tracker of the next frame
-        // starts once the previous frame's convolutions have run, under dense 1 / dense 2, which leave room.
-        if (x->pipe_gate && x->pose_pending) CK(cudaStreamWaitEvent(x->stream, x->conv_done[(x->pipe_idx + 1) & 1], 0));
         // frame k-2 used the same pose inputs / row maps (buffer k & 1): its pose network must be done before
         // dbscan_big_kernel appends rows and the feature kernel fills them.  Queued in front of the tracker kernels (not
         // between dbscan_big_kernel and the feature kernel, whose dependent launch it would undo); already satisfied in
@@ -669,7 +687,7 @@ int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double*
     x->launches += 2;          // step_kernel + dbscan_big_kernel
     prof_mark(x, -1);
     int rc = MMW_OK;
-    if (pipelined) rc = pipeline_pose(x, late);
+    if (pipelined) rc = pipeline_pose(x);
     else if (flags & MMW_STEP_POSE) rc = estimate_posture_impl(x, late);
     if (host_stage >= 0) x->stage_pending = host_stage;      // recorded at the head of the next step (see above)
     return rc;
@@ -682,21 +700,8 @@ static int estimate_posture_impl(mmw_ctx* x, bool late) {
     if (!x->has_weights) return fail(MMW_ERR_STATE, "estimate_posture needs mmw_load_pose_weights first");
     CK(cudaSetDevice(x->device));
     CK(join_pose(x));
-    if (!x->fold_pose_index) {
-        prof_mark(x, MMW_K_POSE_INDEX);
-        CK(launch_pose_index(x->d_scenes, x->S, x->d_pose_total, x->d_counters, x->stream));
-        x->launches++;
-    }
-    PoseFeatArgs fa{x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats,
-                    (x->use_tc && x->tc.ready) ? pose_tc_input(&x->tc) : nullptr, x->d_row_scene, x->d_row_track,
-                    x->d_row_slot, x->fold_pose_index ? x->d_defer + 1 + x->S : nullptr, x->d_pose_total, x->d_counters,
-                    x->S};
-    fa.rows_hint = x->d_rows_hint;
-    fa.late_extra = late ? x->d_pose_extra : nullptr;
-    x->rows_buf = 0;
-    prof_mark(x, MMW_K_POSE_FEATURES);
-    CK(launch_pose_features(fa, x->S, x->stream));
-    x->launches++;
+    const int rc = launch_feature_stage(x, 0, late, x->stream);
+    if (rc != MMW_OK) return rc;
     return run_pose_net(x, x->d_keypoints, x->pose_cap);
 }
 
@@ -704,17 +709,7 @@ int mmw_pose_features_only(mmw_ctx* x) {
     if (!x) return fail(MMW_ERR_INVALID, "ctx is NULL");
     CK(cudaSetDevice(x->device));
     CK(join_pose(x));
-    if (!x->fold_pose_index) {
-        CK(launch_pose_index(x->d_scenes, x->S, x->d_pose_total, x->d_counters, x->stream));
-        x->launches++;
-    }
-    PoseFeatArgs fa{x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats, nullptr, x->d_row_scene,
-                    x->d_row_track, x->d_row_slot, x->fold_pose_index ? x->d_defer + 1 + x->S : nullptr, x->d_pose_total,
-                    x->d_counters, x->S};
-    x->rows_buf = 0;
-    CK(launch_pose_features(fa, x->S, x->stream));
-    x->launches++;
-    return MMW_OK;
+    return launch_feature_stage(x, 0, false, x->stream);
 }
 
 int mmw_set_keypoints(mmw_ctx* x, int scene, int track_index, const float* kp57) {
@@ -1233,24 +1228,11 @@ static int launch_pack_tracks(mmw_ctx* x, float* results) {
     return MMW_OK;
 }
 
-static int pipeline_pose(mmw_ctx* x, bool late) {
+static int pipeline_pose(mmw_ctx* x) {
     const int b = (int)(x->pipe_idx & 1u);
     cudaStream_t T = x->stream, P = x->pose_stream;
-    int32_t *row_scene = b ? x->d_row_scene2 : x->d_row_scene, *row_track = b ? x->d_row_track2 : x->d_row_track,
-            *row_slot = b ? x->d_row_slot2 : x->d_row_slot;
-    int* pose_total = b ? x->d_pose_total2 : x->d_pose_total;
-    if (!x->fold_pose_index) {
-        CK(launch_pose_index(x->d_scenes, x->S, pose_total, x->d_counters, T));
-        x->launches++;
-    }
-    PoseFeatArgs fa{x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats, pose_tc_input(&x->tc, b), row_scene,
-                    row_track, row_slot, x->fold_pose_index ? x->d_defer + 1 + x->S : nullptr, pose_total, x->d_counters,
-                    x->S};
-    fa.rows_hint = x->d_rows_hint;
-    fa.late_extra = late ? x->d_pose_extra + b : nullptr;
-    x->rows_buf = b;
-    CK(launch_pose_features(fa, x->S, T));
-    x->launches++;
+    int rc = launch_feature_stage(x, b, false, T);
+    if (rc != MMW_OK) return rc;
     CK(cudaEventRecord(x->feat_done[b], T));
     // the result records of this frame: buffer b must have been downloaded (frame k-2), and the keypoints the tracker
     // side copies are final once frame k-1's pose network is done
@@ -1259,22 +1241,16 @@ static int pipeline_pose(mmw_ctx* x, bool late) {
         CK(cudaStreamWaitEvent(T, x->results_done[b], 0));
     }
     if (x->pipe_idx >= 1 && x->pose_pending) CK(cudaStreamWaitEvent(T, x->pose_done[b ^ 1], 0));
-    int rc = launch_pack_tracks(x, x->d_results[b]);
+    rc = launch_pack_tracks(x, x->d_results[b]);
     if (rc != MMW_OK) return rc;
     CK(cudaEventRecord(x->packt_done[b], T));
     // pose stream
     CK(cudaStreamWaitEvent(P, x->feat_done[b], 0));
-    PoseTcRun r{pose_total, x->b1, x->b2, x->d_bn1s, x->d_bn1t, x->bd1, x->d_bn2s, x->d_bn2t, x->bd2, x->d_pose_out,
-                x->d_keypoints, row_scene, row_slot, x->tcap, x->d_results[b], row_track, fade_cfg(x)};
-    int nl = 0;
-    if (pose_tc_conv(&x->tc, r, P, &nl, b) != 0) return fail(MMW_ERR_CUDA, std::string("tensor-core conv: ") + pose_tc_error());
-    x->launches += nl;
-    if (x->pipe_gate) CK(cudaEventRecord(x->conv_done[b], P));     // (an event between two kernels undoes their dependent launch)
-    if (pose_tc_fc1(&x->tc, r, x->pose_cap, P, &nl, x->h_rows_hint ? *(volatile int32_t*)x->h_rows_hint : 0) != 0) return fail(MMW_ERR_CUDA, std::string("tensor-core dense 1: ") + pose_tc_error());
-    x->launches += nl;
-    CK(cudaStreamWaitEvent(P, x->packt_done[b], 0));
-    if (pose_tc_fc2(&x->tc, r, x->pose_cap, P, &nl) != 0) return fail(MMW_ERR_CUDA, std::string("tensor-core dense 2: ") + pose_tc_error());
-    x->launches += nl;
+    PoseTcRun r{b ? x->d_pose_total2 : x->d_pose_total, x->b1, x->b2, x->d_bn1s, x->d_bn1t, x->bd1, x->d_bn2s, x->d_bn2t,
+                x->bd2, x->d_pose_out, x->d_keypoints, b ? x->d_row_scene2 : x->d_row_scene, b ? x->d_row_slot2 : x->d_row_slot,
+                x->tcap, x->d_results[b], b ? x->d_row_track2 : x->d_row_track, fade_cfg(x)};
+    rc = run_pose_tc(x, r, x->pose_cap, b, P, x->packt_done[b]);
+    if (rc != MMW_OK) return rc;
     CK(cudaEventRecord(x->pose_done[b], P));
     x->pose_pending = true;
     x->pipe_r = b;

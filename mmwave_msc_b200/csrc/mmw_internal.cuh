@@ -1,6 +1,5 @@
 // Internal device-side data model of libmmw (see DESIGN.md "Data layout in HBM").
 #pragma once
-#include <cstdlib>
 #include <utility>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -13,10 +12,7 @@ constexpr int kFeatPts = 64;      // points kept per track ring frame (format_si
 constexpr int kRawCols = 5;       // x, y, z, doppler, peakVal (sensor frame, fp32)
 constexpr int kKp = 57;           // 19 joints x 3
 constexpr int kHistBytes = 272;   // per ring frame: 256 cell counts of the grid screen (uint8, saturating) + flag + pad
-#ifndef MMW_STEP_THREADS
-#define MMW_STEP_THREADS 128     // threads per scene CTA of the tracker step (profiling builds override it)
-#endif
-constexpr int kStepThreads = MMW_STEP_THREADS;
+constexpr int kStepThreads = 128;    // threads per scene CTA of the tracker step
 constexpr int kStepWarps = kStepThreads / 32;
 constexpr int kMaxTcap = 32;
 
@@ -128,15 +124,6 @@ struct StepArgs {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-inline bool pdl_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char* env = getenv("MMW_PDL");
-        on = (env && env[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-
 // kernel<<<grid, block, smem, st>>>(args...) with the PDL attribute (and an optional cluster shape)
 template <class... KArgs, class... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
@@ -150,11 +137,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
         at[n].val.clusterDim.x = cluster.x; at[n].val.clusterDim.y = cluster.y; at[n].val.clusterDim.z = cluster.z;
         ++n;
     }
-    if (pdl_enabled()) {
-        at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
+    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
     cfg.attrs = at; cfg.numAttrs = n;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }

@@ -11,8 +11,8 @@
 // columns [C,2C); the epilogue adds the two halves, bias, ReLU (+ BatchNorm after conv2) and writes the next layer's
 // split operand directly.
 //
-// Dense layers: 128 x BN tiles (gemm_tc_kernel) or 256 x BN tiles on CTA pairs (gemm_tc_pair_kernel,
-// tcgen05.mma.cta_group::2), K blocks of 64 (SWIZZLE_128B); each pipeline stage holds the four operand tiles
+// Dense layers: dense 1 on 256 x BN tiles of CTA pairs (gemm_tc_pair_kernel, tcgen05.mma.cta_group::2), dense 2 on
+// 128 x 64 tiles (gemm_tc_kernel), K blocks of 64 (SWIZZLE_128B); each pipeline stage holds the four operand tiles
 // {A_hi, A_lo, W_hi, W_lo} of one K block (loaded once by TMA, used by three MMAs per 16-wide K step).
 //
 // Warp roles in the dense kernels: warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM alloc), warps 2-5 = epilogue.
@@ -142,7 +142,6 @@ struct ConvTcArgs {
     const __nv_bfloat16* in;                       // packed input  [row][D][8][8][CK]  (hi | lo per position)
     __nv_bfloat16* out0;                           // MODE 0: act1 packed [row][D][8][8][32]; MODE 1: A_hi [row][Kf]
     __nv_bfloat16* out1;                           // MODE 1: A_lo [row][Kf]
-    int D, taps;
     int dbg;                                       // timing experiments only (MMW_GEMM_DBG): 8 = producers idle,
                                                    // 16 = no MMAs, 32 = no epilogue stores
 };
@@ -181,16 +180,17 @@ __device__ __forceinline__ uint64_t make_desc_interleaved(uint32_t saddr, uint32
 //
 // CK   = K' per tap = 2 * padded input channels (hi | lo): 16 for conv1, 32 for conv2
 // NOUT = MMA N     = 2 * output channels: 32 for conv1, 64 for conv2
-// KD  = taps in depth.  KD == D == 3: define_CNN_3D.  D == 1, KD == 1: define_CNN, one 8 x 8 map per slab (80 of the 128
-// MMA rows of a tile used, the per-sample hand-over paid for every map).  D == 3, KD == 1: define_CNN again, but THREE
-// consecutive samples ride as the three depth planes of one slab -- their packed inputs and outputs are contiguous in
-// exactly the 3-D layout, the depth taps are simply not issued (9 taps, the d padding planes stay unused) -- 240 of 256
-// MMA rows used and a third of the hand-overs: the C4 configuration's convolutions went from 0.83 ms to the figure in
-// DESIGN.md.  Samples past the row count in the last triple are staged as zeros and not stored.
-template <int CK, int NOUT, int MODE, int D, int KD = D>
+// KD   = taps in depth.  A slab always holds D = 3 depth planes.  KD == 3: define_CNN_3D, one sample per slab.
+// KD == 1: define_CNN, THREE consecutive samples ride as the three depth planes of one slab -- their packed inputs and
+// outputs are contiguous in exactly the 3-D layout, the depth taps are simply not issued (9 taps, the d padding planes
+// stay unused) -- 240 of 256 MMA rows used and a third of the per-sample hand-overs of one 8 x 8 map per slab: the C4
+// configuration's convolutions went from 0.83 ms to the figure in DESIGN.md.  Samples past the row count in the last
+// triple are staged as zeros and not stored.
+template <int CK, int NOUT, int MODE, int KD>
 __global__ void __launch_bounds__(kSlabThreads, 1)
 conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) {
-    constexpr bool TRIPLE = D == 3 && KD == 1;
+    constexpr int D = 3;                             // depth planes of a slab
+    constexpr bool TRIPLE = KD == 1;
     constexpr int NCH = CK / 8;                      // 16-byte chunks per position
     constexpr int ATOM = NCH * 128;                  // bytes of one 8-row atom
     constexpr int SLAB_BYTES = kSlabAtoms * ATOM;
@@ -200,7 +200,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) 
     constexpr int COUT = NOUT / 2;
     constexpr uint32_t TCOLS = 4 * NOUT;             // 2 accumulator buffers x 2 M tiles
     constexpr int taps = KD == 3 ? 27 : 9;
-    constexpr int MT = D == 3 ? 2 : 1;               // M tiles of 128 rows per sample (or triple of samples)
+    constexpr int MT = 2;                            // M tiles of 128 rows per sample (or triple of samples)
 
     extern __shared__ unsigned char smem_raw[];
     unsigned char* smem = reinterpret_cast<unsigned char*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -296,47 +296,45 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) 
             for (int j = 0; j < ITEMS; ++j) cur[j] = nxt[j];
         }
     } else if (warp == 4 || warp == 5) {
-        // ===== MMA issuers: warp 4 owns M tile 0, warp 5 loads the weights and owns M tile 1 (3-D net) =====
+        // ===== MMA issuers: warp 4 owns M tile 0, warp 5 owns M tile 1 =====
         // Every operand address is slab/weight base + a compile-time constant, so one MMA costs two 64-bit adds.
         const int mt = warp - 4;
         if (lane == 0) {
-            if (mt < MT) {
-                constexpr uint32_t idesc = make_idesc(NOUT);
-                constexpr uint32_t idesc_lo = make_idesc(NOUT / 2);                    // conv 2, a_lo chunk: N = cout
-                const uint64_t db0 = make_desc<32>(smem_u32(sB));                      // weight rows are one K16 wide
-                const uint64_t da00 = make_desc_interleaved(smem_u32(slab) + (uint32_t)((1 + mt * 16) * ATOM), 128, ATOM);
-                mbar_wait(bfull, 0);
-                int n = 0, u = 0;
-                for (int row = blockIdx.x; row < rows; row += gridDim.x, ++n) {
-                    const int buf = n & 1;
-                    mbar_wait(&tempty[buf], (uint32_t)(((n >> 1) & 1) ^ 1));
+            constexpr uint32_t idesc = make_idesc(NOUT);
+            constexpr uint32_t idesc_lo = make_idesc(NOUT / 2);                    // conv 2, a_lo chunk: N = cout
+            const uint64_t db0 = make_desc<32>(smem_u32(sB));                      // weight rows are one K16 wide
+            const uint64_t da00 = make_desc_interleaved(smem_u32(slab) + (uint32_t)((1 + mt * 16) * ATOM), 128, ATOM);
+            mbar_wait(bfull, 0);
+            int n = 0, u = 0;
+            for (int row = blockIdx.x; row < rows; row += gridDim.x, ++n) {
+                const int buf = n & 1;
+                mbar_wait(&tempty[buf], (uint32_t)(((n >> 1) & 1) ^ 1));
+                tc_fence_after();
+                const uint32_t tmem_d = tmem_base + (uint32_t)((buf * 2 + mt) * NOUT);
+#pragma unroll
+                for (int c = 0; c < 3; ++c, ++u) {
+                    const int slot = u % NSLAB;
+                    mbar_wait(&sfull[slot], (uint32_t)((u / NSLAB) & 1));
                     tc_fence_after();
-                    const uint32_t tmem_d = tmem_base + (uint32_t)((buf * 2 + mt) * NOUT);
+                    const uint64_t da0 = da00 + (uint64_t)((slot * SLAB_BYTES) >> 4);
 #pragma unroll
-                    for (int c = 0; c < 3; ++c, ++u) {
-                        const int slot = u % NSLAB;
-                        mbar_wait(&sfull[slot], (uint32_t)((u / NSLAB) & 1));
-                        tc_fence_after();
-                        const uint64_t da0 = da00 + (uint64_t)((slot * SLAB_BYTES) >> 4);
+                    for (int kdi = 0; kdi < (KD == 3 ? 3 : 1); ++kdi) {
 #pragma unroll
-                        for (int kdi = 0; kdi < (KD == 3 ? 3 : 1); ++kdi) {
+                        for (int kwi = 0; kwi < 3; ++kwi) {
+                            const int kd = KD == 3 ? kdi - 1 : 0, kw = kwi - 1;
+                            const int tap = KD == 3 ? (kdi * 3 + c) * 3 + kwi : c * 3 + kwi;
+                            const bool first = c == 0 && kdi == 0 && kwi == 0;
+                            const int aoff = ((1 + kd) * 10 + kw) * ATOM;        // whole atoms: tap = tile shift
 #pragma unroll
-                            for (int kwi = 0; kwi < 3; ++kwi) {
-                                const int kd = KD == 3 ? kdi - 1 : 0, kw = kwi - 1;
-                                const int tap = KD == 3 ? (kdi * 3 + c) * 3 + kwi : c * 3 + kwi;
-                                const bool first = c == 0 && kdi == 0 && kwi == 0;
-                                const int aoff = ((1 + kd) * 10 + kw) * ATOM;        // whole atoms: tap = tile shift
-#pragma unroll
-                                for (int kk = 0; kk < CK / 16; ++kk)
-                                    if (!(a.dbg & 16)) umma_bf16(tmem_d, da0 + (uint64_t)((aoff + kk * 256) >> 4),
-                                              db0 + (uint64_t)((tap * B_TAP + kk * NOUT * 32) >> 4), kk == 0 ? idesc : idesc_lo,
-                                              (first && kk == 0) ? 0u : 1u);
-                            }
+                            for (int kk = 0; kk < CK / 16; ++kk)
+                                if (!(a.dbg & 16)) umma_bf16(tmem_d, da0 + (uint64_t)((aoff + kk * 256) >> 4),
+                                          db0 + (uint64_t)((tap * B_TAP + kk * NOUT * 32) >> 4), kk == 0 ? idesc : idesc_lo,
+                                          (first && kk == 0) ? 0u : 1u);
                         }
-                        umma_commit(&sempty[slot]);   // the slab may be refilled once both issuers are done with it
                     }
-                    umma_commit(&tfull[buf]);
+                    umma_commit(&sempty[slot]);   // the slab may be refilled once both issuers are done with it
                 }
+                umma_commit(&tfull[buf]);
             }
         }
     } else {
@@ -349,8 +347,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) 
             tc_fence_after();
             float y[2][COUT];
 #pragma unroll
-            for (int mt = 0; mt < 2; ++mt) {
-                if (mt >= MT) break;
+            for (int mt = 0; mt < MT; ++mt) {
                 const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)((buf * 2 + mt) * NOUT);
                 uint32_t v[32];
                 tmem_ld32(taddr, v);
@@ -369,8 +366,7 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) 
             __syncwarp();
             if (lane == 0) mbar_arrive(&tempty[buf]);           // accumulators are in registers now
 #pragma unroll
-            for (int mt = 0; mt < 2; ++mt) {
-                if (mt >= MT) break;
+            for (int mt = 0; mt < MT; ++mt) {
                 const int m = q * 32 + lane;
                 const int aidx = mt * 16 + (m >> 3), hh = m & 7;
                 const int d = aidx / 10, w2 = aidx % 10;
@@ -414,18 +410,18 @@ conv_slab_kernel(const __grid_constant__ CUtensorMap map_b, const ConvTcArgs a) 
 }
 
 // =====================================================================================================
-// Dense layers: split-bf16 GEMM, 128 x BN tiles
+// Dense layers: split-bf16 GEMM
 // =====================================================================================================
 struct GemmTcArgs {
     const int* n_rows;
     const float *bias, *bn_scale, *bn_shift;
-    __nv_bfloat16 *out_hi, *out_lo;      // MODE 0: next layer's operand [row][N]
-    float* out;                          // MODE 1: [row][57]
-    float* keypoints;                    // MODE 1: scatter target or nullptr
+    __nv_bfloat16 *out_hi, *out_lo;      // dense 1: next layer's operand [row][N]
+    float* out;                          // dense 2: [row][57]
+    float* keypoints;                    // dense 2: scatter target or nullptr
     const int32_t *row_scene, *row_slot;
     int K, N, tcap;
     int dbg;                             // timing experiments only (MMW_GEMM_DBG): 1 = no TMA loads, 2 = no MMAs
-    float* results = nullptr;            // MODE 1, throughput mode: packed result records to finish (pose_tc.cuh)
+    float* results = nullptr;            // dense 2, throughput mode: packed result records to finish (pose_tc.cuh)
     const int32_t* row_track = nullptr;
     FadeCfg fade = {0, 0, 0, 0, 0, 0};
 };
@@ -483,15 +479,15 @@ __device__ __forceinline__ void gemm_store_keypoints(const GemmTcArgs& a, const 
 }
 
 template <int BN, int STAGES>
-constexpr int gemm_smem_bytes() { return STAGES * (2 * 128 * kBK * 2 + 2 * BN * kBK * 2) + 1024 + 256 + (3 * BN * 4 > 1536 ? 3 * BN * 4 : 1536); }
+constexpr int gemm_smem_bytes() { return STAGES * (2 * 128 * kBK * 2 + 2 * BN * kBK * 2) + 1024 + 256 + 3 * 128 * 4; }
 
-// MODE 0: out = split(BN(relu(acc + bias)))      MODE 1: out = acc + bias (first 57 columns), scattered to tracks
-// KS > 1 (MODE 1, dense 2): split K over a cluster of KS CTAs (blockIdx.x = cluster rank = K slice).  Dense 2 has only
+// Dense 2 on 128 x BN tiles of one CTA (cta_group::1): out = acc + bias (first 57 columns), scattered to tracks.
+// KS > 1: split K over a cluster of KS CTAs (blockIdx.x = cluster rank = K slice).  Dense 2 has only
 // ceil(rows / 128) row tiles -- 16 CTAs at C2 -- and each of them streamed 1.1 MB of operands through ONE SM's L2 port
 // (14 us of main loop for 0.34 GFLOP).  With the split, KS times as many SMs pull a KS-th each; the partial
 // accumulators go TMEM -> registers -> the leader's shared memory (st.shared::cluster into the idle pipeline stages)
 // and the leader adds them in rank order: the sum of a row does not depend on where the row sits in the batch.
-template <int BN, int STAGES, int MODE, int KS = 1>
+template <int BN, int STAGES, int KS = 1>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                const __grid_constant__ CUtensorMap map_wh, const __grid_constant__ CUtensorMap map_wl,
@@ -504,7 +500,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant
     // (mmw_internal.cuh) that grid had completed before this one could start, so it may be read before pdl_wait()
     // -- which lets the CTAs past the last row leave without holding shared memory while they wait.
     const int rows = __ldcg(a.n_rows);
-    const int m0 = blockIdx.y * BM, n0 = MODE == 1 ? 0 : blockIdx.x * BN;
+    const int m0 = blockIdx.y * BM;
     if (m0 >= rows) return;
 
     extern __shared__ unsigned char smem_raw[];
@@ -514,7 +510,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant
     uint64_t* tmem_full = empty + STAGES;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    static_assert(KS == 1 || MODE == 1, "the K split is written for dense 2");
     const int ks = KS > 1 ? (int)blockIdx.x : 0;         // cluster rank (cluster = (KS, 1, 1), gridDim.x = KS)
     const int nkb = a.K / kBK / KS, kb0 = ks * nkb;
 
@@ -547,8 +542,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant
                 const int k0 = (kb0 + kb) * kBK;
                 tma_load_2d(st, &map_ah, &full[s], k0, m0);
                 tma_load_2d(st + A_BYTES, &map_al, &full[s], k0, m0);
-                tma_load_2d(st + 2 * A_BYTES, &map_wh, &full[s], k0, n0);
-                tma_load_2d(st + 2 * A_BYTES + B_BYTES, &map_wl, &full[s], k0, n0);
+                tma_load_2d(st + 2 * A_BYTES, &map_wh, &full[s], k0, 0);
+                tma_load_2d(st + 2 * A_BYTES + B_BYTES, &map_wl, &full[s], k0, 0);
             }
         }
     } else if (warp == 1) {
@@ -578,57 +573,28 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant
         // accumulators of this K slice into registers; the exchange follows below, outside the role branches
     } else {
         const int q = warp & 3;
-        // bias / BatchNorm constants of this column tile into shared memory while the main loop runs
-        float* sconst = reinterpret_cast<float*>(tmem_slot + 2);
-        if (MODE == 0) {
-            for (int i = threadIdx.x - 64; i < BN; i += 128) {
-                sconst[i] = __ldg(a.bias + n0 + i);
-                sconst[BN + i] = __ldg(a.bn_scale + n0 + i);
-                sconst[2 * BN + i] = __ldg(a.bn_shift + n0 + i);
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-        } else {
-            gemm_load_row_maps(a, reinterpret_cast<int*>(sconst), m0, min(BM, rows - m0), threadIdx.x - 64);
-        }
+        // the rows' scene / slot / track indices into shared memory while the main loop runs
+        int* maps = reinterpret_cast<int*>(tmem_slot + 2);
+        gemm_load_row_maps(a, maps, m0, min(BM, rows - m0), threadIdx.x - 64);
         mbar_wait(tmem_full, 0);
         tc_fence_after();
         const int row = m0 + q * 32 + lane;
+        // the 57 outputs of a row go through shared memory (the pipeline stages are idle now) so that the global writes
+        // below are coalesced; lane-per-row scalar stores cost 32 sectors per instruction
+        float* stg = reinterpret_cast<float*>(smem);
 #pragma unroll 1
         for (int c0 = 0; c0 < BN; c0 += 32) {
             uint32_t v[32];
             tmem_ld32(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);
             if (row >= rows) continue;
-            if (MODE == 0) {
-                __align__(16) __nv_bfloat16 hi[32], lo[32];
 #pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    float x = fmaxf(__uint_as_float(v[j]) + sconst[c0 + j], 0.f);
-                    x = fmaf(x, sconst[BN + c0 + j], sconst[2 * BN + c0 + j]);
-                    split2(x, hi[j], lo[j]);
-                }
-                uint4* oh = reinterpret_cast<uint4*>(a.out_hi + (size_t)row * a.N + n0 + c0);
-                uint4* ol = reinterpret_cast<uint4*>(a.out_lo + (size_t)row * a.N + n0 + c0);
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    oh[i] = reinterpret_cast<const uint4*>(hi)[i];
-                    ol[i] = reinterpret_cast<const uint4*>(lo)[i];
-                }
-            } else {
-                // dense 2: the 57 outputs of a row go through shared memory (the pipeline stages are idle now) so that
-                // the global writes below are coalesced; lane-per-row scalar stores cost 32 sectors per instruction
-                float* stg = reinterpret_cast<float*>(smem);
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int n = c0 + j;
-                    if (n < kKp) stg[(q * 32 + lane) * kKp + n] = __uint_as_float(v[j]) + __ldg(a.bias + n);
-                }
+            for (int j = 0; j < 32; ++j) {
+                const int n = c0 + j;
+                if (n < kKp) stg[(q * 32 + lane) * kKp + n] = __uint_as_float(v[j]) + __ldg(a.bias + n);
             }
         }
-        if (MODE == 1) {
-            asm volatile("bar.sync 1, 128;" ::: "memory");                     // the four epilogue warps
-            gemm_store_keypoints(a, reinterpret_cast<const float*>(smem), reinterpret_cast<const int*>(sconst), m0,
-                                 min(BM, rows - m0), q, lane, threadIdx.x - 64);
-        }
+        asm volatile("bar.sync 1, 128;" ::: "memory");                         // the four epilogue warps
+        gemm_store_keypoints(a, stg, maps, m0, min(BM, rows - m0), q, lane, threadIdx.x - 64);
     }
     if (KS > 1) {
         // Reduce-scatter by row quadrant: the 32 rows TMEM lane quadrant q holds (epilogue warp with warp % 4 == q)
@@ -705,7 +671,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant
 }
 
 // ---- dense 1 on CTA pairs: tcgen05.mma.cta_group::2 ----------------------------------------------------------
-// The single-CTA kernel above keeps only two 80 KB stages in flight, so every K block pays the HBM/L2 round trip
+// A single CTA with 128 x 192 tiles keeps only two 80 KB stages in flight, so every K block pays the HBM/L2 round trip
 // (per K block: (latency + 80 KB transfer + 1152 MMA cycles) / 2 stages ~ 1950 cycles against 1152 of tensor work).
 // A CTA pair (two SMs of one TPC, cluster (2,1,1)) runs ONE 256 x BN MMA per K step: each CTA stages its own 128
 // rows of A and only HALF of the W tile (BN/2 rows), the tensor cores exchange the halves.  A stage shrinks to
@@ -938,16 +904,12 @@ struct TcImpl {
     __nv_bfloat16 *h_hi = nullptr, *h_lo = nullptr;                   // dense-2 operand [rows_pad][H]
     __nv_bfloat16 *w1b = nullptr, *w2b = nullptr;                     // conv B matrices [taps][NOUT][CK]
     __nv_bfloat16 *wd1_hi = nullptr, *wd1_lo = nullptr, *wd2_hi = nullptr, *wd2_lo = nullptr;
-    CUtensorMap m_w1b, m_w2b, m_ah, m_al, m_w1h, m_w1l, m_hh, m_hl, m_w2h, m_w2l, m_w1h_half, m_w1l_half;
-    CUtensorMap m_w1h_half256, m_w1l_half256;                         // W halves of 128 rows: the wide (N = 256) pair kernel
-    CUtensorMap m_w1h_half176, m_w1l_half176;                         // W halves of 88 rows: the narrow (N = 176) pair kernel
-    bool narrow_ok = false;                                           // 9 column tiles of 176: 72 tiles up to 2048 rows
+    CUtensorMap m_w1b, m_w2b, m_ah, m_al, m_hh, m_hl, m_w2h, m_w2l;
+    // dense-1 W halves (BN / 2 rows) of the pair kernels by tile width; 176 and 192 only when 192 divides H
+    CUtensorMap m_w1h_half256, m_w1l_half256, m_w1h_half192, m_w1l_half192, m_w1h_half176, m_w1l_half176;
     int force_bn = 0;                                                 // MMW_FC1_BN = 176 / 192 / 256 (tests)
-    bool wide_ok = false;                                             // N = 192 is the default and N = 256 is available too
-    bool wide_always = false;                                         // MMW_FC1_WIDE=2 (tests)
     int pair_slots = 74;                                              // CTA pairs that run at once (SMs / 2)
     int dbg = 0;
-    int pair = 0;                                                     // dense 1 on CTA pairs (cta_group::2): stages, 0 = off
 };
 
 static std::string g_tc_err;
@@ -1087,10 +1049,8 @@ int pose_tc_init(PoseTc* t, const float* blob, const size_t* off, int D, int row
     if (make_map_2d(&im->m_w1b, im->w1b, (uint64_t)im->taps * 32, 16, 32, 16) ||
         make_map_2d(&im->m_w2b, im->w2b, (uint64_t)im->taps * 96, 16, 96, 16) ||
         make_map_2d(&im->m_ah, im->a_hi, R, im->Kf, 128, 64) || make_map_2d(&im->m_al, im->a_lo, R, im->Kf, 128, 64) ||
-        make_map_2d(&im->m_w1h, im->wd1_hi, im->H, im->Kf, im->H % 192 == 0 ? 192 : 256, 64) ||
-        make_map_2d(&im->m_w1l, im->wd1_lo, im->H, im->Kf, im->H % 192 == 0 ? 192 : 256, 64) ||
-        make_map_2d(&im->m_w1h_half, im->wd1_hi, im->H, im->Kf, im->H % 192 == 0 ? 96 : 128, 64) ||
-        make_map_2d(&im->m_w1l_half, im->wd1_lo, im->H, im->Kf, im->H % 192 == 0 ? 96 : 128, 64) ||
+        make_map_2d(&im->m_w1h_half256, im->wd1_hi, im->H, im->Kf, 128, 64) ||
+        make_map_2d(&im->m_w1l_half256, im->wd1_lo, im->H, im->Kf, 128, 64) ||
         make_map_2d(&im->m_hh, im->h_hi, R, im->H, 128, 64) || make_map_2d(&im->m_hl, im->h_lo, R, im->H, 128, 64) ||
         make_map_2d(&im->m_w2h, im->wd2_hi, 64, im->H, 64, 64) || make_map_2d(&im->m_w2l, im->wd2_lo, 64, im->H, 64, 64))
         return -1;
@@ -1106,25 +1066,17 @@ int pose_tc_init(PoseTc* t, const float* blob, const size_t* off, int D, int row
     set_smem((const void*)conv_slab_kernel<32, 64, 1, 3>, conv_smem_bytes_tc<32, 64>(27));
     set_smem((const void*)conv_slab_kernel<16, 32, 0, 1>, conv_smem_bytes_tc<16, 32>(9));
     set_smem((const void*)conv_slab_kernel<32, 64, 1, 1>, conv_smem_bytes_tc<32, 64>(9));
-    set_smem((const void*)conv_slab_kernel<16, 32, 0, 3, 1>, conv_smem_bytes_tc<16, 32>(9));
-    set_smem((const void*)conv_slab_kernel<32, 64, 1, 3, 1>, conv_smem_bytes_tc<32, 64>(9));
-    set_smem((const void*)gemm_tc_kernel<256, 2, 0>, gemm_smem_bytes<256, 2>());
-    set_smem((const void*)gemm_tc_kernel<192, 2, 0>, gemm_smem_bytes<192, 2>());
-    {
-        // Dense 1 on CTA pairs: deepest pipeline the device accepts for a 2-CTA cluster of this kernel (asked of the
-        // driver, not assumed), else the single-CTA kernel.  MMW_FC1_PAIR=0 forces the single-CTA kernel (the
-        // comparison point of the measurement in DESIGN.md), MMW_FC1_PAIR=<n> caps the stage count.
-        const char* env = getenv("MMW_FC1_PAIR");
-        const int cap = env ? atoi(env) : 99;
-        const bool verbose = getenv("MMW_VERBOSE") != nullptr;
-        const bool n192 = im->H % 192 == 0;
-        auto clusters = [&](const void* fn, int bytes) -> int {
-            if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess ||
-                cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                     cudaSharedmemCarveoutMaxShared) != cudaSuccess) {
-                cudaGetLastError();
-                return -1;
-            }
+    set_smem((const void*)gemm_tc_kernel<64, 4>, gemm_smem_bytes<64, 4>());
+    set_smem((const void*)gemm_tc_kernel<64, 4, 4>, gemm_smem_bytes<64, 4>());
+    if (e != cudaSuccess) { g_tc_err = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e); return -1; }
+    // Dense 1 on CTA pairs with three pipeline stages (four were measured too: no faster than three, the main loop
+    // already runs at the tensor-core floor).  Whether a 2-CTA cluster of every tile width the launcher may pick can
+    // run on this device is asked of the driver, not assumed (on a B200 all three fit: <= 201 KB of shared memory);
+    // a kernel that cannot be scheduled fails the initialisation.
+    auto pair_fits = [&](const void* fn, int bytes, int bn) -> bool {
+        set_smem(fn, bytes);
+        int n = 0;
+        if (e == cudaSuccess) {
             cudaLaunchConfig_t cfg{};
             cfg.gridDim = dim3(2, 8);
             cfg.blockDim = dim3(kGemmThreads);
@@ -1133,54 +1085,44 @@ int pose_tc_init(PoseTc* t, const float* blob, const size_t* off, int D, int row
             at[0].id = cudaLaunchAttributeClusterDimension;
             at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
             cfg.attrs = at; cfg.numAttrs = 1;
-            int n = 0;
-            if (cudaOccupancyMaxActiveClusters(&n, fn, &cfg) != cudaSuccess) { cudaGetLastError(); return -1; }
-            return n;
-        };
-        struct Cand { int stages; const void* fn; int bytes; };
-        // four stages were measured too: no faster than three (the main loop already runs at the tensor-core floor)
-        const Cand c192[] = {{3, (const void*)gemm_tc_pair_kernel<192, 3>, gemm_pair_smem_bytes<192, 3>()},
-                             {2, (const void*)gemm_tc_pair_kernel<192, 2>, gemm_pair_smem_bytes<192, 2>()}};
-        const Cand c256[] = {{3, (const void*)gemm_tc_pair_kernel<256, 3>, gemm_pair_smem_bytes<256, 3>()},
-                             {2, (const void*)gemm_tc_pair_kernel<256, 2>, gemm_pair_smem_bytes<256, 2>()}};
-        im->pair = 0;
-        for (const Cand& c : (n192 ? c192 : c256)) {
-            if (c.stages > cap) continue;
-            const int n = clusters(c.fn, c.bytes);
-            if (verbose)
-                fprintf(stderr, "[mmw] dense 1 pair kernel BN=%d stages=%d smem=%d: %d active clusters\n", n192 ? 192 : 256,
-                        c.stages, c.bytes, n);
-            if (n > 0) { im->pair = c.stages; break; }
+            e = cudaOccupancyMaxActiveClusters(&n, fn, &cfg);
         }
-        if (verbose) fprintf(stderr, "[mmw] dense 1: %s\n", im->pair ? "cta_group::2 pair kernel" : "single-CTA kernel");
-        // 256 x 192 tiles need ceil(rows / 256) * 8 CTA pairs: one wave up to 2304 rows (74 pairs on 148 SMs), two
-        // beyond -- twice the time for one row more.  256 x 256 tiles (6 per row block, 4/3 of the time each) stay in one
-        // wave up to 3072 rows; the launcher takes whichever is cheaper for the row count of an earlier frame.
-        {
-            int dev = 0, sms = 148;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            im->pair_slots = sms / 2;
+        const std::string name = "gemm_tc_pair_kernel<" + std::to_string(bn) + ",3>";
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();     // not left behind for the next launch check to report
+            g_tc_err = name + ": " + cudaGetErrorString(e);
+            return false;
         }
-        const char* wenv = getenv("MMW_FC1_WIDE");
-        if (n192 && im->pair == 3 && im->H % 256 == 0 && !(wenv && atoi(wenv) == 0) &&
-            clusters((const void*)gemm_tc_pair_kernel<256, 3>, gemm_pair_smem_bytes<256, 3>()) > 0 &&
-            make_map_2d(&im->m_w1h_half256, im->wd1_hi, im->H, im->Kf, 128, 64) == 0 &&
-            make_map_2d(&im->m_w1l_half256, im->wd1_lo, im->H, im->Kf, 128, 64) == 0)
-        {
-            im->wide_ok = true;
-            im->wide_always = wenv && atoi(wenv) == 2;
+        if (n < 1) {
+            g_tc_err = name + ": a cluster of two CTAs with " + std::to_string(bytes) +
+                       " bytes of shared memory each cannot be scheduled on this device";
+            return false;
         }
-        if (n192 && im->pair == 3 && !(wenv && atoi(wenv) == 0) &&
-            clusters((const void*)gemm_tc_pair_kernel<176, 3>, gemm_pair_smem_bytes<176, 3>()) > 0 &&
-            make_map_2d(&im->m_w1h_half176, im->wd1_hi, im->H, im->Kf, 88, 64) == 0 &&
-            make_map_2d(&im->m_w1l_half176, im->wd1_lo, im->H, im->Kf, 88, 64) == 0)
-            im->narrow_ok = true;
-        { const char* benv = getenv("MMW_FC1_BN"); im->force_bn = benv ? atoi(benv) : 0; }
+        return true;
+    };
+    // 256 x 192 tiles need ceil(rows / 256) * 8 CTA pairs: one wave up to 2304 rows (74 pairs on 148 SMs), two
+    // beyond -- twice the time for one row more.  256 x 256 tiles (6 per row block, 4/3 of the time each) stay in one
+    // wave up to 3072 rows, 256 x 176 tiles (9 per row block, the last one 128 wide) up to 2048 rows at 11/12 of the
+    // time; the launcher takes whichever is cheapest for the row count of an earlier frame.  The 2-D net (H = 512)
+    // always uses 256-wide tiles.
+    if (!pair_fits((const void*)gemm_tc_pair_kernel<256, 3>, gemm_pair_smem_bytes<256, 3>(), 256)) return -1;
+    if (im->H % 192 == 0) {
+        if (!pair_fits((const void*)gemm_tc_pair_kernel<192, 3>, gemm_pair_smem_bytes<192, 3>(), 192) ||
+            !pair_fits((const void*)gemm_tc_pair_kernel<176, 3>, gemm_pair_smem_bytes<176, 3>(), 176))
+            return -1;
+        if (make_map_2d(&im->m_w1h_half192, im->wd1_hi, im->H, im->Kf, 96, 64) ||
+            make_map_2d(&im->m_w1l_half192, im->wd1_lo, im->H, im->Kf, 96, 64) ||
+            make_map_2d(&im->m_w1h_half176, im->wd1_hi, im->H, im->Kf, 88, 64) ||
+            make_map_2d(&im->m_w1l_half176, im->wd1_lo, im->H, im->Kf, 88, 64))
+            return -1;
     }
-    set_smem((const void*)gemm_tc_kernel<64, 4, 1>, gemm_smem_bytes<64, 4>());
-    set_smem((const void*)gemm_tc_kernel<64, 4, 1, 4>, gemm_smem_bytes<64, 4>());
-    if (e != cudaSuccess) { g_tc_err = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e); return -1; }
+    {
+        int dev = 0, sms = 148;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        im->pair_slots = sms / 2;
+    }
+    { const char* benv = getenv("MMW_FC1_BN"); im->force_bn = benv ? atoi(benv) : 0; }
     t->ready = true;
     return 0;
 }
@@ -1206,27 +1148,20 @@ int pose_tc_pack_input(PoseTc* t, const float* feats, const int* n_rows, cudaStr
 int pose_tc_conv(PoseTc* t, const PoseTcRun& r, cudaStream_t st, int* n_launches, int buf) {
     TcImpl* im = reinterpret_cast<TcImpl*>(t->impl);
     if (!im || !t->ready) { g_tc_err = "tensor-core path not initialised"; return -1; }
-    // 2-D net: three samples per slab unless MMW_CONV2D_TRIPLE=0 (the comparison point)
-    static const bool triple = [] { const char* e = getenv("MMW_CONV2D_TRIPLE"); return !(e && atoi(e) == 0); }();
-    ConvTcArgs c1{r.n_rows, r.b1, nullptr, nullptr, buf ? im->in_p2 : im->in_p, im->act1_p, nullptr, im->D, im->taps, im->dbg};
+    // the 2-D net (KD = 1) runs three samples per slab
+    ConvTcArgs c1{r.n_rows, r.b1, nullptr, nullptr, buf ? im->in_p2 : im->in_p, im->act1_p, nullptr, im->dbg};
     const dim3 one(1, 1, 1);
     cudaError_t le;
     if (im->D == 3)
         le = launch_pdl(conv_slab_kernel<16, 32, 0, 3>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<16, 32>(27), st, one,
                         im->m_w1b, c1);
-    else if (triple)
-        le = launch_pdl(conv_slab_kernel<16, 32, 0, 3, 1>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<16, 32>(9), st, one,
-                        im->m_w1b, c1);
     else
         le = launch_pdl(conv_slab_kernel<16, 32, 0, 1>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<16, 32>(9), st, one,
                         im->m_w1b, c1);
     if (le != cudaSuccess) { g_tc_err = std::string("conv_slab_kernel<conv1>: ") + cudaGetErrorString(le); return -1; }
-    ConvTcArgs c2{r.n_rows, r.b2, r.bn1_scale, r.bn1_shift, im->act1_p, im->a_hi, im->a_lo, im->D, im->taps, im->dbg};
+    ConvTcArgs c2{r.n_rows, r.b2, r.bn1_scale, r.bn1_shift, im->act1_p, im->a_hi, im->a_lo, im->dbg};
     if (im->D == 3)
         le = launch_pdl(conv_slab_kernel<32, 64, 1, 3>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<32, 64>(27), st, one,
-                        im->m_w2b, c2);
-    else if (triple)
-        le = launch_pdl(conv_slab_kernel<32, 64, 1, 3, 1>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<32, 64>(9), st, one,
                         im->m_w2b, c2);
     else
         le = launch_pdl(conv_slab_kernel<32, 64, 1, 1>, dim3(148), dim3(kSlabThreads), conv_smem_bytes_tc<32, 64>(9), st, one,
@@ -1241,51 +1176,32 @@ int pose_tc_fc1(PoseTc* t, const PoseTcRun& r, int max_rows, cudaStream_t st, in
     if (!im || !t->ready) { g_tc_err = "tensor-core path not initialised"; return -1; }
     GemmTcArgs g{r.n_rows, r.bd1, r.bn2_scale, r.bn2_shift, im->h_hi, im->h_lo, nullptr, nullptr, nullptr, nullptr,
                  im->Kf, im->H, r.tcap, im->dbg};
-    // 128 x 192 tiles when they divide N: 1536/192 = 8 column tiles, i.e. 120 CTAs for ~1900 rows instead of 90
-    // CTAs of 128 x 256 on 148 SMs (one wave either way, 25 % less work per CTA)
-    cudaError_t le;
-    if (im->pair) {
-        const bool n192 = im->H % 192 == 0;
-        const dim3 grid((((max_rows + 127) / 128) + 1) & ~1, im->H / (n192 ? 192 : 256)), blk(kGemmThreads), cl(2, 1, 1);
-        bool wide = im->wide_ok && im->wide_always, narrow = false;
-        if (!wide && rows_hint > 0 && n192) {
+    int bn = 256;
+    if (im->H % 192 == 0) {
+        bn = 192;
+        if (rows_hint > 0) {
             // cost of a launch = waves of CTA pairs x tile width; 176 (9 column tiles), 192 (8) or 256 (6) columns
             // (the hint is a frame or two old and the row count drifts by a few rows per frame: plan for 48 more -- one row
             // past a tile-count edge costs a whole second wave)
             const int mt = (rows_hint + 48 + 255) / 256, P = im->pair_slots;
-            auto cost = [&](int bn) { return ((mt * ((im->H + bn - 1) / bn) + P - 1) / P) * bn; };
+            auto cost = [&](int w) { return ((mt * ((im->H + w - 1) / w) + P - 1) / P) * w; };
             int best = cost(192);
-            if (im->wide_ok && cost(256) < best) { best = cost(256); wide = true; }
-            if (im->narrow_ok && cost(176) < best) { wide = false; narrow = true; }
+            if (cost(256) < best) { best = cost(256); bn = 256; }
+            if (cost(176) < best) bn = 176;
         }
-        if (im->force_bn == 256 && im->wide_ok) { wide = true; narrow = false; }
-        if (im->force_bn == 176 && im->narrow_ok) { wide = false; narrow = true; }
-        if (im->force_bn == 192) wide = narrow = false;
-        if (narrow)
-            le = launch_pdl(gemm_tc_pair_kernel<176, 3>, dim3(grid.x, (im->H + 175) / 176), blk, gemm_pair_smem_bytes<176, 3>(),
-                            st, cl, im->m_ah, im->m_al, im->m_w1h_half176, im->m_w1l_half176, g);
-        else if (wide)
-            le = launch_pdl(gemm_tc_pair_kernel<256, 3>, dim3(grid.x, im->H / 256), blk, gemm_pair_smem_bytes<256, 3>(), st,
-                            cl, im->m_ah, im->m_al, im->m_w1h_half256, im->m_w1l_half256, g);
-        else if (n192 && im->pair == 3)
-            le = launch_pdl(gemm_tc_pair_kernel<192, 3>, grid, blk, gemm_pair_smem_bytes<192, 3>(), st, cl, im->m_ah,
-                            im->m_al, im->m_w1h_half, im->m_w1l_half, g);
-        else if (n192)
-            le = launch_pdl(gemm_tc_pair_kernel<192, 2>, grid, blk, gemm_pair_smem_bytes<192, 2>(), st, cl, im->m_ah,
-                            im->m_al, im->m_w1h_half, im->m_w1l_half, g);
-        else if (im->pair == 3)
-            le = launch_pdl(gemm_tc_pair_kernel<256, 3>, grid, blk, gemm_pair_smem_bytes<256, 3>(), st, cl, im->m_ah,
-                            im->m_al, im->m_w1h_half, im->m_w1l_half, g);
-        else
-            le = launch_pdl(gemm_tc_pair_kernel<256, 2>, grid, blk, gemm_pair_smem_bytes<256, 2>(), st, cl, im->m_ah,
-                            im->m_al, im->m_w1h_half, im->m_w1l_half, g);
-    } else if (im->H % 192 == 0) {
-        le = launch_pdl(gemm_tc_kernel<192, 2, 0>, dim3(im->H / 192, (max_rows + 127) / 128), dim3(kGemmThreads),
-                        gemm_smem_bytes<192, 2>(), st, dim3(1, 1, 1), im->m_ah, im->m_al, im->m_w1h, im->m_w1l, g);
-    } else {
-        le = launch_pdl(gemm_tc_kernel<256, 2, 0>, dim3(im->H / 256, (max_rows + 127) / 128), dim3(kGemmThreads),
-                        gemm_smem_bytes<256, 2>(), st, dim3(1, 1, 1), im->m_ah, im->m_al, im->m_w1h, im->m_w1l, g);
+        if (im->force_bn == 176 || im->force_bn == 192 || im->force_bn == 256) bn = im->force_bn;
     }
+    const dim3 grid((((max_rows + 127) / 128) + 1) & ~1, (im->H + bn - 1) / bn), blk(kGemmThreads), cl(2, 1, 1);
+    cudaError_t le;
+    if (bn == 176)
+        le = launch_pdl(gemm_tc_pair_kernel<176, 3>, grid, blk, gemm_pair_smem_bytes<176, 3>(), st, cl, im->m_ah, im->m_al,
+                        im->m_w1h_half176, im->m_w1l_half176, g);
+    else if (bn == 192)
+        le = launch_pdl(gemm_tc_pair_kernel<192, 3>, grid, blk, gemm_pair_smem_bytes<192, 3>(), st, cl, im->m_ah, im->m_al,
+                        im->m_w1h_half192, im->m_w1l_half192, g);
+    else
+        le = launch_pdl(gemm_tc_pair_kernel<256, 3>, grid, blk, gemm_pair_smem_bytes<256, 3>(), st, cl, im->m_ah, im->m_al,
+                        im->m_w1h_half256, im->m_w1l_half256, g);
     if (le != cudaSuccess) { g_tc_err = std::string("dense 1 launch: ") + cudaGetErrorString(le); return -1; }
     if (n_launches) *n_launches = 1;
     return 0;
@@ -1296,15 +1212,13 @@ int pose_tc_fc2(PoseTc* t, const PoseTcRun& r, int max_rows, cudaStream_t st, in
     if (!im || !t->ready) { g_tc_err = "tensor-core path not initialised"; return -1; }
     GemmTcArgs g{r.n_rows, r.bd2, nullptr, nullptr, nullptr, nullptr, r.out, r.keypoints, r.row_scene, r.row_slot,
                  im->H, 64, r.tcap, im->dbg, r.results, r.row_track, r.fade};
-    // K split over a cluster of 4 CTAs per row tile whenever the K blocks divide (1536 / 64 = 24, 512 / 64 = 8);
-    // MMW_FC2_SPLIT=0 keeps the single-CTA kernel (the comparison point)
-    static const bool split = [] { const char* e = getenv("MMW_FC2_SPLIT"); return !e || atoi(e) != 0; }();
+    // K split over a cluster of 4 CTAs per row tile whenever the K blocks divide (1536 / 64 = 24, 512 / 64 = 8)
     cudaError_t le;
-    if (split && (im->H / kBK) % 4 == 0 && (max_rows + 127) / 128 <= 128)      // large batches fill the SMs without it
-        le = launch_pdl(gemm_tc_kernel<64, 4, 1, 4>, dim3(4, (max_rows + 127) / 128), dim3(kGemmThreads),
+    if ((im->H / kBK) % 4 == 0 && (max_rows + 127) / 128 <= 128)      // large batches fill the SMs without it
+        le = launch_pdl(gemm_tc_kernel<64, 4, 4>, dim3(4, (max_rows + 127) / 128), dim3(kGemmThreads),
                         gemm_smem_bytes<64, 4>(), st, dim3(4, 1, 1), im->m_hh, im->m_hl, im->m_w2h, im->m_w2l, g);
     else
-        le = launch_pdl(gemm_tc_kernel<64, 4, 1>, dim3(1, (max_rows + 127) / 128), dim3(kGemmThreads),
+        le = launch_pdl(gemm_tc_kernel<64, 4>, dim3(1, (max_rows + 127) / 128), dim3(kGemmThreads),
                         gemm_smem_bytes<64, 4>(), st, dim3(1, 1, 1), im->m_hh, im->m_hl, im->m_w2h, im->m_w2l, g);
     if (le != cudaSuccess) { g_tc_err = std::string("dense 2 launch: ") + cudaGetErrorString(le); return -1; }
     if (n_launches) *n_launches = 1;

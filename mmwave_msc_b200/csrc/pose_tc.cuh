@@ -35,8 +35,8 @@ __nv_bfloat16* pose_tc_input(PoseTc* tc, int buf = 0);   // buf 0 / 1: the two i
 // fp32 feature maps [rows][D*64][5] -> packed input (used by the stage-level mmw_pose entry point).
 int pose_tc_pack_input(PoseTc* tc, const float* feats, const int* n_rows, cudaStream_t st);
 int pose_tc_conv(PoseTc* tc, const PoseTcRun& r, cudaStream_t st, int* n_launches, int buf = 0);
-// rows_hint: row count of an earlier frame (0 = unknown): picks 256 x 192 or 256 x 256 tiles, whichever needs fewer
-// waves of CTA pairs -- speed only, the two kernels give the same bits
+// rows_hint: row count of an earlier frame (0 = unknown): picks 256 x 176, 256 x 192 or 256 x 256 tiles, whichever
+// costs the least waves of CTA pairs times tile width -- speed only, the three kernels give the same bits
 int pose_tc_fc1(PoseTc* tc, const PoseTcRun& r, int max_rows, cudaStream_t st, int* n_launches, int rows_hint = 0);
 int pose_tc_fc2(PoseTc* tc, const PoseTcRun& r, int max_rows, cudaStream_t st, int* n_launches);
 void pose_tc_free(PoseTc* tc);

@@ -28,12 +28,8 @@
 
 namespace mmw {
 
-#ifndef MMW_KTB
-#define MMW_KTB 1
-#endif
 constexpr int kTile = 2 * kStepThreads;          // points per tile: two per thread
 constexpr int kChunks = kTile / 32;              // warp chunks of 32 consecutive points in a tile
-constexpr int kTB = MMW_KTB;                           // tracks per batch of the element-parallel track phases
 constexpr int kLw = 7;                           // doubles per list row: d0..d5 (w - H x of the point's track), x
 constexpr int kBw = 72;                          // doubles of per-track scratch B
 // inside B from the gate matrices to the association results: gate form (kGateWords = 28) | new N_est | minima of
@@ -381,10 +377,8 @@ __device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, int s, 
         }                                                                                \
     } while (0)
 
-#ifndef MMW_STEP_MINBLOCKS
-#define MMW_STEP_MINBLOCKS 7
-#endif
-__global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(const __grid_constant__ StepArgs a) {
+constexpr int kStepMinBlocks = 7;                // resident scene CTAs per SM the register budget is sized for
+__global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(const __grid_constant__ StepArgs a) {
     const bool dbg_clocks = a.phase_cycles != nullptr;
     long long phase_t0 = dbg_clocks ? clock64() : 0;
     const long long kernel_t0 = phase_t0;
@@ -460,40 +454,26 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
     PHASE_MARK(1);
 
     // ---- 1. predict (Tracking.py:591-596, Q9) and gate matrices (Tracking.py:545-551) -----------------------
-    // Element-parallel, kTB tracks per batch: every thread computes its element of F P F' + Q for all tracks of
-    // the batch from the old P (independent chains, their loads overlap), one barrier, then the stores: P, x = F x,
-    // H x, and the gate matrix C = P[:6,:6] + Rm + G (get_Rm 361-370) into the track's B block.
-    for (int j0 = 0; j0 < T0; j0 += kTB) {
-        double pv[kTB], xv[kTB];
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            const int j = j0 + u;
-            pv[u] = 0.0; xv[u] = 0.0;
-            if (j < T0) {
-                const TrackRec& t = tr[j];
-                const double dte = t.lifetime + dt;
-                if (tid < 81) pv[u] = kf_predict_elem(t.P, dte, c.q_var, el);
-                if (tid < 9) xv[u] = kf_predict_x(t.x, dte, tid);
-            }
-        }
+    // Element-parallel, one track at a time: every thread computes its element of F P F' + Q from the old P, one
+    // barrier, then the stores: P, x = F x, H x, and the gate matrix C = P[:6,:6] + Rm + G (get_Rm 361-370) into the
+    // track's B block.
+    for (int j = 0; j < T0; ++j) {
+        TrackRec& t = tr[j];
+        double pv = 0.0, xv = 0.0;
+        const double dte = t.lifetime + dt;
+        if (tid < 81) pv = kf_predict_elem(t.P, dte, c.q_var, el);
+        if (tid < 9) xv = kf_predict_x(t.x, dte, tid);
         __syncthreads();
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            const int j = j0 + u;
-            if (j < T0) {
-                TrackRec& t = tr[j];
-                if (tid < 81) {
-                    t.P[tid] = pv[u];
-                    if (el.i9 < 6 && el.j9 < 6) {
-                        double v = pv[u];
-                        if (el.i9 == el.j9) { const double h = t.spread[el.i9] / 2; v += h * h; }
-                        Bm[j * kBw + kMin + el.i9 * 6 + el.j9] = v + t.G[el.i9 * 6 + el.j9];
-                    }
-                }
-                if (tid < 9) t.x[tid] = xv[u];
-                if (tid < 6) Bm[j * kBw + kHx + tid] = xv[u];
+        if (tid < 81) {
+            t.P[tid] = pv;
+            if (el.i9 < 6 && el.j9 < 6) {
+                double v = pv;
+                if (el.i9 == el.j9) { const double h = t.spread[el.i9] / 2; v += h * h; }
+                Bm[j * kBw + kMin + el.i9 * 6 + el.j9] = v + t.G[el.i9 * 6 + el.j9];
             }
         }
+        if (tid < 9) t.x[tid] = xv;
+        if (tid < 6) Bm[j * kBw + kHx + tid] = xv;
     }
     __syncthreads();
     PHASE_MARK(2);
@@ -567,14 +547,6 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
         {
             double best0 = INFINITY, best1 = INFINITY;
             int bj0 = -1, bj1 = -1;
-#ifndef MMW_GATE_SEQ
-            for (int j = 0; j < T0; ++j) {
-                const double* gp = Bm + j * kBw + kGp;
-                const double d0 = gate_score(gp, w[0]), d1 = gate_score(gp, w[1]);
-                if (d0 < c.gate && d0 < best0) { best0 = d0; bj0 = j; }
-                if (d1 < c.gate && d1 < best1) { best1 = d1; bj1 = j; }
-            }
-#else
             if (keep[0])
                 for (int j = 0; j < T0; ++j) {
                     const double d0 = gate_score(Bm + j * kBw + kGp, w[0]);
@@ -585,7 +557,6 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
                     const double d1 = gate_score(Bm + j * kBw + kGp, w[1]);
                     if (d1 < c.gate && d1 < best1) { best1 = d1; bj1 = j; }
                 }
-#endif
             grp[0] = keep[0] ? (bj0 < 0 ? T0 : bj0) : 255;
             grp[1] = keep[1] ? (bj1 < 0 ? T0 : bj1) : 255;
             if (keep[0]) a.assoc_out[off + pos[0]] = bj0;
@@ -761,83 +732,67 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
     PHASE_MARK(7);
 
     // ---- 3. per-track association results (Tracking.py:648-653, 314-341) ------------------------------------
-    // Roles by thread (the same for every track, kTB tracks per batch: values first, stores after):
+    // Roles by thread (the same for every track, one track at a time: values first, stores after):
     //   tid < 36      group dispersion entry (_estimate_group_disp_matrix 292-297)
     //   64 <= tid < 70  centroid, extrema, spread of dimension tid - 64 (_estimate_measurement_spread 246-268)
     //   tid == 96     ring bookkeeping, lifetime, point count, status, N_est (_estimate_point_num 232-244)
     int ring_rows = 0;
-    for (int j0 = 0; j0 < T0; j0 += kTB) {
-        double v0[kTB], v1[kTB], v2[kTB], v3[kTB];
-        int nn[kTB];
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            const int j = j0 + u;
-            nn[u] = 0; v0[u] = v1[u] = v2[u] = v3[u] = 0.0;
-            if (j >= T0) continue;
-            const TrackRec& t = tr[j];
-            const int n = misc[kBaseG + (ntiles & 1) * 32 + j];
-            nn[u] = n;
-            ring_rows += n < kFeatPts ? n : kFeatPts;
-            if (n == 0) continue;
-            const double* tv = Bm + j * kBw;
-            const double dn = (double)n;
-            if (tid < 36) {
-                double n_est;
-                if (c.enable_est) n_est = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
-                else n_est = (double)(n > c.est_pointnum ? n : c.est_pointnum);
-                int r = el.i6, q = el.a6;
-                if (r > q) { const int tmp = r; r = q; q = tmp; }
-                const int p = r * 6 - (r * (r - 1)) / 2 + (q - r);
-                const double rn = 1.0 / dn;
-                const double dv = tv[kProd + p] * rn - (tv[kSum + r] * rn) * (tv[kSum + q] * rn);
-                const double al = dn / n_est;
-                v0[u] = (1 - al) * t.G[tid] + al * dv;
-            } else if (tid >= 64 && tid < 70) {
-                const int m = tid - 64;
-                const double mnv = tv[kMin + m], mxv = tv[kMax + m];
-                // centroid[0]: the x column is a sum of lattice values, exact in any order, so this is numpy's mean to the
-                // bit -- the pose features sort on x - centroid[0] against zero pads (Utils.py:505-514)
-                v0[u] = m == 0 ? tv[kSumX] / dn : tv[kHx + m] + tv[kSum + m] / dn;
-                v1[u] = mnv;
-                v2[u] = mxv;
-                double spread = mxv - mnv;
-                if (n != 1) spread = spread * (double)(n + 1) / (double)(n - 1);
-                spread = fmin(2 * c.spread_lim[m], spread);
-                spread = fmax(c.spread_lim[m], spread);
-                v3[u] = spread > t.spread[m] ? spread : (1.0 - c.a_spr) * t.spread[m] + c.a_spr * spread;
-            } else if (tid == 96) {
-                if (c.enable_est) v0[u] = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
-                else v0[u] = (double)(n > c.est_pointnum ? n : c.est_pointnum);
-                const double c3 = tv[kHx + 3] + tv[kSum + 3] / dn, c4 = tv[kHx + 4] + tv[kSum + 4] / dn,
-                             c5 = tv[kHx + 5] + tv[kSum + 5] / dn;
-                v1[u] = sqrt(c3 * c3 + c4 * c4 + c5 * c5) < c.vel_thres ? 1.0 : 0.0;
-            }
+    for (int j = 0; j < T0; ++j) {
+        TrackRec& t = tr[j];
+        const int n = misc[kBaseG + (ntiles & 1) * 32 + j];
+        ring_rows += n < kFeatPts ? n : kFeatPts;
+        if (n == 0) {
+            if (tid == 96) t.lifetime += dt;                     // update_lifetime(dt) (400-407)
+            continue;
         }
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            const int j = j0 + u;
-            if (j >= T0) continue;
-            TrackRec& t = tr[j];
-            const int n = nn[u];
-            if (n == 0) {
-                if (tid == 96) t.lifetime += dt;                 // update_lifetime(dt) (400-407)
-                continue;
-            }
-            if (tid < 36) {
-                t.G[tid] = v0[u];
-            } else if (tid >= 64 && tid < 70) {
-                const int m = tid - 64;
-                t.centroid[m] = v0[u]; t.minv[m] = v1[u]; t.maxv[m] = v2[u]; t.spread[m] = v3[u];
-            } else if (tid == 96) {
-                const int phys = t.ring_n >= c.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, c.ring_size);
-                if (t.ring_n >= c.ring_size) t.ring_head = ring_wrap(t.ring_head + 1, c.ring_size);
-                else t.ring_n += 1;
-                t.ring_cnt[phys] = n < kFeatPts ? n : kFeatPts;
-                t.lifetime = 0.0;
-                t.point_num = n;
-                t.is_static = v1[u] != 0.0 ? 1 : 0;
-                t.n_est = v0[u];         // (the dispersion threads computed their own copy from the old value above)
-            }
+        const double* tv = Bm + j * kBw;
+        const double dn = (double)n;
+        double v0 = 0.0, v1 = 0.0, v2 = 0.0, v3 = 0.0;
+        if (tid < 36) {
+            double n_est;
+            if (c.enable_est) n_est = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
+            else n_est = (double)(n > c.est_pointnum ? n : c.est_pointnum);
+            int r = el.i6, q = el.a6;
+            if (r > q) { const int tmp = r; r = q; q = tmp; }
+            const int p = r * 6 - (r * (r - 1)) / 2 + (q - r);
+            const double rn = 1.0 / dn;
+            const double dv = tv[kProd + p] * rn - (tv[kSum + r] * rn) * (tv[kSum + q] * rn);
+            const double al = dn / n_est;
+            v0 = (1 - al) * t.G[tid] + al * dv;
+        } else if (tid >= 64 && tid < 70) {
+            const int m = tid - 64;
+            const double mnv = tv[kMin + m], mxv = tv[kMax + m];
+            // centroid[0]: the x column is a sum of lattice values, exact in any order, so this is numpy's mean to the
+            // bit -- the pose features sort on x - centroid[0] against zero pads (Utils.py:505-514)
+            v0 = m == 0 ? tv[kSumX] / dn : tv[kHx + m] + tv[kSum + m] / dn;
+            v1 = mnv;
+            v2 = mxv;
+            double spread = mxv - mnv;
+            if (n != 1) spread = spread * (double)(n + 1) / (double)(n - 1);
+            spread = fmin(2 * c.spread_lim[m], spread);
+            spread = fmax(c.spread_lim[m], spread);
+            v3 = spread > t.spread[m] ? spread : (1.0 - c.a_spr) * t.spread[m] + c.a_spr * spread;
+        } else if (tid == 96) {
+            if (c.enable_est) v0 = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
+            else v0 = (double)(n > c.est_pointnum ? n : c.est_pointnum);
+            const double c3 = tv[kHx + 3] + tv[kSum + 3] / dn, c4 = tv[kHx + 4] + tv[kSum + 4] / dn,
+                         c5 = tv[kHx + 5] + tv[kSum + 5] / dn;
+            v1 = sqrt(c3 * c3 + c4 * c4 + c5 * c5) < c.vel_thres ? 1.0 : 0.0;
+        }
+        if (tid < 36) {
+            t.G[tid] = v0;
+        } else if (tid >= 64 && tid < 70) {
+            const int m = tid - 64;
+            t.centroid[m] = v0; t.minv[m] = v1; t.maxv[m] = v2; t.spread[m] = v3;
+        } else if (tid == 96) {
+            const int phys = t.ring_n >= c.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, c.ring_size);
+            if (t.ring_n >= c.ring_size) t.ring_head = ring_wrap(t.ring_head + 1, c.ring_size);
+            else t.ring_n += 1;
+            t.ring_cnt[phys] = n < kFeatPts ? n : kFeatPts;
+            t.lifetime = 0.0;
+            t.point_num = n;
+            t.is_static = v1 != 0.0 ? 1 : 0;
+            t.n_est = v0;         // (the dispersion threads computed their own copy from the old value above)
         }
     }
     {
@@ -884,7 +839,7 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
     PHASE_MARK(9);
 
     // ---- 5. update every surviving track (Tracking.py:598-603, 387-398; Q11-Q13) ----------------------------
-    // Element-parallel steps of the Joseph-form update (linalg.cuh), kTB tracks per batch and step.
+    // Element-parallel steps of the Joseph-form update (linalg.cuh), one track at a time in each step.
     // _get_Rc (299-312): Rm/N + ((N_est - N)/((N_est - 1) N)) * group_disp_est;  S = P[:6,:6] + Rc
     for (int k = 0; k < T1; ++k) {
         if (tid < 36) {
@@ -916,65 +871,30 @@ __global__ void __launch_bounds__(kStepThreads, MMW_STEP_MINBLOCKS) step_kernel(
         }
     }
     __syncthreads();
-    for (int k0 = 0; k0 < T1; k0 += kTB) {               // K = P[:, :6] S^-1
-        double kv[kTB];
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            kv[u] = 0.0;
-            if (k0 + u < T1 && tid < 54) {
-                const int j = misc[kOrder + k0 + u];
-                kv[u] = kf_update_K_elem(tr[j].P, Bm + j * kBw, el);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kTB; ++u)
-            if (k0 + u < T1 && tid < 54) KKm[misc[kOrder + k0 + u] * 108 + tid] = kv[u];
+    for (int k = 0; k < T1; ++k) {                       // K = P[:, :6] S^-1
+        const int j = misc[kOrder + k];
+        if (tid < 54) KKm[j * 108 + tid] = kf_update_K_elem(tr[j].P, Bm + j * kBw, el);
     }
     __syncthreads();
-    for (int k0 = 0; k0 < T1; k0 += kTB) {               // M1 = (I - K H) P, K Rc, x += K y
-        double mv[kTB], rv[kTB], xv[kTB];
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            mv[u] = rv[u] = xv[u] = 0.0;
-            if (k0 + u < T1) {
-                const int j = misc[kOrder + k0 + u];
-                const TrackRec& t = tr[j];
-                const double* K = KKm + j * 108;
-                if (tid < 81) mv[u] = kf_update_M1_elem(t.P, K, el);
-                if (tid < 54) rv[u] = kf_update_KR_elem(K, Bm + j * kBw + 36, el);
-                if (tid >= 96 && tid < 105) xv[u] = kf_update_x(t.x, t.centroid, K, tid - 96);
-            }
-        }
+    for (int k = 0; k < T1; ++k) {                       // M1 = (I - K H) P, K Rc, x += K y
+        const int j = misc[kOrder + k];
+        TrackRec& t = tr[j];
+        const double* K = KKm + j * 108;
+        double mv = 0.0, rv = 0.0, xv = 0.0;
+        if (tid < 81) mv = kf_update_M1_elem(t.P, K, el);
+        if (tid < 54) rv = kf_update_KR_elem(K, Bm + j * kBw + 36, el);
+        if (tid >= 96 && tid < 105) xv = kf_update_x(t.x, t.centroid, K, tid - 96);
         __syncwarp();                    // warp 3: every lane has read the old x
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            if (k0 + u < T1) {
-                const int j = misc[kOrder + k0 + u];
-                if (tid < 81) Am[j * 81 + tid] = mv[u];
-                if (tid < 54) KKm[j * 108 + 54 + tid] = rv[u];
-                if (tid >= 96 && tid < 105) tr[j].x[tid - 96] = xv[u];
-            }
-        }
+        if (tid < 81) Am[j * 81 + tid] = mv;
+        if (tid < 54) KKm[j * 108 + 54 + tid] = rv;
+        if (tid >= 96 && tid < 105) t.x[tid - 96] = xv;
     }
     __syncthreads();
-    for (int k0 = 0; k0 < T1; k0 += kTB) {               // P = M1 (I - K H)' + (K Rc) K'
-        double pv[kTB];
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            pv[u] = 0.0;
-            if (k0 + u < T1 && tid < 81) {
-                const int j = misc[kOrder + k0 + u];
-                pv[u] = kf_update_P_elem(Am + j * 81, KKm + j * 108, KKm + j * 108 + 54, el);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kTB; ++u) {
-            if (k0 + u < T1) {
-                TrackRec& t = tr[misc[kOrder + k0 + u]];
-                if (tid < 81) t.P[tid] = pv[u];
-                if (tid == 96) kf_update_nudge(t.x, t.centroid, t.lifetime == 0.0, c.nudge_thres, c.nudge_gain);
-            }
-        }
+    for (int k = 0; k < T1; ++k) {                       // P = M1 (I - K H)' + (K Rc) K'
+        const int j = misc[kOrder + k];
+        TrackRec& t = tr[j];
+        if (tid < 81) t.P[tid] = kf_update_P_elem(Am + j * 81, KKm + j * 108, KKm + j * 108 + 54, el);
+        if (tid == 96) kf_update_nudge(t.x, t.centroid, t.lifetime == 0.0, c.nudge_thres, c.nudge_gain);
     }
     PHASE_MARK(10);
 
