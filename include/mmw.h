@@ -25,7 +25,9 @@
 extern "C" {
 #endif
 
-#define MMW_ABI_VERSION 4
+/* 5: per-scene sensor table (mmw_scene_sensor, mmw_set/get_scene_sensors) and mmw_reset_scenes.  The state blob
+ * carries this number, so blobs written by version 4 are refused by mmw_state_restore. */
+#define MMW_ABI_VERSION 5
 
 typedef enum mmw_status {
     MMW_OK = 0,
@@ -35,7 +37,8 @@ typedef enum mmw_status {
     MMW_ERR_STATE = -4         /* call order (e.g. pose requested before weights were loaded) */
 } mmw_status;
 
-/* Mirror of the reference's constants.py (file:line = constants.py). */
+/* Mirror of the reference's constants.py (file:line = constants.py).  s_height, s_tilt_deg, z_max, xyz_q_format and
+ * doppler_res are the defaults of every scene's entry in the sensor table (mmw_scene_sensor). */
 typedef struct mmw_config {
     double s_height;               /* S_HEIGHT :41 */
     double s_tilt_deg;             /* S_TILT :42 */
@@ -92,9 +95,10 @@ typedef struct mmw_ctx mmw_ctx;
 #define MMW_STEP_POSE          0x1u   /* run estimate_posture after track (offline_main.py:60) */
 #define MMW_STEP_DEVICE_INPUT  0x2u   /* pts/offsets/dt are device pointers (already resident in HBM) */
 #define MMW_STEP_RECORD_LABELS 0x4u   /* keep the DBSCAN labels of this frame for mmw_get_labels */
-#define MMW_STEP_INPUT_I16     0x10u  /* pts is int16 [sum N, 5] = x, y, z (Q format mmw_config::xyz_q_format), dopplerIdx,
-                                         peakVal -- the sensor's own lattice, 10 bytes per point instead of 20; converted on
-                                         the device (exact: x = value / 2^Q, doppler = dopplerIdx * doppler_res in float64) */
+#define MMW_STEP_INPUT_I16     0x10u  /* pts is int16 [sum N, 5] = x, y, z (Q format: the scene's xyz_q_format, see
+                                         mmw_scene_sensor), dopplerIdx, peakVal -- the sensor's own lattice, 10 bytes per
+                                         point instead of 20; converted on the device (exact: x = value / 2^Q, doppler =
+                                         dopplerIdx * doppler_res in float64) */
 #define MMW_STEP_PIPELINE      0x8u   /* throughput mode (with MMW_STEP_POSE): the pose network of this frame runs on a
                                          second stream and overlaps the tracker of the NEXT frame -- keypoints never feed
                                          back into tracking (Tracking.py:705-734).  The frame's packed result records
@@ -118,18 +122,53 @@ int mmw_destroy(mmw_ctx* ctx);
 const char* mmw_last_error(void);
 int mmw_abi_version(void);
 
-/* Resets every scene to the state of a fresh TrackBuffer() + BatchedData() (Tracking.py:504-511, 38-41). */
+/* Resets every scene to the state of a fresh TrackBuffer() + BatchedData() (Tracking.py:504-511, 38-41).  The sensor
+ * table (mmw_scene_sensor) is configuration and stays as it is. */
 int mmw_reset(mmw_ctx* ctx);
 
-/* Changes mmw_config::doppler_res of a live context (takes effect with the next call; rows already in the rings are
- * re-read in the new unit, so change it only while they hold none -- e.g. before the first frame). */
+/* Changes mmw_config::doppler_res of a live context, the context's unit, and sets it as every scene's doppler_res
+ * (mmw_get_scene_sensors shows the result).  Takes effect with the next call; rows already in the rings are re-read in
+ * the new unit, so change it only while they hold none -- e.g. before the first frame. */
 int mmw_set_doppler_resolution(mmw_ctx* ctx, double doppler_res);
+
+/* ---- per-scene sensor table ----
+ * Each scene is one sensor installation or one recorded experiment, with its own mounting and radar profile.
+ * mmw_create fills every scene's entry from the mmw_config; a context that never changes the table behaves as if it
+ * had none.  A change takes effect with the next mmw_step, mmw_run_frames*, mmw_estimate_posture,
+ * mmw_pose_features_only or mmw_export_track0: it is queued on the context's stream behind all work already queued
+ * there.  Rings store raw sensor rows and world coordinates are recomputed from them, so the rows already in a scene's
+ * rings are re-read under the new parameters: change a scene's entry before its first frame, or together with
+ * mmw_reset_scenes.  The table is not part of the state blob (it is configuration, like mmw_config and the pose
+ * weights): a restored context continues with whatever table it has.  The stateless stage entry points
+ * (mmw_preprocess, mmw_dbscan) and mmw_decode_tlv keep using the values of the mmw_config. */
+typedef struct mmw_scene_sensor {
+    double s_height;               /* S_HEIGHT constants.py:41 */
+    double s_tilt_deg;             /* S_TILT constants.py:42 */
+    double z_max;                  /* scene bound on z', Utils.py:424 */
+    double doppler_res;            /* unit of the Doppler column, as mmw_config::doppler_res (must be > 0 here) */
+    int32_t xyz_q_format;          /* Q format of int16 rows (MMW_STEP_INPUT_I16), 0..15 */
+    int32_t reserved;
+} mmw_scene_sensor;
+
+/* Sets the entries of scenes first_scene .. first_scene + n - 1 from params[0 .. n-1].  All or nothing: a range out of
+ * bounds, a NULL pointer, a non-finite value, doppler_res <= 0 or a Q format outside 0..15 give MMW_ERR_INVALID and
+ * change no entry. */
+int mmw_set_scene_sensors(mmw_ctx* ctx, int first_scene, int n, const mmw_scene_sensor* params);
+/* Reads the entries of scenes first_scene .. first_scene + n - 1 into out[0 .. n-1] (reserved = 0). */
+int mmw_get_scene_sensors(mmw_ctx* ctx, int first_scene, int n, mmw_scene_sensor* out);
+
+/* mmw_reset restricted to the n listed scenes (e.g. a sensor slot handed to a new sensor): their scene record, track
+ * records, ring histograms, per-scene counters of the last step and pose-row count are cleared, so they continue like
+ * fresh scenes (track ids restart at 0).  Other scenes, the sensor table, the accumulated counters and results already
+ * packed for earlier frames are left alone.  Duplicate or out-of-range indices give MMW_ERR_INVALID and reset nothing. */
+int mmw_reset_scenes(mmw_ctx* ctx, const int32_t* scenes, int n);
 
 /* Checkpoint / resume of the tracker state of all scenes (track records, rings, keypoints, id counters): what a
  * replay needs to continue bit-identically in this or another context created with the same n_scenes,
  * max_points_per_frame, max_tracks and frames_batch (e.g. on another GPU).  mmw_state_size() = bytes of the blob;
  * dump / restore take a HOST buffer of at least that size and are synchronous.  The reference has no equivalent
- * (its state lives in Python objects for the length of the process); pose weights are not part of the blob. */
+ * (its state lives in Python objects for the length of the process); pose weights and the sensor table are not part
+ * of the blob, and a blob of another ABI version is refused. */
 size_t mmw_state_size(mmw_ctx* ctx);
 int mmw_state_dump(mmw_ctx* ctx, void* host_blob, size_t bytes);
 int mmw_state_restore(mmw_ctx* ctx, const void* host_blob, size_t bytes);

@@ -14,7 +14,7 @@ MMW_POSE_2D, MMW_POSE_3D = 0, 1
 STEP_POSE, STEP_DEVICE_INPUT, STEP_RECORD_LABELS, STEP_PIPELINE, STEP_INPUT_I16 = 0x1, 0x2, 0x4, 0x8, 0x10
 SCENE_POINT_OVERFLOW, SCENE_TRACK_OVERFLOW = 0x1, 0x2
 RESULT_FLOATS = 72
-ABI_VERSION = 4            # MMW_ABI_VERSION of include/mmw.h this binding was written against
+ABI_VERSION = 5            # MMW_ABI_VERSION of include/mmw.h this binding was written against
 KERNEL_NAMES = ["step", "pose_index", "pose_features", "conv", "fc1", "fc2", "dbscan_big", "k7"]
 
 
@@ -41,6 +41,21 @@ class Config(C.Structure):
         ("fade_size_max", C.c_double), ("fade_size_min", C.c_double), ("fade_weight", C.c_double),
         ("doppler_res", C.c_double),
     ]
+
+
+class SceneSensor(C.Structure):
+    """mmw_scene_sensor: one scene's sensor mounting and radar profile (see include/mmw.h)."""
+    _fields_ = [
+        ("s_height", C.c_double), ("s_tilt_deg", C.c_double), ("z_max", C.c_double), ("doppler_res", C.c_double),
+        ("xyz_q_format", C.c_int32), ("reserved", C.c_int32),
+    ]
+
+
+SCENE_SENSOR_DTYPE = np.dtype([
+    ("s_height", "<f8"), ("s_tilt_deg", "<f8"), ("z_max", "<f8"), ("doppler_res", "<f8"),
+    ("xyz_q_format", "<i4"), ("reserved", "<i4"),
+], align=False)
+assert SCENE_SENSOR_DTYPE.itemsize == C.sizeof(SceneSensor), (SCENE_SENSOR_DTYPE.itemsize, C.sizeof(SceneSensor))
 
 
 class TrackOut(C.Structure):
@@ -76,6 +91,9 @@ SIGNATURES = {
     "mmw_destroy": (C.c_int, [_p]),
     "mmw_reset": (C.c_int, [_p]),
     "mmw_set_doppler_resolution": (C.c_int, [_p, C.c_double]),
+    "mmw_set_scene_sensors": (C.c_int, [_p, C.c_int, C.c_int, _p]),
+    "mmw_get_scene_sensors": (C.c_int, [_p, C.c_int, C.c_int, _p]),
+    "mmw_reset_scenes": (C.c_int, [_p, _p, C.c_int]),
     "mmw_state_size": (C.c_size_t, [_p]),
     "mmw_state_dump": (C.c_int, [_p, _p, C.c_size_t]),
     "mmw_state_restore": (C.c_int, [_p, _p, C.c_size_t]),

@@ -89,9 +89,49 @@ class BatchedTracker:
 
     def set_doppler_resolution(self, doppler_res: float):
         """Unit of the Doppler column of the point rows: doppler [m/s] = row[3] * doppler_res in float64 on the device
-        (mmw_config::doppler_res).  With the sensor's dopplerResolutionMps the rows carry dopplerIdx."""
+        (mmw_config::doppler_res).  With the sensor's dopplerResolutionMps the rows carry dopplerIdx.  Sets the unit of
+        every scene."""
         _lib.check(self.lib.mmw_set_doppler_resolution(self._h, float(doppler_res)))
         self.cfg.doppler_res = float(doppler_res)
+
+    # -- per-scene sensors --------------------------------------------------------------------------
+    def _scene_index(self, scenes) -> np.ndarray:
+        if scenes is None or isinstance(scenes, slice):
+            return np.arange(self.S, dtype=np.int32)[scenes if scenes is not None else slice(None)]
+        return np.ascontiguousarray(np.atleast_1d(scenes), dtype=np.int32).reshape(-1)
+
+    def scene_sensors(self) -> np.ndarray:
+        """Every scene's sensor mounting and radar profile (mmw_scene_sensor): a (S,) structured array
+        (``_lib.SCENE_SENSOR_DTYPE``) with s_height, s_tilt_deg, z_max, doppler_res, xyz_q_format."""
+        out = np.zeros(self.S, _lib.SCENE_SENSOR_DTYPE)
+        _lib.check(self.lib.mmw_get_scene_sensors(self._h, 0, self.S, _lib.ptr(out)))
+        return out
+
+    def set_scene_sensors(self, s_height=None, s_tilt_deg=None, z_max=None, doppler_res=None, xyz_q_format=None,
+                          scenes=None):
+        """Sets the mounting and radar profile of the selected scenes (``scenes``: a slice or index array, default all).
+        Each value is a scalar or an array with one entry per selected scene; None keeps the current value.  Takes
+        effect with the next step.  Rows already in a scene's rings are re-read under the new values: change a scene
+        before its first frame, or together with ``reset_scenes``.  All or nothing: invalid values change no scene."""
+        idx = self._scene_index(scenes)
+        table = self.scene_sensors()
+        for name, v in (("s_height", s_height), ("s_tilt_deg", s_tilt_deg), ("z_max", z_max),
+                        ("doppler_res", doppler_res), ("xyz_q_format", xyz_q_format)):
+            if v is None:
+                continue
+            v = np.asarray(v)
+            if v.ndim and v.shape != idx.shape:
+                raise ValueError("%s: give a scalar or one value per selected scene" % name)
+            if name == "xyz_q_format" and not np.array_equal(v, np.round(v)):
+                raise ValueError("xyz_q_format must be an integer")
+            table[name][idx] = v
+        _lib.check(self.lib.mmw_set_scene_sensors(self._h, 0, self.S, _lib.ptr(table)))
+
+    def reset_scenes(self, scenes):
+        """``reset`` restricted to the selected scenes (a slice or index array): their tracks, rings and id counters
+        start afresh; other scenes and the sensor table are left alone."""
+        idx = self._scene_index(scenes)
+        _lib.check(self.lib.mmw_reset_scenes(self._h, _lib.ptr(idx), idx.size))
 
     @property
     def stream(self) -> int:

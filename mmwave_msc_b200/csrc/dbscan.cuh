@@ -76,6 +76,7 @@ struct NbExact {
 // (the FP64/XU pipe is what bounds this kernel, profiles/).
 struct NbScreened {
     const DevConfig& c;
+    const SensorRec& sr;              // the scene's mounting (shared memory)
     const float *Xf, *Yf, *Zf;        // shared memory, B floats each
     const float* frame[kRing];        // raw rows of the ring frames, oldest first (global)
     int start[kRing + 1];             // first fused index of each frame
@@ -86,7 +87,7 @@ struct NbScreened {
         const int f = (b >= start[1] ? 1 : 0) + (b >= start[2] ? 1 : 0);
         const float* r = rawc != nullptr ? rawc + (size_t)b * kRawCols : frame[f] + (size_t)(b - start[f]) * kRawCols;
         x = (double)r[0];
-        world_yz(c, (double)r[1], (double)r[2], y, z);
+        world_yz(sr, (double)r[1], (double)r[2], y, z);
     }
     // out of line on purpose: its float64 registers must not be live across the fp32 hot loop
     __device__ __noinline__ bool exact(int b, int q) const {

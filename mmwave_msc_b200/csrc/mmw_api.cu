@@ -39,6 +39,9 @@ struct mmw_ctx {
     DevConfig dc;
     int device = 0, S = 0, ncap = 0, tcap = 0;
     cudaStream_t stream = nullptr;
+    // sensor table: each scene's mounting and radar profile as set (host) and as the kernels read it (device, [S])
+    std::vector<mmw_scene_sensor> sensors;
+    SensorRec* d_sensors = nullptr;
     // resident state
     TrackRec* d_tracks = nullptr;
     SceneRec* d_scenes = nullptr;
@@ -138,12 +141,33 @@ static void prof_mark(mmw_ctx* x, int next_kernel) {
     x->marks.emplace_back(e, next_kernel);
 }
 
+// The kernels' form of one sensor-table entry.  Every entry, the context default included, is built here: the transform
+// is bit-exact to numpy's only while std::cos / std::sin of deg * (pi / 180) agree with np.cos / np.sin(np.radians(deg)).
+static SensorRec sensor_rec(const mmw_scene_sensor& p) {
+    SensorRec r{};
+    const double ang = p.s_tilt_deg * (M_PI / 180.0);      // numpy.radians
+    r.cos_t = std::cos(ang);
+    r.sin_t = std::sin(ang);
+    r.s_height = p.s_height;
+    r.z_max = p.z_max;
+    r.doppler_res = p.doppler_res;
+    r.xyz_scale = (float)std::ldexp(1.0, -(p.xyz_q_format));
+    return r;
+}
+
+// The sensor-table entry every scene starts with: the mmw_config's values (doppler_res 0 is read as 1.0).
+static mmw_scene_sensor config_sensor(const mmw_config& c) {
+    mmw_scene_sensor p{};
+    p.s_height = c.s_height;
+    p.s_tilt_deg = c.s_tilt_deg;
+    p.z_max = c.z_max;
+    p.doppler_res = c.doppler_res != 0.0 ? c.doppler_res : 1.0;
+    p.xyz_q_format = c.xyz_q_format;
+    return p;
+}
+
 static void fill_devconfig(const mmw_config& c, int ncap, int tcap, DevConfig* d) {
-    const double ang = c.s_tilt_deg * (M_PI / 180.0);      // numpy.radians
-    d->cos_t = std::cos(ang);
-    d->sin_t = std::sin(ang);
-    d->s_height = c.s_height;
-    d->z_max = c.z_max;
+    d->sensor = sensor_rec(config_sensor(c));
     d->db_z_weight = c.db_z_weight;
     d->db_range_weight = c.db_range_weight;
     d->db_eps = c.db_eps;
@@ -161,8 +185,6 @@ static void fill_devconfig(const mmw_config& c, int ncap, int tcap, DevConfig* d
     d->int_std = c.intensity_std;
     d->nudge_thres = c.x_nudge_thres;
     d->nudge_gain = c.x_nudge_gain;
-    d->doppler_res = c.doppler_res != 0.0 ? c.doppler_res : 1.0;
-    d->xyz_scale = (float)std::ldexp(1.0, -(c.xyz_q_format));
     d->db_min_samples = c.db_min_samples;
     d->ring_size = c.frames_batch + 1;
     d->tr_max_tracks = c.tr_max_tracks;
@@ -213,7 +235,7 @@ int mmw_destroy(mmw_ctx* x) {
     if (!x) return MMW_OK;
     cudaSetDevice(x->device);
     if (x->stream) cudaStreamSynchronize(x->stream);
-    void* ptrs[] = {x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
+    void* ptrs[] = {x->d_sensors, x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
                     x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist, x->d_pts2[0], x->d_pts2[1], x->d_offsets2[0],
                     x->d_offsets2[1], x->d_dt2[0], x->d_dt2[1], x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
                     x->d_bn1t, x->d_bn2s, x->d_bn2t, x->d_feats, x->d_row_scene, x->d_row_track, x->d_row_slot,
@@ -431,8 +453,17 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
     ALLOC(x->d_pose_total2, sizeof(int));
     ALLOC(x->d_feats, sizeof(float) * (size_t)x->pose_cap * kRing * kFeatPts * kRawCols);
     ALLOC(x->d_pose_out, sizeof(float) * (size_t)x->pose_cap * kKp);
+    ALLOC(x->d_sensors, sizeof(SensorRec) * S);
 #undef ALLOC
     cudaMemcpy(x->d_default_posture, cfg->default_posture, sizeof(float) * kKp, cudaMemcpyHostToDevice);
+    x->sensors.assign(S, config_sensor(*cfg));
+    {
+        const std::vector<SensorRec> recs(S, x->dc.sensor);
+        if (cudaMemcpy(x->d_sensors, recs.data(), sizeof(SensorRec) * S, cudaMemcpyHostToDevice) != cudaSuccess) {
+            mmw_destroy(x);
+            return fail(MMW_ERR_CUDA, "upload of the sensor table failed");
+        }
+    }
     cudaMemset(x->d_keypoints, 0, sizeof(float) * S * max_tracks * kKp);
     int rc = mmw_reset(x);
     if (rc != MMW_OK) { mmw_destroy(x); return rc; }
@@ -441,11 +472,74 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
     return MMW_OK;
 }
 
+// Queues the upload of table entries first .. first + n - 1 on the context's stream, behind all work queued there (the
+// previous frame's feature kernel included, which runs on this stream in throughput mode too).  Nothing on the pose
+// stream reads the table: dense 2's fade-square epilogue uses only the context-wide window geometry.  The source is a
+// pageable vector, which cudaMemcpyAsync stages before it returns.
+static int upload_sensors(mmw_ctx* x, int first, int n) {
+    std::vector<SensorRec> recs(n);
+    for (int i = 0; i < n; ++i) recs[i] = sensor_rec(x->sensors[first + i]);
+    CK(cudaSetDevice(x->device));
+    CK(cudaMemcpyAsync(x->d_sensors + first, recs.data(), sizeof(SensorRec) * n, cudaMemcpyHostToDevice, x->stream));
+    return MMW_OK;
+}
+
 int mmw_set_doppler_resolution(mmw_ctx* x, double doppler_res) {
     if (!x) return fail(MMW_ERR_INVALID, "ctx is NULL");
     if (!(doppler_res > 0.0) || !std::isfinite(doppler_res)) return fail(MMW_ERR_INVALID, "doppler_res must be positive and finite");
     x->cfg.doppler_res = doppler_res;
-    x->dc.doppler_res = doppler_res;
+    x->dc.sensor.doppler_res = doppler_res;
+    for (mmw_scene_sensor& p : x->sensors) p.doppler_res = doppler_res;
+    return upload_sensors(x, 0, x->S);
+}
+
+int mmw_set_scene_sensors(mmw_ctx* x, int first, int n, const mmw_scene_sensor* params) {
+    if (!x || !params) return fail(MMW_ERR_INVALID, "ctx/params is NULL");
+    if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
+    for (int i = 0; i < n; ++i) {
+        const mmw_scene_sensor& p = params[i];
+        if (!std::isfinite(p.s_height) || !std::isfinite(p.s_tilt_deg) || !std::isfinite(p.z_max) ||
+            !std::isfinite(p.doppler_res))
+            return fail(MMW_ERR_INVALID, "sensor parameters must be finite");
+        if (!(p.doppler_res > 0.0)) return fail(MMW_ERR_INVALID, "doppler_res must be positive");
+        if (p.xyz_q_format < 0 || p.xyz_q_format > 15) return fail(MMW_ERR_INVALID, "xyz_q_format must be 0..15");
+    }
+    if (n == 0) return MMW_OK;
+    for (int i = 0; i < n; ++i) {
+        x->sensors[first + i] = params[i];
+        x->sensors[first + i].reserved = 0;
+    }
+    return upload_sensors(x, first, n);
+}
+
+int mmw_get_scene_sensors(mmw_ctx* x, int first, int n, mmw_scene_sensor* out) {
+    if (!x || !out) return fail(MMW_ERR_INVALID, "ctx/out is NULL");
+    if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
+    for (int i = 0; i < n; ++i) out[i] = x->sensors[first + i];
+    return MMW_OK;
+}
+
+int mmw_reset_scenes(mmw_ctx* x, const int32_t* scenes, int n) {
+    if (!x || (!scenes && n > 0)) return fail(MMW_ERR_INVALID, "ctx/scenes is NULL");
+    if (n < 0) return fail(MMW_ERR_INVALID, "n must not be negative");
+    std::vector<char> seen(x->S, 0);
+    for (int i = 0; i < n; ++i) {
+        const int s = scenes[i];
+        if (s < 0 || s >= x->S) return fail(MMW_ERR_INVALID, "scene index out of range");
+        if (seen[s]) return fail(MMW_ERR_INVALID, "scene index listed twice");
+        seen[s] = 1;
+    }
+    CK(cudaSetDevice(x->device));
+    if (x->pose_stream) CK(join_pose(x));
+    int32_t* pose_cnt = x->d_defer + 1 + x->S;       // StepArgs::pose_cnt
+    for (int i = 0; i < n; ++i) {
+        const size_t s = scenes[i];
+        CK(cudaMemsetAsync(x->d_scenes + s, 0, sizeof(SceneRec), x->stream));
+        CK(cudaMemsetAsync(x->d_tracks + s * x->tcap, 0, sizeof(TrackRec) * x->tcap, x->stream));
+        CK(cudaMemsetAsync(x->d_ring_hist + s * kRing * kHistBytes, 0, (size_t)kRing * kHistBytes, x->stream));
+        CK(cudaMemsetAsync(x->d_scene_stats + s * 8, 0, sizeof(int32_t) * 8, x->stream));
+        CK(cudaMemsetAsync(pose_cnt + s, 0, sizeof(int32_t), x->stream));
+    }
     return MMW_OK;
 }
 
@@ -584,7 +678,7 @@ static int launch_feature_stage(mmw_ctx* x, int b, bool late, cudaStream_t st) {
         CK(launch_pose_index(x->d_scenes, x->S, pose_total, x->d_counters, st));
         x->launches++;
     }
-    PoseFeatArgs fa{x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats,
+    PoseFeatArgs fa{x->dc, x->d_sensors, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_feats,
                     (x->use_tc && x->tc.ready) ? pose_tc_input(&x->tc, b) : nullptr, b ? x->d_row_scene2 : x->d_row_scene,
                     b ? x->d_row_track2 : x->d_row_track, b ? x->d_row_slot2 : x->d_row_slot,
                     x->fold_pose_index ? x->d_defer + 1 + x->S : nullptr, pose_total, x->d_counters, x->S};
@@ -604,6 +698,7 @@ int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double*
     CK(cudaSetDevice(x->device));
     StepArgs a;
     a.cfg = x->dc;
+    a.sensors = x->d_sensors;
     int host_stage = -1;
     if (flags & MMW_STEP_DEVICE_INPUT) {
         if (!pts) return fail(MMW_ERR_INVALID, "pts is NULL");
@@ -898,13 +993,13 @@ __global__ void preprocess_kernel(DevConfig c, const float* pts, size_t n, doubl
     if (i >= n) return;
     const float* p = pts + i * kRawCols;
     double w[6];
-    world_from_raw(c, p[0], p[1], p[2], p[3], w);
+    world_from_raw(c.sensor, p[0], p[1], p[2], p[3], w);
     double* o = world + i * 8;
 #pragma unroll
     for (int k = 0; k < 6; ++k) o[k] = w[k];
-    o[6] = __dmul_rn((double)p[3], c.doppler_res);
+    o[6] = __dmul_rn((double)p[3], c.sensor.doppler_res);
     o[7] = (double)p[4];
-    keep[i] = ((w[2] <= c.z_max) && (w[2] > 0.0) && (w[1] > 0.0)) ? 1 : 0;
+    keep[i] = ((w[2] <= c.sensor.z_max) && (w[2] > 0.0) && (w[1] > 0.0)) ? 1 : 0;
 }
 
 __global__ void __launch_bounds__(kStepThreads) dbscan_stage_kernel(DevConfig c, const double* xyz,
@@ -1078,10 +1173,11 @@ __global__ void __launch_bounds__(256) tlv_decode_kernel(const uint8_t* bytes, c
 // format_batched_frames :523-548): ring frames newest first, [x - cx, y - cy, z, doppler, peakVal] of the first 64
 // rows per frame in float64, zero padded, unsorted, raw intensity.  One CTA of 64 threads per scene.
 constexpr int kExportRows = kRing * kFeatPts;               // the reference always writes three frames (Utils.py:526)
-__global__ void __launch_bounds__(kFeatPts) export_track0_kernel(DevConfig c, const SceneRec* scenes,
-                                                                 const TrackRec* tracks, const float* track_ring,
-                                                                 double* out, int32_t* valid) {
+__global__ void __launch_bounds__(kFeatPts) export_track0_kernel(DevConfig c, const SensorRec* sensors,
+                                                                 const SceneRec* scenes, const TrackRec* tracks,
+                                                                 const float* track_ring, double* out, int32_t* valid) {
     const int s = blockIdx.x, i = threadIdx.x;
+    const SensorRec& sr = sensors[s];
     const SceneRec sc = scenes[s];
     const TrackRec* t = tracks + (size_t)s * c.tcap;
     double* o = out + (size_t)s * (kExportRows * kRawCols + 2);
@@ -1101,11 +1197,11 @@ __global__ void __launch_bounds__(kFeatPts) export_track0_kernel(DevConfig c, co
             if (i < t->ring_cnt[phys]) {
                 const float* r = track_ring + ((((size_t)s * c.tcap + t->slot) * kRing + phys) * kFeatPts + i) * kRawCols;
                 double yw, zw;
-                world_yz(c, (double)r[1], (double)r[2], yw, zw);
+                world_yz(sr, (double)r[1], (double)r[2], yw, zw);
                 v[0] = __dsub_rn((double)r[0], cx);
                 v[1] = __dsub_rn(yw, cy);
                 v[2] = zw;
-                v[3] = __dmul_rn((double)r[3], c.doppler_res);
+                v[3] = __dmul_rn((double)r[3], sr.doppler_res);
                 v[4] = (double)r[4];
             }
         }
@@ -1301,7 +1397,7 @@ int mmw_decode_tlv(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_off
         TLV_CK(cudaMemcpyAsync(d_poff, point_offsets, sizeof(int32_t) * (n + 1), cudaMemcpyHostToDevice, x->stream));
         const long long threads = 32LL * n;
         tlv_decode_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, x->stream>>>(
-            d_bytes, d_off, n, d_poff, num_doppler_bins / 2 - 1, doppler_res / x->dc.doppler_res, d_pts);
+            d_bytes, d_off, n, d_poff, num_doppler_bins / 2 - 1, doppler_res / x->dc.sensor.doppler_res, d_pts);
         TLV_CK(cudaGetLastError());
         x->launches++;
         TLV_CK(cudaMemcpyAsync(points, d_pts, sizeof(float) * kRawCols * total, cudaMemcpyDeviceToHost, x->stream));
@@ -1320,8 +1416,8 @@ int mmw_export_track0(mmw_ctx* x, double* rows, int32_t* valid, double* centroid
         CK(cudaMalloc((void**)&x->d_export, sizeof(double) * per * x->S));
         CK(cudaMalloc((void**)&x->d_export_valid, sizeof(int32_t) * x->S));
     }
-    export_track0_kernel<<<x->S, kFeatPts, 0, x->stream>>>(x->dc, x->d_scenes, x->d_tracks, x->d_track_ring, x->d_export,
-                                                         x->d_export_valid);
+    export_track0_kernel<<<x->S, kFeatPts, 0, x->stream>>>(x->dc, x->d_sensors, x->d_scenes, x->d_tracks, x->d_track_ring,
+                                                         x->d_export, x->d_export_valid);
     CK(cudaGetLastError());
     x->launches++;
     std::vector<double> h(per * x->S);

@@ -16,16 +16,34 @@ constexpr int kStepThreads = 128;    // threads per scene CTA of the tracker ste
 constexpr int kStepWarps = kStepThreads / 32;
 constexpr int kMaxTcap = 32;
 
+// One scene's sensor mounting and radar profile (mmw_scene_sensor) as the kernels use it: one record per scene in
+// HBM (mmw_ctx::d_sensors), read by every kernel that turns raw rows into world coordinates.
+struct SensorRec {
+    double cos_t, sin_t, s_height, z_max;
+    double doppler_res;        // doppler [m/s] = row[3] * doppler_res (float64 product, ReadDataIWR1443.py:163-165)
+    float xyz_scale;           // 2^-Q of int16 point rows (MMW_STEP_INPUT_I16)
+    int32_t pad;
+};
+static_assert(sizeof(SensorRec) == 48, "SensorRec is three 16-byte chunks (moved with one bulk copy)");
+
+// The record read where it is used: volatile loads are not hoisted out of loops, so a kernel at its register limit does
+// not keep the values live (and spilled) between uses, which kernel parameters never needed.
+__device__ __forceinline__ SensorRec sensor_at_use(const SensorRec& r) {
+    const volatile SensorRec& v = r;
+    SensorRec o;
+    o.cos_t = v.cos_t; o.sin_t = v.sin_t; o.s_height = v.s_height; o.z_max = v.z_max;
+    o.doppler_res = v.doppler_res; o.xyz_scale = v.xyz_scale; o.pad = 0;
+    return o;
+}
+
 // Derived constants handed to kernels by value.
 struct DevConfig {
-    double cos_t, sin_t, s_height, z_max;
+    SensorRec sensor;          // the mmw_config's mounting: the stateless stage entry points use it
     double db_z_weight, db_range_weight, db_eps;
     double life_dyn, life_sta, vel_thres, gate;
     double q_var, p_init, g_init, a_n, a_spr;
     double spread_lim[6];
     double int_mu, int_std, nudge_thres, nudge_gain;
-    float xyz_scale;           // 2^-Q of int16 point rows (MMW_STEP_INPUT_I16)
-    double doppler_res;        // doppler [m/s] = row[3] * doppler_res (float64 product, ReadDataIWR1443.py:163-165)
     int db_min_samples, ring_size, tr_max_tracks, enable_est, est_pointnum;
     int ncap, tcap;
     // grid screen in front of DBSCAN (dbscan.cuh): fixed 16 x 16 cells over world (x, y'), at least one eps reach wide
@@ -78,6 +96,7 @@ static_assert(sizeof(SceneRec) == 64, "SceneRec is one 64-byte record");
 
 struct StepArgs {
     DevConfig cfg;
+    const SensorRec* sensors;  // [S] each scene's mounting and radar profile
     const float* pts;          // [sum N, 5] fp32 rows; int16 rows when flags has MMW_STEP_INPUT_I16
     const int32_t* offsets;    // [S+1]
     const double* dt;          // [S]
@@ -168,7 +187,7 @@ inline cudaError_t ensure_smem_attr(const void* fn, int* configured /*[kMaxDevic
 // ---- world-frame point from a raw sensor point (Utils.py:379-420) -----------------------------------
 // Written with explicit round-to-nearest multiplies/adds (no FMA contraction) so that the
 // scene-bounds predicates and the DBSCAN inputs are bit-identical to the float64 numpy oracle.
-__device__ __forceinline__ void world_yz(const DevConfig& c, double y, double z, double& yw, double& zw) {
+__device__ __forceinline__ void world_yz(const SensorRec& c, double y, double z, double& yw, double& zw) {
     yw = __dadd_rn(__dmul_rn(c.cos_t, y), __dmul_rn(-c.sin_t, z));
     zw = __dadd_rn(__dadd_rn(__dmul_rn(c.sin_t, y), __dmul_rn(c.cos_t, z)), c.s_height);
 }
@@ -193,7 +212,7 @@ __device__ __forceinline__ double div_zero_fast(double num, double den) {
     return z ? (den < 0.0 ? -num : num) : q;
 }
 
-__device__ __forceinline__ void world_from_raw(const DevConfig& c, float fx, float fy, float fz, float fd,
+__device__ __forceinline__ void world_from_raw(const SensorRec& c, float fx, float fy, float fz, float fd,
                                                double w[6]) {
     const double x = fx, y = fy, z = fz, d = __dmul_rn((double)fd, c.doppler_res);
     const double r = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)));

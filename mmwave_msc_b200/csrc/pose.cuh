@@ -8,6 +8,7 @@ namespace mmw {
 
 struct PoseFeatArgs {
     DevConfig cfg;
+    const SensorRec* sensors;   // [S] each scene's mounting and Doppler unit
     const SceneRec* scenes;
     const TrackRec* tracks;
     const float* track_ring;

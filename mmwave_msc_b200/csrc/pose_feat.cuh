@@ -9,14 +9,15 @@
 namespace mmw {
 
 // The feature maps of ONE ring frame of one track by one warp (shared by pose_feature_kernel and, for the tracks it
-// has just spawned, dbscan_big_kernel): src = the frame's 64 raw rows in the track's ring (nullptr: the frame is not in
-// the ring yet, its maps are zero), cnt real rows, (cx, cy) the track's CURRENT centroid.  Scratch per warp: 64 int64
-// keys, 320 floats, 128 uint4 (kFeatItemBytes).  kReadOnly: the rows were written by an earlier kernel (ld.global.nc).
+// has just spawned, dbscan_big_kernel): sr = the scene's mounting and Doppler unit, src = the frame's 64 raw rows in
+// the track's ring (nullptr: the frame is not in the ring yet, its maps are zero), cnt real rows, (cx, cy) the track's
+// CURRENT centroid.  Scratch per warp: 64 int64 keys, 320 floats, 128 uint4 (kFeatItemBytes).  kReadOnly: the rows
+// were written by an earlier kernel (ld.global.nc).
 constexpr int kFeatItemBytes = kFeatPts * 8 + kFeatPts * kRawCols * 4 + kFeatPts * 2 * 16;
 template <bool kReadOnly>
-__device__ __forceinline__ void pose_feature_item(const DevConfig& c, const float* src, int cnt, double cx, double cy, int f,
-                                                  float* out, uint4* pk, long long* keys, float* so, uint4* spk_w, int lane,
-                                                  int dbg) {
+__device__ __forceinline__ void pose_feature_item(const DevConfig& c, const SensorRec& sr, const float* src, int cnt,
+                                                  double cx, double cy, int f, float* out, uint4* pk, long long* keys,
+                                                  float* so, uint4* spk_w, int lane, int dbg) {
     if (src == nullptr) {
         for (int e = lane; e < kFeatPts * kRawCols; e += 32) out[e] = 0.f;
         if (pk)
@@ -60,12 +61,13 @@ __device__ __forceinline__ void pose_feature_item(const DevConfig& c, const floa
             const float x = so[i * kRawCols + 0], y = so[i * kRawCols + 1], z = so[i * kRawCols + 2];
             const float d = so[i * kRawCols + 3], p = so[i * kRawCols + 4];
             double yw, zw;
-            world_yz(c, (double)y, (double)z, yw, zw);
+            const SensorRec m = sensor_at_use(sr);
+            world_yz(m, (double)y, (double)z, yw, zw);
             key = __dsub_rn((double)x, cx);
             v[h][0] = (float)key;
             v[h][1] = (float)__dsub_rn(yw, cy);
             v[h][2] = (float)zw;
-            v[h][3] = (float)__dmul_rn((double)d, c.doppler_res);
+            v[h][3] = (float)__dmul_rn((double)d, m.doppler_res);
             v[h][4] = (float)__ddiv_rn(__dsub_rn((double)p, c.int_mu), c.int_std);
         }
         const long long b = __double_as_longlong(__dadd_rn(key, 0.0));

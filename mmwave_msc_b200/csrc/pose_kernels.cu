@@ -95,6 +95,10 @@ __global__ void __launch_bounds__(kFeatWarps * 32, 7) pose_feature_kernel(PoseFe
         n_tr = sc.last_ran ? sc.n_tracks : 0;
     }
     const DevConfig& c = a.cfg;
+    __shared__ SensorRec sr;             // the scene's mounting and Doppler unit
+    if (threadIdx.x < sizeof(SensorRec) / 8)
+        reinterpret_cast<double*>(&sr)[threadIdx.x] = reinterpret_cast<const double*>(a.sensors + s)[threadIdx.x];
+    __syncthreads();
     const int nfr = c.ring_size;
     const int items = n_tr * nfr;
     for (int item = warp; item < items; item += kFeatWarps) {
@@ -116,8 +120,8 @@ __global__ void __launch_bounds__(kFeatWarps * 32, 7) pose_feature_kernel(PoseFe
             cnt = t->ring_cnt[phys];
             src = a.track_ring + (((size_t)s * c.tcap + slot) * kRing + phys) * (kFeatPts * kRawCols);
         }
-        pose_feature_item<true>(c, src, cnt, t->centroid[0], t->centroid[1], f, out, pk, keys[warp], srow[warp], spk[warp],
-                                lane, a.dbg);
+        pose_feature_item<true>(c, sr, src, cnt, t->centroid[0], t->centroid[1], f, out, pk, keys[warp], srow[warp],
+                                spk[warp], lane, a.dbg);
     }
     if (a.pose_cnt != nullptr && !(a.dbg & 1) && s == a.n_scenes - 1 && threadIdx.x == 0) {
         int total = pose_base + n_tr;

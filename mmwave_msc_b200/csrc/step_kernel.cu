@@ -7,8 +7,9 @@
 // ring rows written and three 272-byte cell histograms for the screen.
 //
 // How the work is laid out (round 2; profiles/r02_*.md):
-//   * inputs arrive by three bulk copies (cp.async.bulk, 1-D TMA) behind one mbarrier: the scene's contiguous block
-//     of raw points (as the 16-byte aligned window around it), its track records and the ring's cell histograms;
+//   * inputs arrive by four bulk copies (cp.async.bulk, 1-D TMA) behind one mbarrier: the scene's contiguous block
+//     of raw points (as the 16-byte aligned window around it), its track records, the ring's cell histograms and the
+//     scene's sensor record (mounting, Doppler unit, Q format; read from shared memory where it is used);
 //   * point phases are thread-per-point, two points per thread per tile of 256, both in flight at once (straight-
 //     line code, two independent float64 chains) -- transform, filter, gate, list positions, ring pushes all work
 //     from registers;
@@ -39,6 +40,7 @@ static_assert(kProd + 21 <= kBw, "B holds the statistics totals next to the gate
 static_assert(kStepThreads == 128, "the element-parallel track phases are written for 128 threads per scene");
 
 // Dynamic shared memory of step_kernel.
+//   sensor  the scene's SensorRec (48 bytes; first, so that its address is a constant)
 //   tracks  TrackRec [tcap]
 //   B       double [tcap][72]   gate..association: see above;  update: S -> S^-1 (0..35) | Rc (36..71)
 //   A       double [tcap][81]   F P (predict), C (gate matrix, first 36), (I - K H) P (update)
@@ -48,7 +50,7 @@ static_assert(kStepThreads == 128, "the element-parallel track phases are writte
 //   and the update; the staged raw points lie over KK when a frame is a single tile, in their own space otherwise
 //   (they must survive the tile loop).
 struct SmemLayout {
-    int tracks, B, A, KK, stage, hist, hnew, misc, total;
+    int sensor, tracks, B, A, KK, stage, hist, hnew, misc, total;
 };
 constexpr int kMiscInts = 192;
 // misc int slots (slot 0-1: the mbarrier)
@@ -59,6 +61,7 @@ static_assert(kCntG + 64 <= kMiscInts, "misc layout");
 __host__ __device__ inline SmemLayout make_layout(int ncap, int tcap) {
     SmemLayout L;
     int o = 0;
+    L.sensor = o;  o += (int)sizeof(SensorRec);
     L.tracks = o;  o += tcap * (int)sizeof(TrackRec);
     L.B = o;       o += tcap * kBw * 8;
     L.A = o;
@@ -141,8 +144,8 @@ __device__ __forceinline__ const float* uring_frame(const StepArgs& a, int s, in
 // over PointCluster(cluster), :120-136): statistics over the 6 world columns recomputed from the ring's raw rows,
 // state x = [centroid, 0, 0, 0], P = KF_P_INIT*I, group dispersion = KF_GROUP_DISP_EST_INIT*I, ring = [first 64
 // cluster rows in fused order], keypoints = MODEL_DEFAULT_POSTURE.  `t` may live in shared or global memory.
-__device__ __forceinline__ void spawn_track(const StepArgs& a, int s, TrackRec& t, int q, int slot, int track_id,
-                                            const int* cl, const int* fcnt, const int* fphys, int lane,
+__device__ __forceinline__ void spawn_track(const StepArgs& a, const SensorRec& sr, int s, TrackRec& t, int q, int slot,
+                                            int track_id, const int* cl, const int* fcnt, const int* fphys, int lane,
                                             const float* rawc = nullptr /* fused raw rows in shared memory */,
                                             const double* w6 = nullptr /* their world 6-vectors, precomputed */) {
     const DevConfig& c = a.cfg;
@@ -168,7 +171,7 @@ __device__ __forceinline__ void spawn_track(const StepArgs& a, int s, TrackRec& 
 #pragma unroll
                     for (int k = 0; k < 6; ++k) w[k] = w6[(size_t)(b0 + i) * 6 + k];
                 } else {
-                    world_from_raw(c, r5[0], r5[1], r5[2], r5[3], w);
+                    world_from_raw(sr, r5[0], r5[1], r5[2], r5[3], w);
                 }
                 ++n;
 #pragma unroll
@@ -328,12 +331,12 @@ __device__ __forceinline__ void spawn_track_block(const StepArgs& a, int s, Trac
 
 // fp32 world coordinates of the fused ring (oldest frame first) into shared memory + the screened predicate over
 // them (dbscan.cuh).  Block-cooperative; ends with __syncthreads().
-__device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, int s, const int* fcnt, const int* fphys,
-                                                      float* Xf, int stride, float* rawc = nullptr) {
+__device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, const SensorRec& sr, int s, const int* fcnt,
+                                                      const int* fphys, float* Xf, int stride, float* rawc = nullptr) {
     const DevConfig& c = a.cfg;
     float* Yf = Xf + stride;
     float* Zf = Yf + stride;
-    NbScreened nb{c, Xf, Yf, Zf, {nullptr, nullptr, nullptr}, {0, 0, 0, 0}, c.db_eps, 0.f, 0.f,
+    NbScreened nb{c, sr, Xf, Yf, Zf, {nullptr, nullptr, nullptr}, {0, 0, 0, 0}, c.db_eps, 0.f, 0.f,
                   (float)c.db_range_weight, (float)c.db_z_weight, rawc};
     const float band = 1e-3f * (float)c.db_eps + 1e-4f;
     nb.lo = (float)c.db_eps - band;
@@ -354,7 +357,7 @@ __device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, int s, 
         const int i = b - nb.start[f];
         const float x = src[i * kRawCols + 0], y = src[i * kRawCols + 1], z = src[i * kRawCols + 2];
         double yw, zw;
-        world_yz(c, (double)y, (double)z, yw, zw);
+        world_yz(sr, (double)y, (double)z, yw, zw);
         Xf[b] = x; Yf[b] = (float)yw; Zf[b] = (float)zw;
         if (rawc != nullptr) {
             float* r = rawc + (size_t)b * kRawCols;
@@ -401,6 +404,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     int* misc = reinterpret_cast<int*>(smem + L.misc);
     uint8_t* cntG = reinterpret_cast<uint8_t*>(misc + kCntG);   // [kChunks][32] points per chunk and track
     uint64_t* mbar = reinterpret_cast<uint64_t*>(smem + L.misc);
+    const SensorRec& sr = *reinterpret_cast<const SensorRec*>(smem);   // this scene's mounting (L.sensor = 0)
 
     const int s = blockIdx.x;
     if (s >= a.n_scenes) return;
@@ -409,7 +413,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     const Elem el(tid);
     const unsigned ltmask = (1u << lane) - 1u;
 
-    // ---- 0. round trip one: scene record, offsets, dt; then the bulk copies ----------------------------------
+    // ---- 0. round trip one: scene record, offsets, dt; then the four bulk copies -----------------------------
     if (tid == 0) sk_mbar_init(mbar, 1);
     SceneRec sc = a.scenes[s];           // every thread keeps a copy; thread 0 writes it back
     const int off = a.offsets[s];
@@ -430,11 +434,12 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     const int16_t* stageh = reinterpret_cast<const int16_t*>(stageb);
     if (tid == 0) {
         const uint32_t tr_bytes = (uint32_t)T0 * (uint32_t)sizeof(TrackRec);
-        sk_mbar_expect_tx(mbar, tr_bytes + (bulk_pts ? win_bytes : 0u) + (uint32_t)(kRing * kHistBytes));
+        sk_mbar_expect_tx(mbar, tr_bytes + (bulk_pts ? win_bytes : 0u) + (uint32_t)(kRing * kHistBytes + sizeof(SensorRec)));
         if (tr_bytes) sk_bulk_g2s(tr, a.tracks + (size_t)s * tcap, tr_bytes, mbar);
         if (bulk_pts && win_bytes)
             sk_bulk_g2s(smem + L.stage, reinterpret_cast<const unsigned char*>(a.pts) + win0, win_bytes, mbar);
         sk_bulk_g2s(hist, a.ring_hist + (size_t)s * (kRing * kHistBytes), kRing * kHistBytes, mbar);
+        sk_bulk_g2s(smem + L.sensor, a.sensors + s, (uint32_t)sizeof(SensorRec), mbar);
     }
     if (!bulk_pts) {
         if (i16) {
@@ -513,14 +518,14 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
             const int ic = i < N ? i : N - 1;                    // lanes past the end redo the last point (discarded)
             if (i16) {                   // value / 2^Q is exact in fp32; the Doppler column is the index
                 const int16_t* p = stageh + ic * kRawCols;
-                raw[r2][0] = (float)p[0] * c.xyz_scale; raw[r2][1] = (float)p[1] * c.xyz_scale;
-                raw[r2][2] = (float)p[2] * c.xyz_scale; raw[r2][3] = (float)p[3]; raw[r2][4] = (float)p[4];
+                raw[r2][0] = (float)p[0] * sr.xyz_scale; raw[r2][1] = (float)p[1] * sr.xyz_scale;
+                raw[r2][2] = (float)p[2] * sr.xyz_scale; raw[r2][3] = (float)p[3]; raw[r2][4] = (float)p[4];
             } else {
 #pragma unroll
                 for (int k = 0; k < kRawCols; ++k) raw[r2][k] = stagef[ic * kRawCols + k];
             }
-            world_from_raw(c, raw[r2][0], raw[r2][1], raw[r2][2], raw[r2][3], w[r2]);
-            keep[r2] = i < N && (w[r2][2] <= c.z_max) && (w[r2][2] > 0.0) && (w[r2][1] > 0.0);   // Utils.py:423-427
+            world_from_raw(sr, raw[r2][0], raw[r2][1], raw[r2][2], raw[r2][3], w[r2]);
+            keep[r2] = i < N && (w[r2][2] <= sr.z_max) && (w[r2][2] > 0.0) && (w[r2][1] > 0.0);   // Utils.py:423-427
         }
 #pragma unroll
         for (int r2 = 0; r2 < 2; ++r2) {
@@ -1006,9 +1011,13 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
             dbg_t = now;
         }
     };
+    __shared__ SensorRec s_sr;            // the scene's mounting
     for (int it = blockIdx.x; it < n_defer; it += gridDim.x) {
         const int s = a.defer_list[it];
         SceneRec sc = a.scenes[s];
+        if (tid < (int)(sizeof(SensorRec) / 8))
+            reinterpret_cast<double*>(&s_sr)[tid] = reinterpret_cast<const double*>(a.sensors + s)[tid];
+        __syncthreads();
         const int T1 = sc.n_tracks;
         int B = 0;
         int fcnt[kRing], fphys[kRing];
@@ -1018,7 +1027,7 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
             B += fcnt[f];
         }
         const bool bits = B <= bits_cap;
-        NbScreened nb = load_fused_ring(a, s, fcnt, fphys, Xf, 3 * ncap, bits ? rawc : nullptr);
+        NbScreened nb = load_fused_ring(a, s_sr, s, fcnt, fphys, Xf, 3 * ncap, bits ? rawc : nullptr);
         stamp(0);
         int ncl = bits ? dbscan_bits_block(nb, B, c.db_min_samples, adj, cm, bws, par, cl, dbg != nullptr ? dbg - 10 : nullptr)
                        : dbscan_block(nb, B, c.db_min_samples, par, cl, scan, dbg != nullptr ? dbg - 10 : nullptr, false,
@@ -1042,7 +1051,7 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                     if (cl[b] >= 0) {
                         const float* r = rawc + (size_t)b * kRawCols;
                         double w[6];
-                        world_from_raw(c, r[0], r[1], r[2], r[3], w);
+                        world_from_raw(s_sr, r[0], r[1], r[2], r[3], w);
 #pragma unroll
                         for (int k = 0; k < 6; ++k) w6[(size_t)b * 6 + k] = w[k];
                     }
@@ -1056,8 +1065,8 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                                       w6, red);
             } else {
                 for (int q = warp; q < ncl; q += kBigThreads / 32)
-                    spawn_track(a, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, fcnt, fphys,
-                                lane, nullptr, nullptr);
+                    spawn_track(a, s_sr, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, fcnt,
+                                fphys, lane, nullptr, nullptr);
             }
             if (a.nr_extra != nullptr) {
                 // Pose rows of the new tracks, behind the rows of all tracks that existed when step_kernel finished (the
@@ -1093,8 +1102,8 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                     uint4* pk = a.nr_packed != nullptr
                                     ? reinterpret_cast<uint4*>(static_cast<unsigned char*>(a.nr_packed) + (size_t)row * nfr * kFeatPts * 32)
                                     : nullptr;
-                    pose_feature_item<false>(c, src, cnt, __ldcg(&t->centroid[0]), __ldcg(&t->centroid[1]), f, out, pk, fkeys,
-                                             fso, fsp, lane, 0);
+                    pose_feature_item<false>(c, s_sr, src, cnt, __ldcg(&t->centroid[0]), __ldcg(&t->centroid[1]), f, out, pk,
+                                             fkeys, fso, fsp, lane, 0);
                 }
             }
             sc.next_id += ncl;

@@ -39,6 +39,26 @@ class ExperimentExport:
                 np.stack(self.centroids) if n else np.zeros((0, 2)))
 
 
+def _experiment_doppler_units(d: np.ndarray, own: Optional[float]):
+    """``_doppler_units`` for one experiment: (index column, unit, own).  The unit in constants.DOPPLER_RESOLUTION (set,
+    or found in an earlier experiment) is used while the experiment's values fit it; an experiment whose values do not
+    (another radar profile) gets a unit of its own, ``own``, which it keeps."""
+    shared = getattr(const, "DOPPLER_RESOLUTION", None)
+    if own is None:
+        try:
+            idx, res = _doppler_units(d)
+            return idx, res, None
+        except ValueError:
+            if shared is None:
+                raise
+    const.DOPPLER_RESOLUTION = None if own in (None, 1.0) else own
+    try:
+        idx, res = _doppler_units(d)
+    finally:
+        const.DOPPLER_RESOLUTION = shared
+    return idx, res, res
+
+
 def preprocess_dataset_batched(experiment_dirs: Sequence[str],
                                frame_pairs: Optional[Sequence[Optional[Iterable[int]]]] = None,
                                max_points: int = 256, max_tracks: int = 8, device: int = 0) -> List[ExperimentExport]:
@@ -47,6 +67,9 @@ def preprocess_dataset_batched(experiment_dirs: Sequence[str],
     experiment_dirs   directories with 1.csv, 2.csv, ... in the reference's log format (DataLogging.py:60-89)
     frame_pairs       per experiment the mmWave frame numbers that have a Kinect partner (``pair()[i][0]``,
                       preprocessing.py:175); None = every frame
+
+    Every experiment keeps its own Doppler unit (experiments recorded with different radar profiles can share the
+    run); the unit may not change within one experiment once it has shown a non-zero Doppler value.
     """
     E = len(experiment_dirs)
     if E == 0:
@@ -62,7 +85,11 @@ def preprocess_dataset_batched(experiment_dirs: Sequence[str],
                         config=config_from_constants(const))
     first_iter = [True] * E
     t_prev = [0.0] * E
-    doppler_seen = False
+    doppler_seen = False                 # a non-zero Doppler value has been stepped in any experiment
+    seen = [False] * E                   # ... in this experiment
+    unit = [bt.cfg.doppler_res] * E      # the Doppler unit of each scene on the device
+    own = [None] * E                     # an experiment's own unit (see _experiment_doppler_units)
+    per_scene = False                    # some scene has a unit of its own
     while True:
         live = [e for e in range(E) if not readers[e].is_finished()]
         if not live:
@@ -87,13 +114,22 @@ def preprocess_dataset_batched(experiment_dirs: Sequence[str],
                 raw32 = raw.astype(np.float32)
                 if not np.array_equal(raw32[:, [0, 1, 2, 4]].astype(np.float64), raw[:, [0, 1, 2, 4]]):
                     raise ValueError("x, y, z, peakVal must be representable in float32 (int16/2^Q lattice values)")
-                raw32[:, 3], res = _doppler_units(raw[:, 3])        # the index; the device multiplies in float64
-                if bt.cfg.doppler_res != res:
-                    if doppler_seen:
-                        raise ValueError("Doppler resolution differs between experiments/frames: set "
-                                         "constants.DOPPLER_RESOLUTION")
-                    bt.set_doppler_resolution(res)
-                doppler_seen = doppler_seen or bool(np.any(raw32[:, 3] != 0))
+                raw32[:, 3], res, own[e] = _experiment_doppler_units(raw[:, 3], own[e])   # the index; the device
+                nonzero = bool(np.any(raw32[:, 3] != 0))                                # multiplies in float64
+                if unit[e] != res and nonzero:                      # (zero rows are the same in every unit)
+                    if seen[e]:
+                        raise ValueError("Doppler resolution changes within experiment %s: set "
+                                         "constants.DOPPLER_RESOLUTION" % out[e].name)
+                    if not doppler_seen and not per_scene:
+                        # nothing stepped so far has a non-zero Doppler value: the context's unit can change
+                        bt.set_doppler_resolution(res)
+                        unit = [res] * E
+                    else:                                           # this experiment's radar profile differs
+                        bt.set_scene_sensors(doppler_res=res, scenes=[e])
+                        unit[e] = res
+                        per_scene = True
+                seen[e] = seen[e] or nonzero
+                doppler_seen = doppler_seen or seen[e]
                 clouds[e] = raw32
                 stepped[e] = True
             else:

@@ -40,6 +40,8 @@ class SceneSpec:
     leave_prob: float = 0.1         # fraction of people who walk out early (their track must time out)
     clutter_box: tuple = (-2.5, 2.5, 0.3, None)   # x0, x1, y0, y1 (None -> r_max) of the uniform clutter
     t0_ms: int = 1_700_000_000_000
+    s_height: float = S_HEIGHT      # mounting of the sensor that sees the scene
+    s_tilt_deg: float = S_TILT_DEG
 
     @staticmethod
     def dense() -> "SceneSpec":
@@ -103,7 +105,7 @@ def gen_scene(scene_id: int, n_frames: int, spec: SceneSpec = SceneSpec()) -> Sc
     v_eff[1:] = (pos[1:] - pos[:-1]) / dtv[1:]
     v_eff[0] = vel[0]
 
-    th = math.radians(S_TILT_DEG)
+    th = math.radians(spec.s_tilt_deg)
     c, s = math.cos(th), math.sin(th)
     frames: List[np.ndarray] = []
     for f in range(F):
@@ -125,15 +127,15 @@ def gen_scene(scene_id: int, n_frames: int, spec: SceneSpec = SceneSpec()) -> Sc
         cy = r_pts.uniform(cb[2], spec.r_max if cb[3] is None else cb[3], size=n_cl)
         cz = r_pts.uniform(0.05, 2.45, size=n_cl)
         X = np.concatenate([wx, cx]); Y = np.concatenate([wy, cy]); Z = np.concatenate([wz, cz])
-        # radial velocity seen from the sensor at (0, 0, S_HEIGHT)
-        rx, ry, rz = X, Y, Z - S_HEIGHT
+        # radial velocity seen from the sensor at (0, 0, s_height)
+        rx, ry, rz = X, Y, Z - spec.s_height
         rr = np.sqrt(rx * rx + ry * ry + rz * rz) + 1e-9
         dop_p = (vx * rx[:n_pp] + vy * ry[:n_pp]) / rr[:n_pp]
         dop_c = r_pts.normal(0, 0.15, size=n_cl)
         dop = np.concatenate([dop_p, dop_c])
         # world -> sensor frame (inverse of Utils.py:312-327: rotate about X by -tilt after removing the height)
-        ys = c * Y + s * (Z - S_HEIGHT)
-        zs = -s * Y + c * (Z - S_HEIGHT)
+        ys = c * Y + s * (Z - spec.s_height)
+        zs = -s * Y + c * (Z - spec.s_height)
         xs = X
         perm = r_pts.permutation(N)          # the sensor does not group points by target
         xs, ys, zs, dop = xs[perm], ys[perm], zs[perm], dop[perm]
