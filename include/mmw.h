@@ -25,9 +25,9 @@
 extern "C" {
 #endif
 
-/* 5: per-scene sensor table (mmw_scene_sensor, mmw_set/get_scene_sensors) and mmw_reset_scenes.  The state blob
- * carries this number, so blobs written by version 4 are refused by mmw_state_restore. */
-#define MMW_ABI_VERSION 5
+/* 6: mmw_step_packets and mmw_scene_sensor::num_doppler_bins (5: per-scene sensor table and mmw_reset_scenes).  The
+ * state blob carries this number, so blobs written by an earlier version are refused by mmw_state_restore. */
+#define MMW_ABI_VERSION 6
 
 typedef enum mmw_status {
     MMW_OK = 0,
@@ -140,21 +140,23 @@ int mmw_set_doppler_resolution(mmw_ctx* ctx, double doppler_res);
  * rings are re-read under the new parameters: change a scene's entry before its first frame, or together with
  * mmw_reset_scenes.  The table is not part of the state blob (it is configuration, like mmw_config and the pose
  * weights): a restored context continues with whatever table it has.  The stateless stage entry points
- * (mmw_preprocess, mmw_dbscan) and mmw_decode_tlv keep using the values of the mmw_config. */
+ * (mmw_preprocess, mmw_dbscan) and mmw_decode_tlv keep using the values of the mmw_config; mmw_step_packets decodes each
+ * scene's packet with its own num_doppler_bins. */
 typedef struct mmw_scene_sensor {
     double s_height;               /* S_HEIGHT constants.py:41 */
     double s_tilt_deg;             /* S_TILT constants.py:42 */
     double z_max;                  /* scene bound on z', Utils.py:424 */
     double doppler_res;            /* unit of the Doppler column, as mmw_config::doppler_res (must be > 0 here) */
     int32_t xyz_q_format;          /* Q format of int16 rows (MMW_STEP_INPUT_I16), 0..15 */
-    int32_t reserved;
+    int32_t num_doppler_bins;      /* the radar profile's numDopplerBins (ReadDataIWR1443.py:167-175), >= 0; only
+                                      mmw_step_packets reads it.  0 (what mmw_create sets) = not set */
 } mmw_scene_sensor;
 
 /* Sets the entries of scenes first_scene .. first_scene + n - 1 from params[0 .. n-1].  All or nothing: a range out of
- * bounds, a NULL pointer, a non-finite value, doppler_res <= 0 or a Q format outside 0..15 give MMW_ERR_INVALID and
- * change no entry. */
+ * bounds, a NULL pointer, a non-finite value, doppler_res <= 0, a Q format outside 0..15 or num_doppler_bins < 0 give
+ * MMW_ERR_INVALID and change no entry. */
 int mmw_set_scene_sensors(mmw_ctx* ctx, int first_scene, int n, const mmw_scene_sensor* params);
-/* Reads the entries of scenes first_scene .. first_scene + n - 1 into out[0 .. n-1] (reserved = 0). */
+/* Reads the entries of scenes first_scene .. first_scene + n - 1 into out[0 .. n-1]. */
 int mmw_get_scene_sensors(mmw_ctx* ctx, int first_scene, int n, mmw_scene_sensor* out);
 
 /* mmw_reset restricted to the n listed scenes (e.g. a sensor slot handed to a new sensor): their scene record, track
@@ -309,6 +311,29 @@ int mmw_decode_tlv(mmw_ctx* ctx, const uint8_t* packets, const int64_t* packet_o
                    double num_doppler_bins, double doppler_res, float* points, size_t max_points_total,
                    int32_t* point_offsets, int32_t* frame_numbers, int32_t* data_ok);
 
+/* One radar frame for every scene straight from its sensor's packet: the online loop's ReadIWR14xx.read()
+ * (ReadDataIWR1443.py:88-201) followed by mmw_step, with each scene's own radar profile.
+ *   packets, packet_offsets[S+1]  host; scene s's packet is bytes [packet_offsets[s], packet_offsets[s+1]): one framed
+ *                                 packet as mmw_decode_tlv takes it, or an empty range for no packet.  packet_offsets[0]
+ *                                 must be 0.
+ *   dt [S]                        host, as for mmw_step
+ *   frame_numbers [S], data_ok [S] host or NULL; written before the call returns, as mmw_decode_tlv writes them
+ * Each packet is decoded as ReadIWR14xx.read() decodes it: x, y, z = int16 / 2^(the packet's own xyzQFormat), and the
+ * Doppler column carries the corrected dopplerIdx, using the scene's num_doppler_bins; the step multiplies it by the
+ * scene's doppler_res in float64, so doppler_res must be the profile's dopplerResolutionMps.  A packet with dataOK = 0,
+ * or no packet, is an empty frame: the scene is skipped as mmw_step skips it.  The result (overflow bits included) is
+ * that of mmw_decode_tlv with doppler_res = mmw_config::doppler_res followed by mmw_step, bit for bit.
+ * The headers (a few dozen bytes per packet) are read on the host, to validate the batch and lay out the rows; the
+ * bytes go up once, into double-buffered staging on the upload stream, and the objects are decoded on the device into
+ * the step's input.  flags: MMW_STEP_POSE, MMW_STEP_PIPELINE and MMW_STEP_RECORD_LABELS as for mmw_step;
+ * MMW_STEP_INPUT_I16 and MMW_STEP_DEVICE_INPUT give MMW_ERR_INVALID.  Errors, with nothing queued: MMW_ERR_INVALID for
+ * bad offsets or a NULL pointer; MMW_ERR_CAPACITY for more decoded points than n_scenes * max_points_per_frame;
+ * MMW_ERR_STATE for a scene whose packet yields objects while its num_doppler_bins is 0.  Host buffers as for mmw_step:
+ * keep them unchanged until the next-but-one step; asynchronous for pinned memory.  mmw_get_point_assoc,
+ * mmw_get_labels, mmw_read_results_async and the throughput mode work after it as after mmw_step. */
+int mmw_step_packets(mmw_ctx* ctx, const uint8_t* packets, const int64_t* packet_offsets, const double* dt, uint32_t flags,
+                     int32_t* frame_numbers, int32_t* data_ok);
+
 /* ---- dataset-builder mode (SURVEY 8(f) row 3) ---- */
 
 /* What preprocessing.preprocess_dataset (preprocessing.py:185-216) writes after a frame, for every scene at once:
@@ -387,7 +412,7 @@ int mmw_get_counters(mmw_ctx* ctx, uint64_t out[8], int reset);
  * 0 = CUDA-core fp32 path (kept for numerics comparison). */
 int mmw_set_dense_path(mmw_ctx* ctx, int use_tensor_cores);
 
-/* Per-kernel device time: while enabled, every launch of mmw_step is bracketed by CUDA events on the context's
+/* Per-kernel device time: while enabled, every launch of mmw_step / mmw_step_packets is bracketed by CUDA events on the context's
  * stream.  mmw_get_kernel_ms returns the accumulated milliseconds and launch counts per kernel class. */
 #define MMW_K_STEP 0           /* fused tracker step (normalize + track) */
 #define MMW_K_POSE_INDEX 1     /* pose row compaction */
@@ -396,6 +421,7 @@ int mmw_set_dense_path(mmw_ctx* ctx, int use_tensor_cores);
 #define MMW_K_FC1 4            /* dense 1 (+ operand split when the tensor-core path is on) */
 #define MMW_K_FC2 5            /* dense 2 */
 #define MMW_K_DBSCAN_BIG 6     /* union / border / spawn of the few scenes per frame in which clusters form */
+#define MMW_K_PACKETS 7        /* decode of the packets of mmw_step_packets into the step's input */
 #define MMW_N_KERNELS 8
 int mmw_profile(mmw_ctx* ctx, int enable);
 int mmw_get_kernel_ms(mmw_ctx* ctx, double* total_ms /*[MMW_N_KERNELS]*/, uint64_t* calls /*[MMW_N_KERNELS]*/);

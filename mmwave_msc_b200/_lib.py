@@ -14,8 +14,8 @@ MMW_POSE_2D, MMW_POSE_3D = 0, 1
 STEP_POSE, STEP_DEVICE_INPUT, STEP_RECORD_LABELS, STEP_PIPELINE, STEP_INPUT_I16 = 0x1, 0x2, 0x4, 0x8, 0x10
 SCENE_POINT_OVERFLOW, SCENE_TRACK_OVERFLOW = 0x1, 0x2
 RESULT_FLOATS = 72
-ABI_VERSION = 5            # MMW_ABI_VERSION of include/mmw.h this binding was written against
-KERNEL_NAMES = ["step", "pose_index", "pose_features", "conv", "fc1", "fc2", "dbscan_big", "k7"]
+ABI_VERSION = 6            # MMW_ABI_VERSION of include/mmw.h this binding was written against
+KERNEL_NAMES = ["step", "pose_index", "pose_features", "conv", "fc1", "fc2", "dbscan_big", "packets"]
 
 
 class MmwError(RuntimeError):
@@ -47,13 +47,13 @@ class SceneSensor(C.Structure):
     """mmw_scene_sensor: one scene's sensor mounting and radar profile (see include/mmw.h)."""
     _fields_ = [
         ("s_height", C.c_double), ("s_tilt_deg", C.c_double), ("z_max", C.c_double), ("doppler_res", C.c_double),
-        ("xyz_q_format", C.c_int32), ("reserved", C.c_int32),
+        ("xyz_q_format", C.c_int32), ("num_doppler_bins", C.c_int32),
     ]
 
 
 SCENE_SENSOR_DTYPE = np.dtype([
     ("s_height", "<f8"), ("s_tilt_deg", "<f8"), ("z_max", "<f8"), ("doppler_res", "<f8"),
-    ("xyz_q_format", "<i4"), ("reserved", "<i4"),
+    ("xyz_q_format", "<i4"), ("num_doppler_bins", "<i4"),
 ], align=False)
 assert SCENE_SENSOR_DTYPE.itemsize == C.sizeof(SceneSensor), (SCENE_SENSOR_DTYPE.itemsize, C.sizeof(SceneSensor))
 
@@ -120,6 +120,7 @@ SIGNATURES = {
     "mmw_gate": (C.c_int, [_p, _p, C.c_int, _p, _p, C.c_int, _p, _p]),
     "mmw_pose": (C.c_int, [_p, _p, C.c_int, _p]),
     "mmw_decode_tlv": (C.c_int, [_p, _p, _p, C.c_int, C.c_double, C.c_double, _p, C.c_size_t, _p, _p, _p]),
+    "mmw_step_packets": (C.c_int, [_p, _p, _p, _p, C.c_uint32, _p, _p]),
     "mmw_export_track0": (C.c_int, [_p, _p, _p, _p]),
     "mmw_pack_results": (C.c_int, [_p, _p]),
     "mmw_gather_nccl": (C.c_int, [_p, _p, C.c_int, _p]),

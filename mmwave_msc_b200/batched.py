@@ -57,6 +57,15 @@ def config_from_constants(const) -> _lib.Config:
         doppler_res=float(getattr(const, "DOPPLER_RESOLUTION", None) or 1.0))
 
 
+def concat_packets(packets: Sequence[Optional[bytes]]) -> Tuple[np.ndarray, np.ndarray]:
+    """One framed UART packet (bytes) or None per scene -> (blob (bytes,) uint8, offsets (S+1,) int64), the layout
+    ``BatchedTracker.step_packets`` takes: scene s's packet is blob[offsets[s]:offsets[s+1]], empty for None."""
+    parts = [b"" if p is None else bytes(p) for p in packets]
+    offsets = np.zeros(len(parts) + 1, np.int64)
+    offsets[1:] = np.cumsum([len(p) for p in parts])
+    return np.frombuffer(b"".join(parts), dtype=np.uint8).copy(), offsets
+
+
 class BatchedTracker:
     """S scenes resident on one GPU.  ``step`` = the loop body of the reference's offline_main.py:45-60
     for every scene at once."""
@@ -102,28 +111,31 @@ class BatchedTracker:
 
     def scene_sensors(self) -> np.ndarray:
         """Every scene's sensor mounting and radar profile (mmw_scene_sensor): a (S,) structured array
-        (``_lib.SCENE_SENSOR_DTYPE``) with s_height, s_tilt_deg, z_max, doppler_res, xyz_q_format."""
+        (``_lib.SCENE_SENSOR_DTYPE``) with s_height, s_tilt_deg, z_max, doppler_res, xyz_q_format, num_doppler_bins."""
         out = np.zeros(self.S, _lib.SCENE_SENSOR_DTYPE)
         _lib.check(self.lib.mmw_get_scene_sensors(self._h, 0, self.S, _lib.ptr(out)))
         return out
 
     def set_scene_sensors(self, s_height=None, s_tilt_deg=None, z_max=None, doppler_res=None, xyz_q_format=None,
-                          scenes=None):
+                          scenes=None, num_doppler_bins=None):
         """Sets the mounting and radar profile of the selected scenes (``scenes``: a slice or index array, default all).
         Each value is a scalar or an array with one entry per selected scene; None keeps the current value.  Takes
         effect with the next step.  Rows already in a scene's rings are re-read under the new values: change a scene
-        before its first frame, or together with ``reset_scenes``.  All or nothing: invalid values change no scene."""
+        before its first frame, or together with ``reset_scenes``.  All or nothing: invalid values change no scene.
+        ``num_doppler_bins`` is the radar profile's numDopplerBins, which ``step_packets`` needs (with ``doppler_res`` =
+        the profile's dopplerResolutionMps)."""
         idx = self._scene_index(scenes)
         table = self.scene_sensors()
         for name, v in (("s_height", s_height), ("s_tilt_deg", s_tilt_deg), ("z_max", z_max),
-                        ("doppler_res", doppler_res), ("xyz_q_format", xyz_q_format)):
+                        ("doppler_res", doppler_res), ("xyz_q_format", xyz_q_format),
+                        ("num_doppler_bins", num_doppler_bins)):
             if v is None:
                 continue
             v = np.asarray(v)
             if v.ndim and v.shape != idx.shape:
                 raise ValueError("%s: give a scalar or one value per selected scene" % name)
-            if name == "xyz_q_format" and not np.array_equal(v, np.round(v)):
-                raise ValueError("xyz_q_format must be an integer")
+            if name in ("xyz_q_format", "num_doppler_bins") and not np.array_equal(v, np.round(v)):
+                raise ValueError("%s must be an integer" % name)
             table[name][idx] = v
         _lib.check(self.lib.mmw_set_scene_sensors(self._h, 0, self.S, _lib.ptr(table)))
 
@@ -167,6 +179,31 @@ class BatchedTracker:
                  (_lib.STEP_PIPELINE if pipeline else 0) | (_lib.STEP_INPUT_I16 if i16 else 0))
         self._n_last = points.shape[0]
         _lib.check(self.lib.mmw_step(self._h, _lib.ptr(points), _lib.ptr(offsets), _lib.ptr(dt), flags))
+
+    def step_packets(self, blob: np.ndarray, offsets: np.ndarray, dt: np.ndarray, pose: bool = True,
+                     record_labels: bool = False, pipeline: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+        """One frame for every scene from its sensor's UART packet (mmw_step_packets): ReadIWR14xx.read() on the
+        device, with each scene's own num_doppler_bins (``set_scene_sensors``), then ``step``.  blob (bytes,) uint8 and
+        offsets (S+1,) int64 as ``concat_packets`` builds them, dt (S,) float64.  Returns (frame_numbers (S,) int32,
+        data_ok (S,) bool); a scene without a packet or with dataOK = 0 is skipped this frame.  Asynchronous when blob
+        is pinned memory; keep it unchanged until the next-but-one step."""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8).reshape(-1)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        dt = np.ascontiguousarray(dt, dtype=np.float64)
+        if offsets.shape != (self.S + 1,) or dt.shape != (self.S,):
+            raise ValueError("offsets must have S+1 entries and dt S entries")
+        if int(offsets[0]) != 0 or int(offsets[-1]) > blob.size:
+            raise ValueError("offsets must start at 0 and end within the blob")
+        flags = ((_lib.STEP_POSE if pose else 0) | (_lib.STEP_RECORD_LABELS if record_labels else 0) |
+                 (_lib.STEP_PIPELINE if pipeline else 0))
+        frames = np.zeros(self.S, np.int32)
+        ok = np.zeros(self.S, np.int32)
+        _lib.check(self.lib.mmw_step_packets(self._h, _lib.ptr(blob), _lib.ptr(offsets), _lib.ptr(dt), flags,
+                                             _lib.ptr(frames), _lib.ptr(ok)))
+        # rows of the step (for point_assoc): numObj (u16 at byte 44) of every packet that yielded objects
+        at = offsets[:-1][ok != 0] + 44
+        self._n_last = int((blob[at].astype(np.int64) | (blob[at + 1].astype(np.int64) << 8)).sum())
+        return frames, ok.astype(bool)
 
     def step_device(self, points_ptr: int, offsets_ptr: int, dt_ptr: int, n_points: int, pose: bool = True,
                     pipeline: bool = False):

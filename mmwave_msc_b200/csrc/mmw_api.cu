@@ -42,6 +42,7 @@ struct mmw_ctx {
     // sensor table: each scene's mounting and radar profile as set (host) and as the kernels read it (device, [S])
     std::vector<mmw_scene_sensor> sensors;
     SensorRec* d_sensors = nullptr;
+    double* d_doppler_wrap = nullptr; // [S] num_doppler_bins / 2 - 1 of each scene: the Doppler threshold of mmw_step_packets
     // resident state
     TrackRec* d_tracks = nullptr;
     SceneRec* d_scenes = nullptr;
@@ -67,6 +68,8 @@ struct mmw_ctx {
     float* d_pts2[2] = {nullptr, nullptr};
     int32_t* d_offsets2[2] = {nullptr, nullptr};
     double* d_dt2[2] = {nullptr, nullptr};
+    uint8_t* d_pk2[2] = {nullptr, nullptr};   // mmw_step_packets: [S+1] packet offsets (int64) + packet bytes, same buffers
+    size_t pk_cap[2] = {0, 0};                //   index and events as the fp32 staging; grown on demand
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;
     // mmw_run_frames: the inputs of kGroup consecutive frames go up in ONE copy per array (a 2 MB copy runs at 15 GB/s
     // on a link that gives 24 GB/s at 8 MB: per-copy cost, not bandwidth), double-buffered by group
@@ -155,7 +158,12 @@ static SensorRec sensor_rec(const mmw_scene_sensor& p) {
     return r;
 }
 
-// The sensor-table entry every scene starts with: the mmw_config's values (doppler_res 0 is read as 1.0).
+// Threshold of the dopplerIdx correction of mmw_step_packets (ReadDataIWR1443.py:167-175): the value mmw_decode_tlv
+// computes from its num_doppler_bins argument.
+static double doppler_wrap(const mmw_scene_sensor& p) { return (double)p.num_doppler_bins / 2 - 1; }
+
+// The sensor-table entry every scene starts with: the mmw_config's values (doppler_res 0 is read as 1.0), no
+// num_doppler_bins.
 static mmw_scene_sensor config_sensor(const mmw_config& c) {
     mmw_scene_sensor p{};
     p.s_height = c.s_height;
@@ -235,7 +243,7 @@ int mmw_destroy(mmw_ctx* x) {
     if (!x) return MMW_OK;
     cudaSetDevice(x->device);
     if (x->stream) cudaStreamSynchronize(x->stream);
-    void* ptrs[] = {x->d_sensors, x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
+    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_pk2[0], x->d_pk2[1], x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
                     x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist, x->d_pts2[0], x->d_pts2[1], x->d_offsets2[0],
                     x->d_offsets2[1], x->d_dt2[0], x->d_dt2[1], x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
                     x->d_bn1t, x->d_bn2s, x->d_bn2t, x->d_feats, x->d_row_scene, x->d_row_track, x->d_row_slot,
@@ -454,12 +462,15 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
     ALLOC(x->d_feats, sizeof(float) * (size_t)x->pose_cap * kRing * kFeatPts * kRawCols);
     ALLOC(x->d_pose_out, sizeof(float) * (size_t)x->pose_cap * kKp);
     ALLOC(x->d_sensors, sizeof(SensorRec) * S);
+    ALLOC(x->d_doppler_wrap, sizeof(double) * S);
 #undef ALLOC
     cudaMemcpy(x->d_default_posture, cfg->default_posture, sizeof(float) * kKp, cudaMemcpyHostToDevice);
     x->sensors.assign(S, config_sensor(*cfg));
     {
         const std::vector<SensorRec> recs(S, x->dc.sensor);
-        if (cudaMemcpy(x->d_sensors, recs.data(), sizeof(SensorRec) * S, cudaMemcpyHostToDevice) != cudaSuccess) {
+        const std::vector<double> wrap(S, doppler_wrap(x->sensors[0]));
+        if (cudaMemcpy(x->d_sensors, recs.data(), sizeof(SensorRec) * S, cudaMemcpyHostToDevice) != cudaSuccess ||
+            cudaMemcpy(x->d_doppler_wrap, wrap.data(), sizeof(double) * S, cudaMemcpyHostToDevice) != cudaSuccess) {
             mmw_destroy(x);
             return fail(MMW_ERR_CUDA, "upload of the sensor table failed");
         }
@@ -474,13 +485,18 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
 
 // Queues the upload of table entries first .. first + n - 1 on the context's stream, behind all work queued there (the
 // previous frame's feature kernel included, which runs on this stream in throughput mode too).  Nothing on the pose
-// stream reads the table: dense 2's fade-square epilogue uses only the context-wide window geometry.  The source is a
-// pageable vector, which cudaMemcpyAsync stages before it returns.
+// stream reads the table: dense 2's fade-square epilogue uses only the context-wide window geometry.  The sources are
+// pageable vectors, which cudaMemcpyAsync stages before it returns.
 static int upload_sensors(mmw_ctx* x, int first, int n) {
     std::vector<SensorRec> recs(n);
-    for (int i = 0; i < n; ++i) recs[i] = sensor_rec(x->sensors[first + i]);
+    std::vector<double> wrap(n);
+    for (int i = 0; i < n; ++i) {
+        recs[i] = sensor_rec(x->sensors[first + i]);
+        wrap[i] = doppler_wrap(x->sensors[first + i]);
+    }
     CK(cudaSetDevice(x->device));
     CK(cudaMemcpyAsync(x->d_sensors + first, recs.data(), sizeof(SensorRec) * n, cudaMemcpyHostToDevice, x->stream));
+    CK(cudaMemcpyAsync(x->d_doppler_wrap + first, wrap.data(), sizeof(double) * n, cudaMemcpyHostToDevice, x->stream));
     return MMW_OK;
 }
 
@@ -503,12 +519,10 @@ int mmw_set_scene_sensors(mmw_ctx* x, int first, int n, const mmw_scene_sensor* 
             return fail(MMW_ERR_INVALID, "sensor parameters must be finite");
         if (!(p.doppler_res > 0.0)) return fail(MMW_ERR_INVALID, "doppler_res must be positive");
         if (p.xyz_q_format < 0 || p.xyz_q_format > 15) return fail(MMW_ERR_INVALID, "xyz_q_format must be 0..15");
+        if (p.num_doppler_bins < 0) return fail(MMW_ERR_INVALID, "num_doppler_bins must not be negative");
     }
     if (n == 0) return MMW_OK;
-    for (int i = 0; i < n; ++i) {
-        x->sensors[first + i] = params[i];
-        x->sensors[first + i].reserved = 0;
-    }
+    for (int i = 0; i < n; ++i) x->sensors[first + i] = params[i];
     return upload_sensors(x, first, n);
 }
 
@@ -691,6 +705,8 @@ static int launch_feature_stage(mmw_ctx* x, int b, bool late, cudaStream_t st) {
     return MMW_OK;
 }
 
+static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage);
+
 int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double* dt, uint32_t flags) {
     if (!x || !offsets || !dt) return fail(MMW_ERR_INVALID, "ctx/offsets/dt is NULL");
     if ((flags & MMW_STEP_POSE) && !x->has_weights)
@@ -735,6 +751,13 @@ int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double*
         a.pts = x->d_pts2[k]; a.offsets = x->d_offsets2[k]; a.dt = x->d_dt2[k];
         host_stage = k;
     }
+    return step_queue(x, a, flags, host_stage);
+}
+
+// The tracker kernels of a step whose inputs a.pts / a.offsets / a.dt are in place, then its pose stage.  host_stage:
+// the input staging buffer they were uploaded into (its stage_free event is recorded at the head of the next step), or
+// -1 for device-resident input.
+static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage) {
     a.tracks = x->d_tracks; a.scenes = x->d_scenes; a.track_ring = x->d_track_ring; a.uring = x->d_uring;
     a.keypoints = x->d_keypoints; a.default_posture = x->d_default_posture; a.assoc_out = x->d_assoc;
     a.labels_out = (flags & MMW_STEP_RECORD_LABELS) ? x->d_labels : nullptr;
@@ -1112,14 +1135,17 @@ __global__ void __launch_bounds__(128) gate_stage_kernel(const double* pts, int 
 }
 
 // ---- UART TLV packets -> fp32 point rows (ReadDataIWR1443.py:88-201) ------------------------------------
+// The header walk runs on the host too (mmw_step_packets): one definition for both.
 constexpr int kTlvHeader = 36;
-__device__ __forceinline__ uint32_t rd_u32(const uint8_t* p) {
+__host__ __device__ __forceinline__ uint32_t rd_u32(const uint8_t* p) {
     return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
 }
-__device__ __forceinline__ int rd_i16(const uint8_t* p) { return (int)(int16_t)((uint16_t)p[0] | ((uint16_t)p[1] << 8)); }
+__host__ __device__ __forceinline__ int rd_i16(const uint8_t* p) {
+    return (int)(int16_t)((uint16_t)p[0] | ((uint16_t)p[1] << 8));
+}
 
 // Number of objects a packet yields (0 when the reference would return dataOK = 0) and its frame number.
-__device__ __forceinline__ int tlv_packet_objects(const uint8_t* p, long long len, int* frame) {
+__host__ __device__ __forceinline__ int tlv_packet_objects(const uint8_t* p, long long len, int* frame) {
     const uint8_t magic[8] = {2, 1, 4, 3, 6, 5, 8, 7};
     *frame = 0;
     if (len < kTlvHeader) return 0;
@@ -1144,14 +1170,17 @@ __global__ void tlv_count_kernel(const uint8_t* bytes, const long long* off, int
     frames[i] = fr;
 }
 
-// One warp per packet, one lane per object (12 bytes in, 20 bytes out).
+// One warp per packet, one lane per object (12 bytes in, 20 bytes out).  The dopplerIdx threshold is half_bins_m1, or
+// half_bins_m1_s[packet] when that is given (one radar profile per scene).
 __global__ void __launch_bounds__(256) tlv_decode_kernel(const uint8_t* bytes, const long long* off, int n,
                                                          const int32_t* point_off, double half_bins_m1,
-                                                         double doppler_res, float* points) {
+                                                         const double* half_bins_m1_s, double doppler_res,
+                                                         float* points) {
     const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (w >= n) return;
     const int n_obj = point_off[w + 1] - point_off[w];
     if (n_obj == 0) return;
+    if (half_bins_m1_s) half_bins_m1 = half_bins_m1_s[w];
     const uint8_t* p = bytes + off[w];
     const int q = (int)((uint32_t)p[kTlvHeader + 10] | ((uint32_t)p[kTlvHeader + 11] << 8));
     const double scale = exp2((double)q);                                // 2 ** xyzQFormat (:126-128)
@@ -1397,7 +1426,7 @@ int mmw_decode_tlv(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_off
         TLV_CK(cudaMemcpyAsync(d_poff, point_offsets, sizeof(int32_t) * (n + 1), cudaMemcpyHostToDevice, x->stream));
         const long long threads = 32LL * n;
         tlv_decode_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, x->stream>>>(
-            d_bytes, d_off, n, d_poff, num_doppler_bins / 2 - 1, doppler_res / x->dc.sensor.doppler_res, d_pts);
+            d_bytes, d_off, n, d_poff, num_doppler_bins / 2 - 1, nullptr, doppler_res / x->dc.sensor.doppler_res, d_pts);
         TLV_CK(cudaGetLastError());
         x->launches++;
         TLV_CK(cudaMemcpyAsync(points, d_pts, sizeof(float) * kRawCols * total, cudaMemcpyDeviceToHost, x->stream));
@@ -1406,6 +1435,94 @@ int mmw_decode_tlv(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_off
 #undef TLV_CK
     cleanup();
     return MMW_OK;
+}
+
+int mmw_step_packets(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_offsets, const double* dt, uint32_t flags,
+                     int32_t* frame_numbers, int32_t* data_ok) {
+    if (!x || !packet_offsets || !dt) return fail(MMW_ERR_INVALID, "ctx/packet_offsets/dt is NULL");
+    if (flags & (MMW_STEP_DEVICE_INPUT | MMW_STEP_INPUT_I16))
+        return fail(MMW_ERR_INVALID, "mmw_step_packets takes host packets: MMW_STEP_DEVICE_INPUT / MMW_STEP_INPUT_I16 do not apply");
+    if ((flags & MMW_STEP_POSE) && !x->has_weights)
+        return fail(MMW_ERR_STATE, "MMW_STEP_POSE needs mmw_load_pose_weights first");
+    // the flag checks of step_queue, made here so that a refused call has queued nothing
+    if ((flags & MMW_STEP_PIPELINE) && (!(flags & MMW_STEP_POSE) || !(x->use_tc && x->tc.ready)))
+        return fail(MMW_ERR_STATE, "MMW_STEP_PIPELINE needs MMW_STEP_POSE and the tensor-core pose path");
+    if ((flags & MMW_STEP_PIPELINE) && (flags & MMW_STEP_RECORD_LABELS))
+        return fail(MMW_ERR_INVALID, "MMW_STEP_PIPELINE cannot record labels");
+    const int S = x->S;
+    if (packet_offsets[0] != 0) return fail(MMW_ERR_INVALID, "packet_offsets[0] must be 0");
+    for (int s = 0; s < S; ++s)
+        if (packet_offsets[s + 1] < packet_offsets[s]) return fail(MMW_ERR_INVALID, "packet_offsets must be non-decreasing");
+    const size_t nbytes = (size_t)packet_offsets[S];
+    if (nbytes && !packets) return fail(MMW_ERR_INVALID, "packets is NULL");
+    // Headers on the host: dataOK, the frame number and the row layout of every packet (the step needs validated
+    // offsets and the capacity check before launch; counting on the device would need a synchronisation).
+    std::vector<int32_t> rows(S + 1), frames(S);
+    rows[0] = 0;
+    const size_t cap = (size_t)S * x->ncap;
+    size_t total = 0;
+    for (int s = 0; s < S; ++s) {
+        int fr = 0;
+        const int n_obj = tlv_packet_objects(packets + packet_offsets[s], packet_offsets[s + 1] - packet_offsets[s], &fr);
+        if (n_obj > 0 && x->sensors[s].num_doppler_bins == 0)
+            return fail(MMW_ERR_STATE, "scene " + std::to_string(s) + ": a packet with objects, but the scene's "
+                                       "num_doppler_bins is not set (mmw_set_scene_sensors)");
+        total += (size_t)n_obj;
+        if (total > cap) return fail(MMW_ERR_CAPACITY, "more points than n_scenes * max_points_per_frame");
+        rows[s + 1] = (int32_t)total;
+        frames[s] = fr;
+    }
+    for (int s = 0; s < S; ++s) {
+        if (frame_numbers) frame_numbers[s] = frames[s];
+        if (data_ok) data_ok[s] = rows[s + 1] > rows[s] ? 1 : 0;
+    }
+    CK(cudaSetDevice(x->device));
+    // Upload into the staging buffers of this step (see mmw_step): [S+1] packet offsets and the packet bytes into byte
+    // staging k, the row offsets and dt into d_offsets2[k] / d_dt2[k].
+    const int k = (int)(x->stage_idx & 1u);
+    if (x->stage_pending >= 0) {
+        CK(cudaEventRecord(x->stage_free[x->stage_pending], x->stream));
+        x->stage_pending = -1;
+    }
+    const size_t off_bytes = sizeof(int64_t) * (S + 1);
+    const size_t need = off_bytes + nbytes;
+    if (need > x->pk_cap[k]) {
+        // sized for full frames of one detected-points TLV per scene at first use; a growth waits for the step that
+        // last read the buffer
+        const size_t full = off_bytes + (size_t)S * (kTlvHeader + 12 + 12 * (size_t)x->ncap);
+        const size_t bytes = std::max(need + need / 4, full);
+        CK(cudaEventSynchronize(x->stage_free[k]));
+        if (x->d_pk2[k]) { CK(cudaFree(x->d_pk2[k])); x->d_pk2[k] = nullptr; x->pk_cap[k] = 0; }
+        CK(cudaMalloc((void**)&x->d_pk2[k], bytes));
+        x->pk_cap[k] = bytes;
+    }
+    x->stage_idx++;
+    CK(cudaStreamWaitEvent(x->h2d_stream, x->stage_free[k], 0));
+    CK(cudaMemcpyAsync(x->d_pk2[k], packet_offsets, off_bytes, cudaMemcpyHostToDevice, x->h2d_stream));
+    if (nbytes) CK(cudaMemcpyAsync(x->d_pk2[k] + off_bytes, packets, nbytes, cudaMemcpyHostToDevice, x->h2d_stream));
+    x->h_offsets = rows;
+    // pageable source: staged before the call returns
+    CK(cudaMemcpyAsync(x->d_offsets2[k], x->h_offsets.data(), sizeof(int32_t) * (S + 1), cudaMemcpyHostToDevice,
+                       x->h2d_stream));
+    CK(cudaMemcpyAsync(x->d_dt2[k], dt, sizeof(double) * S, cudaMemcpyHostToDevice, x->h2d_stream));
+    CK(cudaEventRecord(x->h2d_done[k], x->h2d_stream));
+    CK(cudaStreamWaitEvent(x->stream, x->h2d_done[k], 0));
+    // Decode straight into the fp32 staging the step reads (it keeps the slack of the step's aligned windows): rows
+    // carry dopplerIdx (factor 1), corrected with each scene's own threshold.
+    if (total) {
+        prof_mark(x, MMW_K_PACKETS);
+        tlv_decode_kernel<<<(unsigned)((32LL * S + 255) / 256), 256, 0, x->stream>>>(
+            x->d_pk2[k] + off_bytes, reinterpret_cast<const long long*>(x->d_pk2[k]), S, x->d_offsets2[k], 0.0,
+            x->d_doppler_wrap, 1.0, x->d_pts2[k]);
+        CK(cudaGetLastError());
+        x->launches++;
+        prof_mark(x, -1);
+    }
+    StepArgs a;
+    a.cfg = x->dc;
+    a.sensors = x->d_sensors;
+    a.pts = x->d_pts2[k]; a.offsets = x->d_offsets2[k]; a.dt = x->d_dt2[k];
+    return step_queue(x, a, flags, k);
 }
 
 int mmw_export_track0(mmw_ctx* x, double* rows, int32_t* valid, double* centroid) {
