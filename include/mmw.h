@@ -190,6 +190,7 @@ int mmw_load_pose_weights(mmw_ctx* ctx, int variant, const float* blob, size_t n
  *   dt      [S]        fp64 seconds since the scene's previous frame (trackbuffer.dt, offline_main.py:45-49)
  * Scenes whose frame is empty after the scene-bounds filter are skipped entirely, as offline_main.py:55 does.
  * Asynchronous on the context's stream unless the inputs are pageable host memory.
+ * The flags are checked before the inputs, and a refused call queues nothing.
  */
 int mmw_step(mmw_ctx* ctx, const float* pts, const int32_t* offsets, const double* dt, uint32_t flags);
 

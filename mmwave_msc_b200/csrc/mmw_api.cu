@@ -34,6 +34,23 @@ static int fail(int code, const std::string& msg) {
             return fail(MMW_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e__));        \
     } while (0)
 
+// mmw_run_frames uploads the inputs of kGroup consecutive frames in ONE copy per array (a 2 MB copy runs at 15 GB/s on a
+// link that gives 24 GB/s at 8 MB: per-copy cost, not bandwidth)
+constexpr int kGroup = 4;
+constexpr size_t kStageSlack = 64;   // the step kernel copies 16-byte aligned windows around a scene's rows
+
+// One slot of the input staging of the host-input entry points (see stage_acquire): the inputs of one step, or of a
+// group of up to kGroup frames.
+struct StageSlot {
+    float* pts = nullptr;            // point rows (fp32, or int16 with MMW_STEP_INPUT_I16) of the step or group
+    size_t pts_cap = 0;              //   bytes, kStageSlack included
+    int32_t* offsets = nullptr;      // [kGroup][S+1]
+    double* dt = nullptr;            // [kGroup][S]
+    uint8_t* pk = nullptr;           // mmw_step_packets: [S+1] packet offsets (int64) + packet bytes
+    size_t pk_cap = 0;
+    cudaEvent_t uploaded = nullptr, free = nullptr;
+};
+
 struct mmw_ctx {
     mmw_config cfg;
     DevConfig dc;
@@ -63,22 +80,11 @@ struct mmw_ctx {
     int32_t* d_scene_stats = nullptr; // [S][8] per-scene counters of the last step (summed on the device)
     int32_t* d_defer = nullptr;      // [2 + S + S]: counter, the work list of dbscan_big_kernel, pose rows per scene, finished-CTA ticket
     bool fold_pose_index = true;     // pose-row scan inside pose_feature_kernel (S <= 4096) instead of pose_index_kernel
-    // input staging (host-input path): double-buffered, copied on a side stream so that the upload of frame k+1
-    // overlaps the kernels of frame k
-    float* d_pts2[2] = {nullptr, nullptr};
-    int32_t* d_offsets2[2] = {nullptr, nullptr};
-    double* d_dt2[2] = {nullptr, nullptr};
-    uint8_t* d_pk2[2] = {nullptr, nullptr};   // mmw_step_packets: [S+1] packet offsets (int64) + packet bytes, same buffers
-    size_t pk_cap[2] = {0, 0};                //   index and events as the fp32 staging; grown on demand
+    // input staging of the host-input entry points, copied on a side stream (see stage_acquire)
+    StageSlot stage[2];
+    unsigned stage_idx = 0;          // slots taken so far
+    unsigned stage_pending = 0;      // bit k: slot k is released, its free event is still to be recorded
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;
-    // mmw_run_frames: the inputs of kGroup consecutive frames go up in ONE copy per array (a 2 MB copy runs at 15 GB/s
-    // on a link that gives 24 GB/s at 8 MB: per-copy cost, not bandwidth), double-buffered by group
-    void* d_ptsG[2] = {nullptr, nullptr};
-    size_t ptsG_cap = 0;
-    int32_t* d_offG[2] = {nullptr, nullptr};
-    double* d_dtG[2] = {nullptr, nullptr};
-    cudaEvent_t h2dG_done[2] = {nullptr, nullptr}, stageG_free[2] = {nullptr, nullptr};
-    long long dev_row0 = 0;          // StepArgs::pts_row0 of the next MMW_STEP_DEVICE_INPUT step (reset by it)
     // throughput mode (MMW_STEP_PIPELINE): pose network on its own stream, its inputs double-buffered
     cudaStream_t pose_stream = nullptr;
     cudaEvent_t feat_done[2] = {nullptr, nullptr}, packt_done[2] = {nullptr, nullptr}, pose_done[2] = {nullptr, nullptr};
@@ -89,14 +95,11 @@ struct mmw_ctx {
     unsigned pipe_idx = 0;           // pipelined steps so far
     int pipe_r = -1;                 // result buffer the last step filled itself (-1: the last step was serial)
     bool pose_pending = false;       // the pose stream has work the main stream has not waited for
-    cudaEvent_t h2d_done[2] = {nullptr, nullptr}, stage_free[2] = {nullptr, nullptr};
-    int stage_pending = -1;              // staging buffer whose stage_free event is still to be recorded
     cudaEvent_t packed[2] = {nullptr, nullptr}, results_done[2] = {nullptr, nullptr};
     float* d_results[2] = {nullptr, nullptr};
     double* d_export = nullptr;      // [S][192*5 + 2] rows + centroid of mmw_export_track0 (allocated on first use)
     int32_t* d_export_valid = nullptr;
-    unsigned stage_idx = 0, result_idx = 0;
-    std::vector<int32_t> h_offsets;
+    unsigned result_idx = 0;
     // pose
     int variant = -1;
     bool has_weights = false;
@@ -243,9 +246,9 @@ int mmw_destroy(mmw_ctx* x) {
     if (!x) return MMW_OK;
     cudaSetDevice(x->device);
     if (x->stream) cudaStreamSynchronize(x->stream);
-    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_pk2[0], x->d_pk2[1], x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
-                    x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist, x->d_pts2[0], x->d_pts2[1], x->d_offsets2[0],
-                    x->d_offsets2[1], x->d_dt2[0], x->d_dt2[1], x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
+    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
+                    x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist,
+                    x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
                     x->d_bn1t, x->d_bn2s, x->d_bn2t, x->d_feats, x->d_row_scene, x->d_row_track, x->d_row_slot,
                     x->d_pose_total, x->d_act2, x->d_act3, x->d_pose_out, x->d_row_scene2, x->d_row_track2, x->d_row_slot2,
                     x->d_pose_total2, x->d_pose_extra};
@@ -255,16 +258,13 @@ int mmw_destroy(mmw_ctx* x) {
     if (x->h_defer_hint) cudaFreeHost(x->h_defer_hint);
     if (x->h_rows_hint) cudaFreeHost(x->h_rows_hint);
     for (int i = 0; i < 2; ++i) {
-        if (x->d_ptsG[i]) cudaFree(x->d_ptsG[i]);
-        if (x->d_offG[i]) cudaFree(x->d_offG[i]);
-        if (x->d_dtG[i]) cudaFree(x->d_dtG[i]);
-        if (x->h2dG_done[i]) cudaEventDestroy(x->h2dG_done[i]);
-        if (x->stageG_free[i]) cudaEventDestroy(x->stageG_free[i]);
-    }
-    for (int i = 0; i < 2; ++i)
-        for (cudaEvent_t e : {x->h2d_done[i], x->stage_free[i], x->packed[i], x->results_done[i], x->feat_done[i],
-                              x->packt_done[i], x->pose_done[i]})
+        const StageSlot& s = x->stage[i];
+        for (void* p : {(void*)s.pts, (void*)s.offsets, (void*)s.dt, (void*)s.pk})
+            if (p) cudaFree(p);
+        for (cudaEvent_t e : {s.uploaded, s.free, x->packed[i], x->results_done[i], x->feat_done[i], x->packt_done[i],
+                              x->pose_done[i]})
             if (e) cudaEventDestroy(e);
+    }
     if (x->h2d_stream) cudaStreamDestroy(x->h2d_stream);
     if (x->d2h_stream) cudaStreamDestroy(x->d2h_stream);
     if (x->pose_stream) { cudaStreamSynchronize(x->pose_stream); cudaStreamDestroy(x->pose_stream); }
@@ -425,12 +425,14 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
         x->fold_pose_index = S <= 4096 && !(env && env[0] == '0');
     }
     for (int i = 0; i < 2; ++i) {
-        ALLOC(x->d_pts2[i], sizeof(float) * kRawCols * S * max_points + 16);
-        ALLOC(x->d_offsets2[i], sizeof(int32_t) * (S + 1));
-        ALLOC(x->d_dt2[i], sizeof(double) * S);
+        StageSlot& st = x->stage[i];
+        st.pts_cap = sizeof(float) * kRawCols * S * max_points + kStageSlack;      // one full frame (run_frames grows it)
+        ALLOC(st.pts, st.pts_cap);
+        ALLOC(st.offsets, sizeof(int32_t) * kGroup * (S + 1));
+        ALLOC(st.dt, sizeof(double) * kGroup * S);
         ALLOC(x->d_results[i], sizeof(float) * S * max_tracks * MMW_RESULT_FLOATS);
-        if (cudaEventCreateWithFlags(&x->h2d_done[i], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&x->stage_free[i], cudaEventDisableTiming) != cudaSuccess ||
+        if (cudaEventCreateWithFlags(&st.uploaded, cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&st.free, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->packed[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->results_done[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&x->feat_done[i], cudaEventDisableTiming) != cudaSuccess ||
@@ -705,59 +707,103 @@ static int launch_feature_stage(mmw_ctx* x, int b, bool late, cudaStream_t st) {
     return MMW_OK;
 }
 
-static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage);
+// The flag checks of every step entry point, made before anything is queued.
+static int check_step_flags(const mmw_ctx* x, uint32_t flags) {
+    if ((flags & MMW_STEP_POSE) && !x->has_weights)
+        return fail(MMW_ERR_STATE, "MMW_STEP_POSE needs mmw_load_pose_weights first");
+    if ((flags & MMW_STEP_PIPELINE) && (!(flags & MMW_STEP_POSE) || !(x->use_tc && x->tc.ready)))
+        return fail(MMW_ERR_STATE, "MMW_STEP_PIPELINE needs MMW_STEP_POSE and the tensor-core pose path");
+    if ((flags & MMW_STEP_PIPELINE) && (flags & MMW_STEP_RECORD_LABELS))
+        return fail(MMW_ERR_INVALID, "MMW_STEP_PIPELINE cannot record labels");
+    return MMW_OK;
+}
+
+// The number of rows of a frame's offsets [S+1], or -1 unless offsets[0] == 0 and they do not decrease.
+static long long offsets_total(const int32_t* offsets, int S) {
+    if (offsets[0] != 0) return -1;
+    for (int i = 0; i < S; ++i)
+        if (offsets[i] > offsets[i + 1]) return -1;
+    return offsets[S];
+}
+
+// ---- input staging: a ring of two slots, filled on the upload stream so that the upload of the next step (or group
+// of frames) overlaps the kernels of this one.  A slot is free once the steps that read it have run.  That event is
+// recorded at the head of the NEXT acquire, where the main stream has to wait for an upload anyway -- not behind a
+// step's last kernel, where it would sit between dense 2 and the result pack and undo their dependent launch.
+
+static cudaError_t grow(void** buf, size_t* cap, size_t bytes) {
+    if (bytes <= *cap) return cudaSuccess;
+    cudaError_t e = cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    if (e == cudaSuccess && (e = cudaMalloc(buf, bytes)) == cudaSuccess) *cap = bytes;
+    return e;
+}
+
+// Takes the next slot (*k) for pts_bytes of point rows and pk_bytes of packets, and makes the upload stream wait until
+// the slot is free.  A slot that is too small is reallocated once the steps that last read it are done.
+static int stage_acquire(mmw_ctx* x, size_t pts_bytes, size_t pk_bytes, int* k) {
+    for (int i = 0; i < 2; ++i)
+        if (x->stage_pending & (1u << i)) CK(cudaEventRecord(x->stage[i].free, x->stream));
+    x->stage_pending = 0;
+    *k = (int)(x->stage_idx++ & 1u);
+    StageSlot& s = x->stage[*k];
+    if (pts_bytes + kStageSlack > s.pts_cap || pk_bytes > s.pk_cap) {
+        CK(cudaEventSynchronize(s.free));
+        CK(grow((void**)&s.pts, &s.pts_cap, pts_bytes + kStageSlack));
+        CK(grow((void**)&s.pk, &s.pk_cap, pk_bytes));
+    }
+    CK(cudaStreamWaitEvent(x->h2d_stream, s.free, 0));
+    return MMW_OK;
+}
+
+// The slot's uploads are queued: the main stream waits for them.
+static int stage_submit(mmw_ctx* x, int k) {
+    CK(cudaEventRecord(x->stage[k].uploaded, x->h2d_stream));
+    CK(cudaStreamWaitEvent(x->stream, x->stage[k].uploaded, 0));
+    return MMW_OK;
+}
+
+// Every step that reads the slot is queued: its free event is recorded by the next stage_acquire.
+static void stage_release(mmw_ctx* x, int k) { x->stage_pending |= 1u << k; }
+
+static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags);
 
 int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double* dt, uint32_t flags) {
     if (!x || !offsets || !dt) return fail(MMW_ERR_INVALID, "ctx/offsets/dt is NULL");
-    if ((flags & MMW_STEP_POSE) && !x->has_weights)
-        return fail(MMW_ERR_STATE, "MMW_STEP_POSE needs mmw_load_pose_weights first");
+    if ((flags & MMW_STEP_DEVICE_INPUT) && !pts) return fail(MMW_ERR_INVALID, "pts is NULL");
+    int rc = check_step_flags(x, flags);
+    if (rc != MMW_OK) return rc;
     CK(cudaSetDevice(x->device));
     StepArgs a;
-    a.cfg = x->dc;
-    a.sensors = x->d_sensors;
-    int host_stage = -1;
     if (flags & MMW_STEP_DEVICE_INPUT) {
-        if (!pts) return fail(MMW_ERR_INVALID, "pts is NULL");
         a.pts = pts; a.offsets = offsets; a.dt = dt;
-        a.pts_row0 = x->dev_row0;
-        x->dev_row0 = 0;
-    } else {
-        const size_t total = (size_t)offsets[x->S];
-        if (offsets[0] != 0) return fail(MMW_ERR_INVALID, "offsets[0] must be 0");
-        if (total > (size_t)x->S * x->ncap)
-            return fail(MMW_ERR_CAPACITY, "more points than n_scenes * max_points_per_frame");
-        if (total > 0 && !pts) return fail(MMW_ERR_INVALID, "pts is NULL");
-        for (int i = 0; i < x->S; ++i)
-            if (offsets[i] < 0 || offsets[i] > offsets[i + 1])
-                return fail(MMW_ERR_INVALID, "offsets must be non-negative and non-decreasing");
-        const int k = (int)(x->stage_idx++ & 1u);
-        // The staging buffer is free once the step kernel that last read it has run.  That event is recorded here, at
-        // the head of the NEXT step, where the stream has to wait for the upload anyway -- not behind the previous
-        // step's last kernel, where it would sit between dense 2 and the result pack and undo their dependent launch.
-        if (x->stage_pending >= 0) {
-            CK(cudaEventRecord(x->stage_free[x->stage_pending], x->stream));
-            x->stage_pending = -1;
-        }
-        CK(cudaStreamWaitEvent(x->h2d_stream, x->stage_free[k], 0));
-        if (total)
-            CK(cudaMemcpyAsync(x->d_pts2[k], pts, ((flags & MMW_STEP_INPUT_I16) ? sizeof(int16_t) : sizeof(float)) * kRawCols * total,
-                               cudaMemcpyHostToDevice, x->h2d_stream));
-        CK(cudaMemcpyAsync(x->d_offsets2[k], offsets, sizeof(int32_t) * (x->S + 1), cudaMemcpyHostToDevice,
-                           x->h2d_stream));
-        CK(cudaMemcpyAsync(x->d_dt2[k], dt, sizeof(double) * x->S, cudaMemcpyHostToDevice, x->h2d_stream));
-        CK(cudaEventRecord(x->h2d_done[k], x->h2d_stream));
-        CK(cudaStreamWaitEvent(x->stream, x->h2d_done[k], 0));
-        x->h_offsets.assign(offsets, offsets + x->S + 1);
-        a.pts = x->d_pts2[k]; a.offsets = x->d_offsets2[k]; a.dt = x->d_dt2[k];
-        host_stage = k;
+        return step_queue(x, a, flags);
     }
-    return step_queue(x, a, flags, host_stage);
+    const long long total = offsets_total(offsets, x->S);
+    if (total < 0) return fail(MMW_ERR_INVALID, "offsets must start at 0 and must not decrease");
+    if (total > (long long)x->S * x->ncap)
+        return fail(MMW_ERR_CAPACITY, "more points than n_scenes * max_points_per_frame");
+    if (total > 0 && !pts) return fail(MMW_ERR_INVALID, "pts is NULL");
+    const size_t bytes = ((flags & MMW_STEP_INPUT_I16) ? sizeof(int16_t) : sizeof(float)) * kRawCols * total;
+    int k;
+    if ((rc = stage_acquire(x, bytes, 0, &k)) != MMW_OK) return rc;
+    const StageSlot& s = x->stage[k];
+    if (total) CK(cudaMemcpyAsync(s.pts, pts, bytes, cudaMemcpyHostToDevice, x->h2d_stream));
+    CK(cudaMemcpyAsync(s.offsets, offsets, sizeof(int32_t) * (x->S + 1), cudaMemcpyHostToDevice, x->h2d_stream));
+    CK(cudaMemcpyAsync(s.dt, dt, sizeof(double) * x->S, cudaMemcpyHostToDevice, x->h2d_stream));
+    if ((rc = stage_submit(x, k)) != MMW_OK) return rc;
+    a.pts = s.pts; a.offsets = s.offsets; a.dt = s.dt;
+    rc = step_queue(x, a, flags);
+    stage_release(x, k);
+    return rc;
 }
 
-// The tracker kernels of a step whose inputs a.pts / a.offsets / a.dt are in place, then its pose stage.  host_stage:
-// the input staging buffer they were uploaded into (its stage_free event is recorded at the head of the next step), or
-// -1 for device-resident input.
-static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage) {
+// The tracker kernels of a step whose inputs a.pts / a.offsets / a.dt / a.pts_row0 are in place, then its pose stage.
+// The flags have passed check_step_flags.
+static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags) {
+    a.cfg = x->dc;
+    a.sensors = x->d_sensors;
     a.tracks = x->d_tracks; a.scenes = x->d_scenes; a.track_ring = x->d_track_ring; a.uring = x->d_uring;
     a.keypoints = x->d_keypoints; a.default_posture = x->d_default_posture; a.assoc_out = x->d_assoc;
     a.labels_out = (flags & MMW_STEP_RECORD_LABELS) ? x->d_labels : nullptr;
@@ -785,9 +831,6 @@ static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage) {
         a.nr_extra = x->d_pose_extra;
     }
     if (pipelined) {
-        if (!(flags & MMW_STEP_POSE) || !(x->use_tc && x->tc.ready))
-            return fail(MMW_ERR_STATE, "MMW_STEP_PIPELINE needs MMW_STEP_POSE and the tensor-core pose path");
-        if (flags & MMW_STEP_RECORD_LABELS) return fail(MMW_ERR_INVALID, "MMW_STEP_PIPELINE cannot record labels");
         // frame k-2 used the same pose inputs / row maps (buffer k & 1): its pose network must be done before
         // dbscan_big_kernel appends rows and the feature kernel fills them.  Queued in front of the tracker kernels (not
         // between dbscan_big_kernel and the feature kernel, whose dependent launch it would undo); already satisfied in
@@ -804,11 +847,9 @@ static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags, int host_stage) {
     CK(launch_dbscan_big(a, x->stream, x->h_defer_hint ? *(volatile int32_t*)x->h_defer_hint : 16));
     x->launches += 2;          // step_kernel + dbscan_big_kernel
     prof_mark(x, -1);
-    int rc = MMW_OK;
-    if (pipelined) rc = pipeline_pose(x);
-    else if (flags & MMW_STEP_POSE) rc = estimate_posture_impl(x, late);
-    if (host_stage >= 0) x->stage_pending = host_stage;      // recorded at the head of the next step (see above)
-    return rc;
+    if (pipelined) return pipeline_pose(x);
+    if (flags & MMW_STEP_POSE) return estimate_posture_impl(x, late);
+    return MMW_OK;
 }
 
 int mmw_estimate_posture(mmw_ctx* x) { return estimate_posture_impl(x, false); }
@@ -1442,13 +1483,8 @@ int mmw_step_packets(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_o
     if (!x || !packet_offsets || !dt) return fail(MMW_ERR_INVALID, "ctx/packet_offsets/dt is NULL");
     if (flags & (MMW_STEP_DEVICE_INPUT | MMW_STEP_INPUT_I16))
         return fail(MMW_ERR_INVALID, "mmw_step_packets takes host packets: MMW_STEP_DEVICE_INPUT / MMW_STEP_INPUT_I16 do not apply");
-    if ((flags & MMW_STEP_POSE) && !x->has_weights)
-        return fail(MMW_ERR_STATE, "MMW_STEP_POSE needs mmw_load_pose_weights first");
-    // the flag checks of step_queue, made here so that a refused call has queued nothing
-    if ((flags & MMW_STEP_PIPELINE) && (!(flags & MMW_STEP_POSE) || !(x->use_tc && x->tc.ready)))
-        return fail(MMW_ERR_STATE, "MMW_STEP_PIPELINE needs MMW_STEP_POSE and the tensor-core pose path");
-    if ((flags & MMW_STEP_PIPELINE) && (flags & MMW_STEP_RECORD_LABELS))
-        return fail(MMW_ERR_INVALID, "MMW_STEP_PIPELINE cannot record labels");
+    int rc = check_step_flags(x, flags);
+    if (rc != MMW_OK) return rc;
     const int S = x->S;
     if (packet_offsets[0] != 0) return fail(MMW_ERR_INVALID, "packet_offsets[0] must be 0");
     for (int s = 0; s < S; ++s)
@@ -1477,52 +1513,35 @@ int mmw_step_packets(mmw_ctx* x, const uint8_t* packets, const int64_t* packet_o
         if (data_ok) data_ok[s] = rows[s + 1] > rows[s] ? 1 : 0;
     }
     CK(cudaSetDevice(x->device));
-    // Upload into the staging buffers of this step (see mmw_step): [S+1] packet offsets and the packet bytes into byte
-    // staging k, the row offsets and dt into d_offsets2[k] / d_dt2[k].
-    const int k = (int)(x->stage_idx & 1u);
-    if (x->stage_pending >= 0) {
-        CK(cudaEventRecord(x->stage_free[x->stage_pending], x->stream));
-        x->stage_pending = -1;
-    }
+    // [S+1] packet offsets and the packet bytes go into the slot's packet staging, sized for full frames of one
+    // detected-points TLV per scene at first use; the row offsets and dt as for mmw_step.
     const size_t off_bytes = sizeof(int64_t) * (S + 1);
-    const size_t need = off_bytes + nbytes;
-    if (need > x->pk_cap[k]) {
-        // sized for full frames of one detected-points TLV per scene at first use; a growth waits for the step that
-        // last read the buffer
-        const size_t full = off_bytes + (size_t)S * (kTlvHeader + 12 + 12 * (size_t)x->ncap);
-        const size_t bytes = std::max(need + need / 4, full);
-        CK(cudaEventSynchronize(x->stage_free[k]));
-        if (x->d_pk2[k]) { CK(cudaFree(x->d_pk2[k])); x->d_pk2[k] = nullptr; x->pk_cap[k] = 0; }
-        CK(cudaMalloc((void**)&x->d_pk2[k], bytes));
-        x->pk_cap[k] = bytes;
-    }
-    x->stage_idx++;
-    CK(cudaStreamWaitEvent(x->h2d_stream, x->stage_free[k], 0));
-    CK(cudaMemcpyAsync(x->d_pk2[k], packet_offsets, off_bytes, cudaMemcpyHostToDevice, x->h2d_stream));
-    if (nbytes) CK(cudaMemcpyAsync(x->d_pk2[k] + off_bytes, packets, nbytes, cudaMemcpyHostToDevice, x->h2d_stream));
-    x->h_offsets = rows;
+    const size_t full = off_bytes + (size_t)S * (kTlvHeader + 12 + 12 * (size_t)x->ncap);
+    int k;
+    if ((rc = stage_acquire(x, sizeof(float) * kRawCols * total, std::max(off_bytes + nbytes, full), &k)) != MMW_OK) return rc;
+    const StageSlot& st = x->stage[k];
+    CK(cudaMemcpyAsync(st.pk, packet_offsets, off_bytes, cudaMemcpyHostToDevice, x->h2d_stream));
+    if (nbytes) CK(cudaMemcpyAsync(st.pk + off_bytes, packets, nbytes, cudaMemcpyHostToDevice, x->h2d_stream));
     // pageable source: staged before the call returns
-    CK(cudaMemcpyAsync(x->d_offsets2[k], x->h_offsets.data(), sizeof(int32_t) * (S + 1), cudaMemcpyHostToDevice,
-                       x->h2d_stream));
-    CK(cudaMemcpyAsync(x->d_dt2[k], dt, sizeof(double) * S, cudaMemcpyHostToDevice, x->h2d_stream));
-    CK(cudaEventRecord(x->h2d_done[k], x->h2d_stream));
-    CK(cudaStreamWaitEvent(x->stream, x->h2d_done[k], 0));
-    // Decode straight into the fp32 staging the step reads (it keeps the slack of the step's aligned windows): rows
-    // carry dopplerIdx (factor 1), corrected with each scene's own threshold.
+    CK(cudaMemcpyAsync(st.offsets, rows.data(), sizeof(int32_t) * (S + 1), cudaMemcpyHostToDevice, x->h2d_stream));
+    CK(cudaMemcpyAsync(st.dt, dt, sizeof(double) * S, cudaMemcpyHostToDevice, x->h2d_stream));
+    if ((rc = stage_submit(x, k)) != MMW_OK) return rc;
+    // Decode straight into the fp32 rows the step reads: rows carry dopplerIdx (factor 1), corrected with each scene's
+    // own threshold.
     if (total) {
         prof_mark(x, MMW_K_PACKETS);
         tlv_decode_kernel<<<(unsigned)((32LL * S + 255) / 256), 256, 0, x->stream>>>(
-            x->d_pk2[k] + off_bytes, reinterpret_cast<const long long*>(x->d_pk2[k]), S, x->d_offsets2[k], 0.0,
-            x->d_doppler_wrap, 1.0, x->d_pts2[k]);
+            st.pk + off_bytes, reinterpret_cast<const long long*>(st.pk), S, st.offsets, 0.0, x->d_doppler_wrap, 1.0,
+            st.pts);
         CK(cudaGetLastError());
         x->launches++;
         prof_mark(x, -1);
     }
     StepArgs a;
-    a.cfg = x->dc;
-    a.sensors = x->d_sensors;
-    a.pts = x->d_pts2[k]; a.offsets = x->d_offsets2[k]; a.dt = x->d_dt2[k];
-    return step_queue(x, a, flags, k);
+    a.pts = st.pts; a.offsets = st.offsets; a.dt = st.dt;
+    rc = step_queue(x, a, flags);
+    stage_release(x, k);
+    return rc;
 }
 
 int mmw_export_track0(mmw_ctx* x, double* rows, int32_t* valid, double* centroid) {
@@ -1730,18 +1749,17 @@ static int run_frames_impl(mmw_ctx* x, int n_frames, const void* pts, const int6
     if (n_frames < 0) return fail(MMW_ERR_INVALID, "n_frames must not be negative");
     if (flags & (MMW_STEP_DEVICE_INPUT | MMW_STEP_RECORD_LABELS))
         return fail(MMW_ERR_INVALID, "mmw_run_frames takes host buffers and does not record labels");
+    int rc = check_step_flags(x, flags);
+    if (rc != MMW_OK) return rc;
     const size_t row_bytes = (flags & MMW_STEP_INPUT_I16) ? sizeof(int16_t) * kRawCols : sizeof(float) * kRawCols;
     const size_t per_frame = (size_t)x->S * x->tcap * MMW_RESULT_FLOATS;
     // Every frame has its own host buffers, so the host never has to wait for a frame's results before queueing the
     // next one -- the device-side buffers (input staging, pose inputs, result records) are handed over by stream
     // events.  The host only keeps the queue bounded: at most kAhead frames in flight.  (Waiting for frame f-1 before
     // queueing f+1 would put the upload of f+1 behind the download of f-1 and leave the pose stream idle for a
-    // third of every frame.)
-    constexpr int kAheadMax = 8;
-    // timing experiments only: MMW_RUN_AHEAD = frames in flight (default 4), MMW_RUN_NODL = 1 leaves the results on the device
-    static const int kAhead = [] { const char* e = getenv("MMW_RUN_AHEAD"); const int v = e ? atoi(e) : 4; return v < 1 ? 1 : (v > kAheadMax ? kAheadMax : v); }();
-    static const bool no_download = [] { const char* e = getenv("MMW_RUN_NODL"); return e && atoi(e) != 0; }();
-    cudaEvent_t done[kAheadMax] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // third of every frame.  2 to 8 frames in flight measured the same: profiles/r02_e2e_variants2.txt.)
+    constexpr int kAhead = 4;
+    cudaEvent_t done[kAhead] = {nullptr, nullptr, nullptr, nullptr};
     CK(cudaSetDevice(x->device));
     float* dev_results = nullptr;
     int32_t* dev_counts = nullptr;
@@ -1753,85 +1771,60 @@ static int run_frames_impl(mmw_ctx* x, int n_frames, const void* pts, const int6
             return fail(MMW_ERR_INVALID, "mmw_run_frames_compact needs results and n_records in pinned (device-mapped) host memory");
         }
     }
+    for (int f = 0; f < n_frames; ++f)
+        if (frame_row_offsets[f + 1] < frame_row_offsets[f]) return fail(MMW_ERR_INVALID, "frame_row_offsets must not decrease");
     for (int i = 0; i < kAhead; ++i) CK(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming));
-    // ---- input staging by groups of kGroup frames -----------------------------------------------------------
-    constexpr int kGroup = 4;
+    // The inputs of each group of kGroup frames go up into one staging slot, under the kernels of the group before.
+    // The first call grows the slots to kGroup full frames (no re-allocation -- and no device synchronisation -- when a
+    // later call brings more points).
     const int n_groups = (n_frames + kGroup - 1) / kGroup;
-    {
-        size_t need = 0;
-        for (int g = 0; g < n_groups; ++g) {
-            const int f0 = g * kGroup, f1 = f0 + kGroup < n_frames ? f0 + kGroup : n_frames;
-            if (frame_row_offsets[f1] < frame_row_offsets[f0]) return fail(MMW_ERR_INVALID, "frame_row_offsets must not decrease");
-            const size_t b = (size_t)(frame_row_offsets[f1] - frame_row_offsets[f0]) * row_bytes;
-            if (b > need) need = b;
-        }
-        // sized for full frames once (no re-allocation -- and no device synchronisation -- when a later call brings more points)
-        const size_t cap_all = (size_t)kGroup * x->S * x->ncap * kRawCols * sizeof(float);
-        if (need < cap_all) need = cap_all;
-        need += 64;                      // the step kernel copies 16-byte aligned windows around a scene's rows
-        if (need > x->ptsG_cap || !x->d_offG[0]) {
-            CK(sync_main(x));
-            for (int i = 0; i < 2; ++i) {
-                if (x->d_ptsG[i]) { cudaFree(x->d_ptsG[i]); x->d_ptsG[i] = nullptr; }
-                CK(cudaMalloc(&x->d_ptsG[i], need));
-                if (!x->d_offG[i]) {
-                    CK(cudaMalloc((void**)&x->d_offG[i], sizeof(int32_t) * kGroup * (x->S + 1)));
-                    CK(cudaMalloc((void**)&x->d_dtG[i], sizeof(double) * kGroup * x->S));
-                    CK(cudaEventCreateWithFlags(&x->h2dG_done[i], cudaEventDisableTiming));
-                    CK(cudaEventCreateWithFlags(&x->stageG_free[i], cudaEventDisableTiming));
-                }
-            }
-            x->ptsG_cap = need;
-        }
-    }
-    auto upload_group = [&](int g) -> int {
-        const int k = g & 1, f0 = g * kGroup, f1 = f0 + kGroup < n_frames ? f0 + kGroup : n_frames;
+    const size_t full = (size_t)kGroup * x->S * x->ncap * kRawCols * sizeof(float);
+    auto upload_group = [&](int g, int* k) -> int {
+        const int f0 = g * kGroup, f1 = std::min(f0 + kGroup, n_frames);
         const size_t bytes = (size_t)(frame_row_offsets[f1] - frame_row_offsets[f0]) * row_bytes;
-        CK(cudaStreamWaitEvent(x->h2d_stream, x->stageG_free[k], 0));        // the group two back has been consumed
-        if (bytes) {
-            if (!pts) return fail(MMW_ERR_INVALID, "pts is NULL");
-            CK(cudaMemcpyAsync(x->d_ptsG[k], static_cast<const unsigned char*>(pts) + (size_t)frame_row_offsets[f0] * row_bytes,
+        if (bytes && !pts) return fail(MMW_ERR_INVALID, "pts is NULL");
+        const int rc = stage_acquire(x, std::max(bytes, full), 0, k);
+        if (rc != MMW_OK) return rc;
+        const StageSlot& s = x->stage[*k];
+        if (bytes)
+            CK(cudaMemcpyAsync(s.pts, static_cast<const unsigned char*>(pts) + (size_t)frame_row_offsets[f0] * row_bytes,
                                bytes, cudaMemcpyHostToDevice, x->h2d_stream));
-        }
-        CK(cudaMemcpyAsync(x->d_offG[k], offsets + (size_t)f0 * (x->S + 1), sizeof(int32_t) * (size_t)(f1 - f0) * (x->S + 1),
+        CK(cudaMemcpyAsync(s.offsets, offsets + (size_t)f0 * (x->S + 1), sizeof(int32_t) * (size_t)(f1 - f0) * (x->S + 1),
                            cudaMemcpyHostToDevice, x->h2d_stream));
-        CK(cudaMemcpyAsync(x->d_dtG[k], dt + (size_t)f0 * x->S, sizeof(double) * (size_t)(f1 - f0) * x->S,
+        CK(cudaMemcpyAsync(s.dt, dt + (size_t)f0 * x->S, sizeof(double) * (size_t)(f1 - f0) * x->S,
                            cudaMemcpyHostToDevice, x->h2d_stream));
-        CK(cudaEventRecord(x->h2dG_done[k], x->h2d_stream));
         return MMW_OK;
     };
-    int rc = n_groups > 0 ? upload_group(0) : MMW_OK;
+    int k = -1, next = -1;                  // slots of this group and of the next
+    rc = n_groups > 0 ? upload_group(0, &next) : MMW_OK;
     for (int f = 0; f < n_frames && rc == MMW_OK; ++f) {
-        const int g = f / kGroup, k = g & 1, f0 = g * kGroup;
+        const int g = f / kGroup, f0 = g * kGroup;
         if (f == f0) {
-            if (g + 1 < n_groups && (rc = upload_group(g + 1)) != MMW_OK) break;    // goes up under this group's kernels
-            if (cudaStreamWaitEvent(x->stream, x->h2dG_done[k], 0) != cudaSuccess) { rc = fail(MMW_ERR_CUDA, "cudaStreamWaitEvent failed"); break; }
+            if (k >= 0) stage_release(x, k);                // the previous group's last frame is queued
+            k = next;
+            if ((rc = stage_submit(x, k)) != MMW_OK) break;
+            if (g + 1 < n_groups && (rc = upload_group(g + 1, &next)) != MMW_OK) break;
         }
         if (f >= kAhead && cudaEventSynchronize(done[f % kAhead]) != cudaSuccess) { rc = fail(MMW_ERR_CUDA, "cudaEventSynchronize failed"); break; }
-        const int32_t* off = offsets + (size_t)f * (x->S + 1);
-        {
-            const size_t total = (size_t)off[x->S];
-            bool ok = off[0] == 0 && total <= (size_t)x->S * x->ncap &&
-                      total <= (size_t)(frame_row_offsets[f + 1] - frame_row_offsets[f]);
-            for (int i = 0; i < x->S && ok; ++i) ok = off[i] >= 0 && off[i] <= off[i + 1];
-            if (!ok) { rc = fail(MMW_ERR_INVALID, "mmw_run_frames: bad offsets (each frame: 0 = offsets[0] <= ... <= offsets[S] <= its rows, <= S * max_points)"); break; }
+        const long long total = offsets_total(offsets + (size_t)f * (x->S + 1), x->S);
+        if (total < 0 || total > (long long)x->S * x->ncap || total > frame_row_offsets[f + 1] - frame_row_offsets[f]) {
+            rc = fail(MMW_ERR_INVALID, "mmw_run_frames: bad offsets (each frame: 0 = offsets[0] <= ... <= offsets[S] <= its rows, <= S * max_points)");
+            break;
         }
-        x->dev_row0 = frame_row_offsets[f] - frame_row_offsets[f0];
-        rc = mmw_step(x, static_cast<const float*>(x->d_ptsG[k]), x->d_offG[k] + (size_t)(f - f0) * (x->S + 1),
-                      x->d_dtG[k] + (size_t)(f - f0) * x->S, flags | MMW_STEP_DEVICE_INPUT);
+        StepArgs a;
+        a.pts = x->stage[k].pts;
+        a.offsets = x->stage[k].offsets + (size_t)(f - f0) * (x->S + 1);
+        a.dt = x->stage[k].dt + (size_t)(f - f0) * x->S;
+        a.pts_row0 = frame_row_offsets[f] - frame_row_offsets[f0];
+        if ((rc = step_queue(x, a, flags)) != MMW_OK) break;
+        rc = read_results_impl(x, results + (size_t)f * per_frame, nullptr, compact ? dev_results + (size_t)f * per_frame : nullptr,
+                               compact ? dev_counts + f : nullptr);
         if (rc != MMW_OK) break;
-        x->h_offsets.assign(off, off + x->S + 1);
-        if ((f + 1 == n_frames || (f + 1) % kGroup == 0) &&
-            cudaEventRecord(x->stageG_free[k], x->stream) != cudaSuccess) { rc = fail(MMW_ERR_CUDA, "cudaEventRecord failed"); break; }
-        if (!no_download)
-            rc = read_results_impl(x, results + (size_t)f * per_frame, nullptr, compact ? dev_results + (size_t)f * per_frame : nullptr,
-                                   compact ? dev_counts + f : nullptr);
-        if (rc != MMW_OK) break;
-        if (cudaEventRecord(done[f % kAhead], no_download ? x->stream : x->d2h_stream) != cudaSuccess) rc = fail(MMW_ERR_CUDA, "cudaEventRecord failed");
+        if (cudaEventRecord(done[f % kAhead], x->d2h_stream) != cudaSuccess) rc = fail(MMW_ERR_CUDA, "cudaEventRecord failed");
     }
+    if (k >= 0) stage_release(x, k);
     if (cudaStreamSynchronize(x->d2h_stream) != cudaSuccess && rc == MMW_OK) rc = fail(MMW_ERR_CUDA, "cudaStreamSynchronize failed");
     for (int i = 0; i < kAhead; ++i) cudaEventDestroy(done[i]);
-    if (no_download && sync_main(x) != cudaSuccess && rc == MMW_OK) rc = fail(MMW_ERR_CUDA, "synchronisation failed");
     return rc;
 }
 

@@ -56,5 +56,4 @@ for rep in range(REPS + 1):
                       pipeline=not variant.endswith("_serial"))
     torch.cuda.synchronize()
     out.append((time.perf_counter() - t0) / K * 1e6)
-print("%-10s AHEAD=%s NODL=%s : us per frame %s (first = warm-up)" % (variant, os.environ.get("MMW_RUN_AHEAD", "4"),
-                                                                  os.environ.get("MMW_RUN_NODL", "0"), [round(v) for v in out]))
+print("%-10s : us per frame %s (first = warm-up)" % (variant, [round(v) for v in out]))
