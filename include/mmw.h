@@ -413,6 +413,19 @@ int mmw_get_counters(mmw_ctx* ctx, uint64_t out[8], int reset);
  * 0 = CUDA-core fp32 path (kept for numerics comparison). */
 int mmw_set_dense_path(mmw_ctx* ctx, int use_tensor_cores);
 
+/* Test hook: intermediates of the last pose-network run on the context's main stream (mmw_pose, or a serial
+ * mmw_step / mmw_estimate_posture with MMW_STEP_POSE), rows in that run's order, positions in Keras order (d, h, w, c):
+ *   layer 0: network input as split for the tensor cores    [n][D*64][5]
+ *   layer 1: conv 1 after ReLU                               [n][D*64][16]
+ *   layer 2: conv 2 after ReLU and BN 1 (the Flatten order)  [n][D*64*32]
+ *   layer 3: dense 1 after ReLU and BN 2                     [n][H]
+ * Tensor-core path: two uint16 planes of n * (values per row) each, the raw bf16 bits of hi, then of lo.  CUDA-core
+ * path: fp32, layers 2 and 3 only (MMW_ERR_INVALID for 0 and 1).  *n_rows = n of that run; host_out may be NULL to
+ * ask for n only, otherwise it must hold the whole layer (MMW_ERR_CAPACITY).  MMW_ERR_STATE: no weights loaded, no run
+ * since they were loaded (or since mmw_reset / mmw_pose_features_only), or the last run was in throughput mode (its
+ * intermediates belong to a frame that may still be in flight).  Synchronous. */
+int mmw_pose_intermediate(mmw_ctx* ctx, int layer, int* n_rows, void* host_out, size_t bytes);
+
 /* Per-kernel device time: while enabled, every launch of mmw_step / mmw_step_packets is bracketed by CUDA events on the context's
  * stream.  mmw_get_kernel_ms returns the accumulated milliseconds and launch counts per kernel class. */
 #define MMW_K_STEP 0           /* fused tracker step (normalize + track) */

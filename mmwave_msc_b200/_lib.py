@@ -133,6 +133,7 @@ SIGNATURES = {
     "mmw_run_frames_compact": (C.c_int, [_p, C.c_int, _p, _p, _p, _p, _p, _p, C.c_uint32]),
     "mmw_get_counters": (C.c_int, [_p, _p, C.c_int]),
     "mmw_set_dense_path": (C.c_int, [_p, C.c_int]),
+    "mmw_pose_intermediate": (C.c_int, [_p, C.c_int, C.POINTER(C.c_int), _p, C.c_size_t]),
     "mmw_profile": (C.c_int, [_p, C.c_int]),
     "mmw_get_kernel_ms": (C.c_int, [_p, _p, _p]),
     "mmw_phase_clocks": (C.c_int, [_p, C.c_int, _p]),

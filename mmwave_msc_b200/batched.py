@@ -161,6 +161,18 @@ class BatchedTracker:
     def set_dense_path(self, tensor_cores: bool):
         _lib.check(self.lib.mmw_set_dense_path(self._h, 1 if tensor_cores else 0))
 
+    def pose_intermediate(self, layer: int, tensor_cores: bool = True):
+        """Test hook: layer 0..3 of the last serial pose-network run (include/mmw.h, mmw_pose_intermediate), one row per
+        pose row, values in Keras order.  Tensor-core path: (hi, lo) uint16 arrays of the raw bf16 bits; CUDA-core path
+        (``tensor_cores=False``, layers 2 and 3): float32."""
+        n = C.c_int(0)
+        _lib.check(self.lib.mmw_pose_intermediate(self._h, int(layer), C.byref(n), None, 0))
+        D = self.cfg.frames_batch + 1
+        per = [D * 64 * 5, D * 64 * 16, D * 64 * 32, D * 512][layer]
+        out = np.zeros((2, n.value, per) if tensor_cores else (n.value, per), np.uint16 if tensor_cores else np.float32)
+        _lib.check(self.lib.mmw_pose_intermediate(self._h, int(layer), C.byref(n), _lib.ptr(out), out.nbytes))
+        return (out[0], out[1]) if tensor_cores else out
+
     # -- the hot path -----------------------------------------------------------------------------
     def step(self, points: np.ndarray, offsets: np.ndarray, dt: np.ndarray, pose: bool = True,
              record_labels: bool = False, pipeline: bool = False):

@@ -115,6 +115,9 @@ struct mmw_ctx {
     int pose_cap = 0;
     PoseTc tc;              // tensor-core dense path (pose_tc.cu)
     bool use_tc = true;
+    // the last pose-network run, for mmw_pose_intermediate: 0 = none (or its buffers were overwritten since),
+    // 1 = serial on the tensor cores, 2 = serial on the CUDA cores, 3 = throughput mode
+    int last_pose_run = 0;
     uint64_t launches = 0;
     // per-kernel CUDA-event profiling (mmw_profile)
     bool profiling = false;
@@ -278,6 +281,7 @@ int mmw_reset(mmw_ctx* x) {
     CK(cudaSetDevice(x->device));
     if (x->pose_stream) CK(join_pose(x));
     x->pipe_r = -1;
+    x->last_pose_run = 0;
     CK(cudaMemsetAsync(x->d_scenes, 0, sizeof(SceneRec) * x->S, x->stream));
     CK(cudaMemsetAsync(x->d_tracks, 0, sizeof(TrackRec) * (size_t)x->S * x->tcap, x->stream));
     CK(cudaMemsetAsync(x->d_counters, 0, sizeof(unsigned long long) * 8, x->stream));
@@ -591,6 +595,7 @@ int mmw_load_pose_weights(mmw_ctx* x, int variant, const float* blob, size_t n) 
     CK(cudaSetDevice(x->device));
     CK(sync_main(x));
     x->has_weights = false;              // a failed reload must not leave the old pointers in use
+    x->last_pose_run = 0;
     if (x->d_blob) { cudaFree(x->d_blob); x->d_blob = nullptr; }
     for (float** p : {&x->d_bn1s, &x->d_bn1t, &x->d_bn2s, &x->d_bn2t, &x->d_act2, &x->d_act3})
         if (*p) { cudaFree(*p); *p = nullptr; }
@@ -649,6 +654,7 @@ static int run_pose_tc(mmw_ctx* x, const PoseTcRun& r, int max_rows, int b, cuda
 }
 
 static int run_pose_net(mmw_ctx* x, float* keypoints_by_slot, int max_rows) {
+    x->last_pose_run = x->use_tc && x->tc.ready ? 1 : 2;
     if (x->use_tc && x->tc.ready) {
         PoseTcRun r{x->d_pose_total, x->b1, x->b2, x->d_bn1s, x->d_bn1t, x->bd1, x->d_bn2s, x->d_bn2t, x->bd2,
                     x->d_pose_out, keypoints_by_slot, x->d_row_scene, x->d_row_slot, x->tcap};
@@ -868,6 +874,7 @@ int mmw_pose_features_only(mmw_ctx* x) {
     if (!x) return fail(MMW_ERR_INVALID, "ctx is NULL");
     CK(cudaSetDevice(x->device));
     CK(join_pose(x));
+    x->last_pose_run = 0;                // the network input and the row count now belong to no run
     return launch_feature_stage(x, 0, false, x->stream);
 }
 
@@ -1397,6 +1404,7 @@ static int launch_pack_tracks(mmw_ctx* x, float* results) {
 static int pipeline_pose(mmw_ctx* x) {
     const int b = (int)(x->pipe_idx & 1u);
     cudaStream_t T = x->stream, P = x->pose_stream;
+    x->last_pose_run = 3;
     int rc = launch_feature_stage(x, b, false, T);
     if (rc != MMW_OK) return rc;
     CK(cudaEventRecord(x->feat_done[b], T));
@@ -2056,6 +2064,36 @@ int mmw_phase_clocks(mmw_ctx* x, int enable, uint64_t* out16) {
 int mmw_set_dense_path(mmw_ctx* x, int use_tensor_cores) {
     if (!x) return fail(MMW_ERR_INVALID, "ctx is NULL");
     x->use_tc = use_tensor_cores != 0;
+    return MMW_OK;
+}
+
+/* Test hook: the intermediates of the last serial pose-network run (include/mmw.h). */
+int mmw_pose_intermediate(mmw_ctx* x, int layer, int* n_rows, void* host_out, size_t bytes) {
+    if (!x || !n_rows) return fail(MMW_ERR_INVALID, "ctx/n_rows is NULL");
+    if (layer < 0 || layer > 3) return fail(MMW_ERR_INVALID, "layer must be 0..3");
+    if (!x->has_weights) return fail(MMW_ERR_STATE, "no pose weights loaded");
+    if (x->last_pose_run == 0) return fail(MMW_ERR_STATE, "no pose-network run since the weights were loaded");
+    if (x->last_pose_run == 3)
+        return fail(MMW_ERR_STATE, "the last pose-network run was in throughput mode (its frame may still be in flight)");
+    const bool tc = x->last_pose_run == 1;
+    if (!tc && layer < 2) return fail(MMW_ERR_INVALID, "the CUDA-core path keeps layers 2 and 3 only");
+    CK(cudaSetDevice(x->device));
+    CK(sync_main(x));
+    int n = 0;
+    CK(cudaMemcpy(&n, x->d_pose_total, sizeof(int), cudaMemcpyDeviceToHost));
+    *n_rows = n;
+    if (!host_out) return MMW_OK;
+    const size_t P = (size_t)x->D * 64;
+    const size_t per = layer == 0 ? P * 5 : layer == 1 ? P * 16 : layer == 2 ? (size_t)x->Kf : (size_t)x->H;
+    const size_t need = (size_t)n * per * (tc ? 2 * sizeof(uint16_t) : sizeof(float));
+    if (bytes < need) return fail(MMW_ERR_CAPACITY, "host_out too small for this layer");
+    if (n == 0) return MMW_OK;
+    if (tc) {
+        if (pose_tc_intermediate(&x->tc, layer, n, static_cast<uint16_t*>(host_out)) != 0)
+            return fail(MMW_ERR_CUDA, std::string("pose intermediate: ") + pose_tc_error());
+    } else {
+        CK(cudaMemcpy(host_out, layer == 2 ? x->d_act2 : x->d_act3, need, cudaMemcpyDeviceToHost));
+    }
     return MMW_OK;
 }
 

@@ -1225,6 +1225,43 @@ int pose_tc_fc2(PoseTc* t, const PoseTcRun& r, int max_rows, cudaStream_t st, in
     return 0;
 }
 
+int pose_tc_intermediate(PoseTc* t, int layer, int n, uint16_t* out) {
+    TcImpl* im = reinterpret_cast<TcImpl*>(t->impl);
+    if (!im || !t->ready) { g_tc_err = "tensor-core path not initialised"; return -1; }
+    const size_t P = (size_t)im->D * 64, rows = (size_t)n;
+    const size_t per = layer == 0 ? P * 5 : layer == 1 ? P * 16 : layer == 2 ? (size_t)im->Kf : (size_t)im->H;
+    uint16_t* lo_out = out + rows * per;
+    if (layer >= 2) {
+        const __nv_bfloat16* src[2] = {layer == 2 ? im->a_hi : im->h_hi, layer == 2 ? im->a_lo : im->h_lo};
+        for (int p = 0; p < 2; ++p)
+            if (cudaMemcpy(p ? lo_out : out, src[p], rows * per * 2, cudaMemcpyDeviceToHost) != cudaSuccess) {
+                g_tc_err = "cudaMemcpy (intermediate)";
+                return -1;
+            }
+        return 0;
+    }
+    // slab order [row][d][w][chunk][h][8]: the input has chunks (hi c0..4 | lo c0..4), conv 1's output
+    // (hi c0..7, hi c8..15, lo c0..7, lo c8..15)
+    const int nch = layer == 0 ? 2 : 4, cout = layer == 0 ? 5 : 16;
+    std::vector<uint16_t> h(rows * P * nch * 8);
+    if (cudaMemcpy(h.data(), layer == 0 ? im->in_p : im->act1_p, h.size() * 2, cudaMemcpyDeviceToHost) != cudaSuccess) {
+        g_tc_err = "cudaMemcpy (intermediate)";
+        return -1;
+    }
+    for (size_t r = 0; r < rows; ++r)
+        for (size_t pos = 0; pos < P; ++pos) {
+            const size_t d = pos / 64, hh = (pos / 8) % 8, w = pos % 8;
+            const size_t base = ((r * im->D + d) * 8 + w) * nch;
+            for (int c = 0; c < cout; ++c) {
+                const int chunk_hi = c / 8, chunk_lo = nch / 2 + c / 8;
+                const size_t o = (r * P + pos) * cout + c;
+                out[o] = h[((base + chunk_hi) * 8 + hh) * 8 + c % 8];
+                lo_out[o] = h[((base + chunk_lo) * 8 + hh) * 8 + c % 8];
+            }
+        }
+    return 0;
+}
+
 void pose_tc_free(PoseTc* t) {
     TcImpl* im = reinterpret_cast<TcImpl*>(t->impl);
     if (im) {

@@ -39,6 +39,9 @@ int pose_tc_conv(PoseTc* tc, const PoseTcRun& r, cudaStream_t st, int* n_launche
 // costs the least waves of CTA pairs times tile width -- speed only, the three kernels give the same bits
 int pose_tc_fc1(PoseTc* tc, const PoseTcRun& r, int max_rows, cudaStream_t st, int* n_launches, int rows_hint = 0);
 int pose_tc_fc2(PoseTc* tc, const PoseTcRun& r, int max_rows, cudaStream_t st, int* n_launches);
+// Test hook: layer 0..3 of the last run on input buffer 0, rows [0, n), positions in Keras order (d, h, w, c), as two
+// planes (bf16 hi bits, then lo bits) of n * per-row values each (mmw_pose_intermediate).  Synchronous.
+int pose_tc_intermediate(PoseTc* tc, int layer, int n, uint16_t* out);
 void pose_tc_free(PoseTc* tc);
 const char* pose_tc_error();
 
