@@ -25,9 +25,10 @@
 extern "C" {
 #endif
 
-/* 6: mmw_step_packets and mmw_scene_sensor::num_doppler_bins (5: per-scene sensor table and mmw_reset_scenes).  The
- * state blob carries this number, so blobs written by an earlier version are refused by mmw_state_restore. */
-#define MMW_ABI_VERSION 6
+/* 7: per-scene export / import (mmw_scene_blob_header, mmw_export_scenes, mmw_import_scenes) (6: mmw_step_packets and
+ * mmw_scene_sensor::num_doppler_bins; 5: per-scene sensor table and mmw_reset_scenes).  The state blob and the scene
+ * blob carry this number, so blobs written by another version are refused by mmw_state_restore and mmw_import_scenes. */
+#define MMW_ABI_VERSION 7
 
 typedef enum mmw_status {
     MMW_OK = 0,
@@ -174,6 +175,43 @@ int mmw_reset_scenes(mmw_ctx* ctx, const int32_t* scenes, int n);
 size_t mmw_state_size(mmw_ctx* ctx);
 int mmw_state_dump(mmw_ctx* ctx, void* host_blob, size_t bytes);
 int mmw_state_restore(mmw_ctx* ctx, const void* host_blob, size_t bytes);
+
+/* ---- per-scene export / import: live scenes move between slots, contexts and GPUs ----
+ * A scene blob holds the tracker state of n listed scenes of one context -- each scene's slice of what the state blob
+ * holds (scene record, track records, keypoints, track rings, unassigned ring, ring histograms, pose-row count) --
+ * together with each scene's sensor-table entry: the rings hold raw sensor rows, which are re-read under the entry of
+ * the slot they sit in.  Layout: this 64-byte header, the n source scene indices (int32, padded to 16 bytes), then n
+ * records of record_bytes each, in list order.  The record's layout is private to the library and versioned by
+ * MMW_ABI_VERSION.  Not carried: the outputs of the scene's last frame (point associations, labels, pose rows, packed
+ * records), the accumulated counters, and the mmw_config (the tracker constants are the destination's). */
+#define MMW_SCENE_BLOB_MAGIC 0x4d4d574du   /* "MMWM"; the state blob's is "MMWS" */
+typedef struct mmw_scene_blob_header {
+    uint32_t magic;                /* MMW_SCENE_BLOB_MAGIC */
+    uint32_t abi_version;          /* MMW_ABI_VERSION of the library that wrote it */
+    int32_t n;                     /* scenes in the blob */
+    int32_t max_points_per_frame;  /* shape of the context it was exported from: an import needs the same values */
+    int32_t max_tracks;
+    int32_t frames_batch;
+    uint64_t record_bytes;         /* bytes of one scene record (a multiple of 16) */
+    uint64_t total_bytes;          /* bytes of the whole blob: mmw_scene_state_size(ctx, n) */
+    uint32_t reserved[6];          /* 0 */
+} mmw_scene_blob_header;
+
+/* Bytes of a scene blob of n scenes of this context's shape (0 for a NULL ctx or n < 0). */
+size_t mmw_scene_state_size(mmw_ctx* ctx, int n);
+/* Writes the scenes scenes[0 .. n-1] into host_blob (at least mmw_scene_state_size(ctx, n) bytes, pageable or pinned)
+ * and leaves them unchanged: moving a scene is export, import, and mmw_reset_scenes on the source if its slot is to be
+ * reused.  Synchronous: waits for the work queued so far, the throughput mode's pose network included.  Errors, with
+ * nothing queued: MMW_ERR_INVALID for a NULL pointer, n < 0, or an index out of range or listed twice;
+ * MMW_ERR_CAPACITY when bytes is too small.  n = 0 writes a header only. */
+int mmw_export_scenes(mmw_ctx* ctx, const int32_t* scenes, int n, void* host_blob, size_t bytes);
+/* Puts record i of a scene blob into slot scenes[i] of this context, sensor-table entry included; n must equal the
+ * blob's n.  The header (magic, ABI version, shape, sizes), the destination indices and every record field the kernels
+ * use as an index or a count are checked on the host first: a failure gives MMW_ERR_INVALID and changes nothing.
+ * The slots' per-scene counters of the last step are cleared, as mmw_reset_scenes clears them; their tracks continue
+ * where the source's left off (track ids included).  Synchronous, queued behind all work already queued.  n = 0 checks
+ * the header and does nothing. */
+int mmw_import_scenes(mmw_ctx* ctx, const int32_t* scenes, int n, const void* host_blob, size_t bytes);
 
 /*
  * Loads the keypoint regressor's weights (replaces keras load_model, offline_main.py:33).

@@ -14,7 +14,7 @@ MMW_POSE_2D, MMW_POSE_3D = 0, 1
 STEP_POSE, STEP_DEVICE_INPUT, STEP_RECORD_LABELS, STEP_PIPELINE, STEP_INPUT_I16 = 0x1, 0x2, 0x4, 0x8, 0x10
 SCENE_POINT_OVERFLOW, SCENE_TRACK_OVERFLOW = 0x1, 0x2
 RESULT_FLOATS = 72
-ABI_VERSION = 6            # MMW_ABI_VERSION of include/mmw.h this binding was written against
+ABI_VERSION = 7            # MMW_ABI_VERSION of include/mmw.h this binding was written against
 KERNEL_NAMES = ["step", "pose_index", "pose_features", "conv", "fc1", "fc2", "dbscan_big", "packets"]
 
 
@@ -58,6 +58,21 @@ SCENE_SENSOR_DTYPE = np.dtype([
 assert SCENE_SENSOR_DTYPE.itemsize == C.sizeof(SceneSensor), (SCENE_SENSOR_DTYPE.itemsize, C.sizeof(SceneSensor))
 
 
+SCENE_BLOB_MAGIC = 0x4D4D574D    # MMW_SCENE_BLOB_MAGIC
+
+
+class SceneBlobHeader(C.Structure):
+    """mmw_scene_blob_header: the 64 bytes that open a scene blob (mmw_export_scenes)."""
+    _fields_ = [
+        ("magic", C.c_uint32), ("abi_version", C.c_uint32), ("n", C.c_int32), ("max_points_per_frame", C.c_int32),
+        ("max_tracks", C.c_int32), ("frames_batch", C.c_int32), ("record_bytes", C.c_uint64),
+        ("total_bytes", C.c_uint64), ("reserved", C.c_uint32 * 6),
+    ]
+
+
+assert C.sizeof(SceneBlobHeader) == 64
+
+
 class TrackOut(C.Structure):
     """mmw_track_out"""
     _fields_ = [
@@ -97,6 +112,9 @@ SIGNATURES = {
     "mmw_state_size": (C.c_size_t, [_p]),
     "mmw_state_dump": (C.c_int, [_p, _p, C.c_size_t]),
     "mmw_state_restore": (C.c_int, [_p, _p, C.c_size_t]),
+    "mmw_scene_state_size": (C.c_size_t, [_p, C.c_int]),
+    "mmw_export_scenes": (C.c_int, [_p, _p, C.c_int, _p, C.c_size_t]),
+    "mmw_import_scenes": (C.c_int, [_p, _p, C.c_int, _p, C.c_size_t]),
     "mmw_load_pose_weights": (C.c_int, [_p, C.c_int, _p, C.c_size_t]),
     "mmw_step": (C.c_int, [_p, _p, _p, _p, C.c_uint32]),
     "mmw_estimate_posture": (C.c_int, [_p]),

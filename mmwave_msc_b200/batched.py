@@ -66,6 +66,25 @@ def concat_packets(packets: Sequence[Optional[bytes]]) -> Tuple[np.ndarray, np.n
     return np.frombuffer(b"".join(parts), dtype=np.uint8).copy(), offsets
 
 
+def scene_blob_info(blob) -> dict:
+    """Header and source scene indices of a scene blob (``BatchedTracker.export_scenes``), read on the host: n,
+    abi_version, max_points_per_frame, max_tracks, frames_batch, record_bytes, total_bytes and scenes ((n,) int32).
+    ValueError for a blob that is not a scene blob or is shorter than its header says."""
+    blob = np.ascontiguousarray(blob, dtype=np.uint8).reshape(-1)
+    hs = C.sizeof(_lib.SceneBlobHeader)
+    if blob.size < hs:
+        raise ValueError("scene blob is truncated: %d bytes, the header alone has %d" % (blob.size, hs))
+    h = _lib.SceneBlobHeader.from_buffer_copy(blob[:hs].tobytes())
+    if h.magic != _lib.SCENE_BLOB_MAGIC:
+        raise ValueError("not a scene blob (magic 0x%08x)" % h.magic)
+    if h.n < 0 or blob.size < h.total_bytes or h.total_bytes < hs + (4 * h.n + 15) // 16 * 16 + h.n * h.record_bytes:
+        raise ValueError("scene blob is truncated or its sizes are inconsistent")
+    info = {k: int(getattr(h, k)) for k in ("n", "abi_version", "max_points_per_frame", "max_tracks", "frames_batch",
+                                            "record_bytes", "total_bytes")}
+    info["scenes"] = blob[hs:hs + 4 * h.n].view(np.int32).copy()
+    return info
+
+
 class BatchedTracker:
     """S scenes resident on one GPU.  ``step`` = the loop body of the reference's offline_main.py:45-60
     for every scene at once."""
@@ -400,6 +419,31 @@ class BatchedTracker:
     def state_restore(self, blob: np.ndarray):
         blob = np.ascontiguousarray(blob, dtype=np.uint8)
         _lib.check(self.lib.mmw_state_restore(self._h, _lib.ptr(blob), blob.size))
+
+    def scene_state_size(self, n: int) -> int:
+        """Bytes of a scene blob of n scenes of this context's shape (mmw_scene_state_size)."""
+        return int(self.lib.mmw_scene_state_size(self._h, int(n)))
+
+    def export_scenes(self, scenes, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """Tracker state and sensor-table entry of the selected scenes (a slice or index array) as one uint8 scene blob
+        (mmw_export_scenes); the scenes are left unchanged.  ``out``: a contiguous uint8 buffer of at least
+        ``scene_state_size(n)`` bytes to write into (e.g. pinned memory); the blob is its head."""
+        idx = self._scene_index(scenes)
+        need = self.scene_state_size(idx.size)
+        if out is None:
+            out = np.empty(need, np.uint8)
+        elif out.dtype != np.uint8 or out.ndim != 1 or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError("out must be a contiguous 1-D uint8 array")
+        _lib.check(self.lib.mmw_export_scenes(self._h, _lib.ptr(idx), idx.size, _lib.ptr(out), out.size))
+        return out[:need]
+
+    def import_scenes(self, blob: np.ndarray, scenes=None):
+        """Puts the scenes of a scene blob into the selected slots (a slice or index array, one per scene of the blob;
+        default: the blob's own source indices), sensor-table entries included (mmw_import_scenes).  Their tracks
+        continue where the exported ones left off.  A malformed blob changes nothing (MmwError)."""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8).reshape(-1)
+        idx = scene_blob_info(blob)["scenes"] if scenes is None else self._scene_index(scenes)
+        _lib.check(self.lib.mmw_import_scenes(self._h, _lib.ptr(idx), idx.size, _lib.ptr(blob), blob.size))
 
     def export_track0(self):
         """Dataset-builder export (preprocessing.py:185-216): (rows [S,192,5] float64, valid [S] bool,

@@ -99,6 +99,8 @@ struct mmw_ctx {
     float* d_results[2] = {nullptr, nullptr};
     double* d_export = nullptr;      // [S][192*5 + 2] rows + centroid of mmw_export_track0 (allocated on first use)
     int32_t* d_export_valid = nullptr;
+    unsigned char* d_move = nullptr; // scene blob of mmw_export_scenes / mmw_import_scenes (grown inside those calls only)
+    size_t move_cap = 0;
     unsigned result_idx = 0;
     // pose
     int variant = -1;
@@ -249,7 +251,7 @@ int mmw_destroy(mmw_ctx* x) {
     if (!x) return MMW_OK;
     cudaSetDevice(x->device);
     if (x->stream) cudaStreamSynchronize(x->stream);
-    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_export, x->d_export_valid, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
+    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_export, x->d_export_valid, x->d_move, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
                     x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist,
                     x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
                     x->d_bn1t, x->d_bn2s, x->d_bn2t, x->d_feats, x->d_row_scene, x->d_row_track, x->d_row_slot,
@@ -304,6 +306,8 @@ struct StateHeader {
 };
 constexpr uint32_t kStateMagic = 0x4d4d5753u;   // "MMWS"
 struct StatePart { void* dev; size_t bytes; };
+// Every part is [S][...]: a scene blob record holds each part's per-scene slice, in this order.
+enum { kPartScene, kPartTracks, kPartTrackRing, kPartURing, kPartHist, kPartKeypoints, kPartPoseCnt, kNumStateParts };
 std::vector<StatePart> state_parts(mmw_ctx* x) {
     const size_t S = x->S;
     return {{x->d_scenes, sizeof(SceneRec) * S},
@@ -515,18 +519,22 @@ int mmw_set_doppler_resolution(mmw_ctx* x, double doppler_res) {
     return upload_sensors(x, 0, x->S);
 }
 
+// What is wrong with a sensor-table entry, or nullptr: the rules of mmw_set_scene_sensors.
+static const char* sensor_error(const mmw_scene_sensor& p) {
+    if (!std::isfinite(p.s_height) || !std::isfinite(p.s_tilt_deg) || !std::isfinite(p.z_max) ||
+        !std::isfinite(p.doppler_res))
+        return "sensor parameters must be finite";
+    if (!(p.doppler_res > 0.0)) return "doppler_res must be positive";
+    if (p.xyz_q_format < 0 || p.xyz_q_format > 15) return "xyz_q_format must be 0..15";
+    if (p.num_doppler_bins < 0) return "num_doppler_bins must not be negative";
+    return nullptr;
+}
+
 int mmw_set_scene_sensors(mmw_ctx* x, int first, int n, const mmw_scene_sensor* params) {
     if (!x || !params) return fail(MMW_ERR_INVALID, "ctx/params is NULL");
     if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
-    for (int i = 0; i < n; ++i) {
-        const mmw_scene_sensor& p = params[i];
-        if (!std::isfinite(p.s_height) || !std::isfinite(p.s_tilt_deg) || !std::isfinite(p.z_max) ||
-            !std::isfinite(p.doppler_res))
-            return fail(MMW_ERR_INVALID, "sensor parameters must be finite");
-        if (!(p.doppler_res > 0.0)) return fail(MMW_ERR_INVALID, "doppler_res must be positive");
-        if (p.xyz_q_format < 0 || p.xyz_q_format > 15) return fail(MMW_ERR_INVALID, "xyz_q_format must be 0..15");
-        if (p.num_doppler_bins < 0) return fail(MMW_ERR_INVALID, "num_doppler_bins must not be negative");
-    }
+    for (int i = 0; i < n; ++i)
+        if (const char* e = sensor_error(params[i])) return fail(MMW_ERR_INVALID, e);
     if (n == 0) return MMW_OK;
     for (int i = 0; i < n; ++i) x->sensors[first + i] = params[i];
     return upload_sensors(x, first, n);
@@ -539,8 +547,8 @@ int mmw_get_scene_sensors(mmw_ctx* x, int first, int n, mmw_scene_sensor* out) {
     return MMW_OK;
 }
 
-int mmw_reset_scenes(mmw_ctx* x, const int32_t* scenes, int n) {
-    if (!x || (!scenes && n > 0)) return fail(MMW_ERR_INVALID, "ctx/scenes is NULL");
+// MMW_OK, or MMW_ERR_INVALID for a list of n scene indices with one out of range or listed twice.
+static int check_scene_list(const mmw_ctx* x, const int32_t* scenes, int n) {
     if (n < 0) return fail(MMW_ERR_INVALID, "n must not be negative");
     std::vector<char> seen(x->S, 0);
     for (int i = 0; i < n; ++i) {
@@ -549,6 +557,13 @@ int mmw_reset_scenes(mmw_ctx* x, const int32_t* scenes, int n) {
         if (seen[s]) return fail(MMW_ERR_INVALID, "scene index listed twice");
         seen[s] = 1;
     }
+    return MMW_OK;
+}
+
+int mmw_reset_scenes(mmw_ctx* x, const int32_t* scenes, int n) {
+    if (!x || (!scenes && n > 0)) return fail(MMW_ERR_INVALID, "ctx/scenes is NULL");
+    const int rc = check_scene_list(x, scenes, n);
+    if (rc != MMW_OK) return rc;
     CK(cudaSetDevice(x->device));
     if (x->pose_stream) CK(join_pose(x));
     int32_t* pose_cnt = x->d_defer + 1 + x->S;       // StepArgs::pose_cnt
@@ -1386,6 +1401,45 @@ __global__ void __launch_bounds__(128) compact_results_kernel(const float* __res
     }
 }
 
+// ---- per-scene export / import (mmw_export_scenes, mmw_import_scenes) ----------------------------------------
+// One part of a scene's state: scene s at dev + s * dev_stride, list entry i of the move buffer at buf + i * buf_stride.
+// buf == nullptr (scatter only): the scene's bytes are zeroed.  Every size is a multiple of 4 bytes.
+struct MovePart {
+    unsigned char* dev;
+    unsigned char* buf;
+    unsigned long long dev_stride, buf_stride;
+    unsigned bytes, pad;
+};
+constexpr int kMaxMoveParts = 10;
+struct MoveParts { MovePart p[kMaxMoveParts]; int n; };
+
+// One CTA per listed scene copies all its parts, between the context's state and the move buffer (a device buffer the
+// context owns: no kernel touches host memory).  16-byte vectors where both sides and the size allow -- the unassigned
+// ring's stride 60 * ncap and the keypoints' 228 * tcap are not always 16-aligned -- 4-byte words otherwise.
+template <bool kGather>
+__global__ void __launch_bounds__(256) scene_move_kernel(const __grid_constant__ MoveParts m, const int32_t* scenes,
+                                                         int S) {
+    const int i = blockIdx.x;
+    const int s = scenes[i];
+    if (s < 0 || s >= S) return;         // the host has validated the list: a second guard only
+    for (int k = 0; k < m.n; ++k) {
+        const MovePart& p = m.p[k];
+        unsigned char* d = p.dev + (size_t)s * p.dev_stride;
+        unsigned char* b = p.buf != nullptr ? p.buf + (size_t)i * p.buf_stride : nullptr;
+        unsigned char* dst = kGather ? b : d;
+        const unsigned char* src = kGather ? d : b;
+        if ((((uintptr_t)dst | (uintptr_t)src | p.bytes) & 15) == 0) {
+            uint4* o = reinterpret_cast<uint4*>(dst);
+            const uint4* q = reinterpret_cast<const uint4*>(src);
+            for (unsigned e = threadIdx.x; e < p.bytes / 16; e += blockDim.x) o[e] = q != nullptr ? q[e] : make_uint4(0, 0, 0, 0);
+        } else {
+            uint32_t* o = reinterpret_cast<uint32_t*>(dst);
+            const uint32_t* q = reinterpret_cast<const uint32_t*>(src);
+            for (unsigned e = threadIdx.x; e < p.bytes / 4; e += blockDim.x) o[e] = q != nullptr ? q[e] : 0u;
+        }
+    }
+}
+
 }  // namespace mmw
 
 extern "C" {
@@ -1589,6 +1643,197 @@ int mmw_pack_results(mmw_ctx* x, float* device_out) {
                   (const SceneRec*)x->d_scenes, (const TrackRec*)x->d_tracks, (const float*)x->d_keypoints, x->S, x->tcap,
                   device_out, fc));
     x->launches++;
+    return MMW_OK;
+}
+
+// ---- per-scene export / import ----------------------------------------------------------------------------------
+static size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
+
+// A scene record: the scene's sensor-table entry at 0, then its slice of every state part (kPart* order), each at a
+// 16-byte boundary.
+struct SceneLayout {
+    size_t per[kNumStateParts];          // bytes of the part per scene
+    size_t off[kNumStateParts];          // offset of the part in the record
+    size_t rec;                          // record bytes, a multiple of 16
+};
+static SceneLayout scene_layout(mmw_ctx* x) {
+    SceneLayout L;
+    const std::vector<StatePart> parts = state_parts(x);
+    size_t o = align16(sizeof(mmw_scene_sensor));
+    for (int k = 0; k < kNumStateParts; ++k) {
+        L.per[k] = parts[k].bytes / x->S;
+        L.off[k] = o;
+        o += align16(L.per[k]);
+    }
+    L.rec = o;
+    return L;
+}
+static size_t scene_head_bytes(int n) { return sizeof(mmw_scene_blob_header) + align16(sizeof(int32_t) * n); }
+
+// The state parts of the listed scenes <-> the records of the scene blob in the move buffer.
+static MoveParts scene_move_parts(mmw_ctx* x, const SceneLayout& L, int n) {
+    MoveParts m{};
+    const std::vector<StatePart> parts = state_parts(x);
+    unsigned char* rec0 = x->d_move + scene_head_bytes(n);
+    for (int k = 0; k < kNumStateParts; ++k)
+        m.p[m.n++] = MovePart{static_cast<unsigned char*>(parts[k].dev), rec0 + L.off[k], L.per[k], L.rec, (unsigned)L.per[k], 0};
+    return m;
+}
+
+// The move buffer holds at least `bytes`.  Only called inside the synchronous export / import, after the pose stream
+// has joined the main stream: the previous call has finished with the buffer.
+static int grow_move(mmw_ctx* x, size_t bytes) {
+    CK(grow((void**)&x->d_move, &x->move_cap, bytes));
+    return MMW_OK;
+}
+
+// What is wrong with a record of a scene blob, or nullptr.  Checked: every field a kernel takes as an index or a count.
+//   sensor entry     the rules of mmw_set_scene_sensors (doppler_res > 0, Q format 0..15, ...)
+//   SceneRec         0 <= n_tracks <= tcap                    (step_kernel's bulk copy of T0 records, the list)
+//                    0 <= ring_n <= ring_size, 0 <= ring_head < ring_size   (ring_wrap, uring / histogram frames)
+//                    0 <= ring_cnt[f] <= ncap                 (fused cloud of DBSCAN: at most 3 * ncap rows, labels)
+//                    slot_mask = the set of the listed tracks' slots: spawning takes the lowest free slot of
+//                      ~slot_mask for each new track, and a spare bit would leave fewer than tcap - n_tracks
+//   TrackRec k < n_tracks   0 <= slot < tcap, no two alike  (track ring / keypoints by slot, 1 << slot)
+//                    0 <= ring_n <= ring_size, 0 <= ring_head < ring_size, 0 <= ring_cnt[f] <= 64   (feature maps)
+//   pose_cnt         0 <= pose_cnt <= tcap                    (prefix sum of pose rows: at most S * tcap rows)
+// Not indices or counts: next_id, flags, last_M, last_ran (selects n_tracks), dbscan_n (host only), ring_ph_gone,
+// pose_base (rewritten before every read, pose_kernels.cu), the float64 track state, the histogram bytes (summed into
+// 16-bit cell counts that only steer the DBSCAN screen) and the rows of the rings.
+static const char* scene_record_error(const mmw_ctx* x, const SceneLayout& L, const unsigned char* r) {
+    mmw_scene_sensor p;
+    std::memcpy(&p, r, sizeof(p));
+    if (const char* e = sensor_error(p)) return e;
+    const int rs = x->dc.ring_size, tcap = x->tcap, ncap = x->ncap;
+    SceneRec sc;
+    std::memcpy(&sc, r + L.off[kPartScene], sizeof(sc));
+    if (sc.n_tracks < 0 || sc.n_tracks > tcap) return "n_tracks out of range";
+    if (sc.ring_n < 0 || sc.ring_n > rs || sc.ring_head < 0 || sc.ring_head >= rs) return "unassigned ring position out of range";
+    for (int f = 0; f < kRing; ++f)
+        if (sc.ring_cnt[f] < 0 || sc.ring_cnt[f] > ncap) return "unassigned ring count out of range";
+    uint32_t used = 0;
+    for (int k = 0; k < sc.n_tracks; ++k) {
+        TrackRec t;
+        std::memcpy(&t, r + L.off[kPartTracks] + sizeof(TrackRec) * k, sizeof(t));
+        if (t.slot < 0 || t.slot >= tcap) return "track slot out of range";
+        if (used & (1u << t.slot)) return "two tracks hold the same slot";
+        used |= 1u << t.slot;
+        if (t.ring_n < 0 || t.ring_n > rs || t.ring_head < 0 || t.ring_head >= rs) return "track ring position out of range";
+        for (int f = 0; f < kRing; ++f)
+            if (t.ring_cnt[f] < 0 || t.ring_cnt[f] > kFeatPts) return "track ring count out of range";
+    }
+    if (sc.slot_mask != used) return "slot_mask is not the set of the tracks' slots";
+    int32_t pose_cnt;
+    std::memcpy(&pose_cnt, r + L.off[kPartPoseCnt], sizeof(pose_cnt));
+    if (pose_cnt < 0 || pose_cnt > tcap) return "pose-row count out of range";
+    return nullptr;
+}
+
+size_t mmw_scene_state_size(mmw_ctx* x, int n) {
+    if (!x || n < 0) return 0;
+    return scene_head_bytes(n) + (size_t)n * scene_layout(x).rec;
+}
+
+int mmw_export_scenes(mmw_ctx* x, const int32_t* scenes, int n, void* host_blob, size_t bytes) {
+    if (!x || !host_blob || (!scenes && n > 0)) return fail(MMW_ERR_INVALID, "ctx/scenes/host_blob is NULL");
+    int rc = check_scene_list(x, scenes, n);
+    if (rc != MMW_OK) return rc;
+    const size_t need = mmw_scene_state_size(x, n);
+    if (bytes < need) return fail(MMW_ERR_CAPACITY, "scene blob buffer is smaller than mmw_scene_state_size()");
+    const SceneLayout L = scene_layout(x);
+    const size_t head = scene_head_bytes(n);
+    std::vector<unsigned char> h(head, 0);
+    mmw_scene_blob_header hd{};
+    hd.magic = MMW_SCENE_BLOB_MAGIC;
+    hd.abi_version = MMW_ABI_VERSION;
+    hd.n = n;
+    hd.max_points_per_frame = x->ncap;
+    hd.max_tracks = x->tcap;
+    hd.frames_batch = x->cfg.frames_batch;
+    hd.record_bytes = L.rec;
+    hd.total_bytes = need;
+    std::memcpy(h.data(), &hd, sizeof(hd));
+    if (n > 0) std::memcpy(h.data() + sizeof(hd), scenes, sizeof(int32_t) * n);
+    unsigned char* o = static_cast<unsigned char*>(host_blob);
+    if (n == 0) {
+        std::memcpy(o, h.data(), head);
+        return MMW_OK;
+    }
+    CK(cudaSetDevice(x->device));
+    CK(join_pose(x));
+    if ((rc = grow_move(x, need)) != MMW_OK) return rc;
+    // header and source indices go up with the list the kernel reads; the zero fill makes the padding of the records 0
+    CK(cudaMemcpyAsync(x->d_move, h.data(), head, cudaMemcpyHostToDevice, x->stream));
+    CK(cudaMemsetAsync(x->d_move + head, 0, need - head, x->stream));
+    scene_move_kernel<true><<<n, 256, 0, x->stream>>>(scene_move_parts(x, L, n),
+                                                     reinterpret_cast<const int32_t*>(x->d_move + sizeof(hd)), x->S);
+    CK(cudaGetLastError());
+    x->launches++;
+    CK(cudaMemcpyAsync(o, x->d_move, need, cudaMemcpyDeviceToHost, x->stream));
+    CK(sync_main(x));
+    for (int i = 0; i < n; ++i)                          // the sensor table is host state
+        std::memcpy(o + head + L.rec * i, &x->sensors[scenes[i]], sizeof(mmw_scene_sensor));
+    return MMW_OK;
+}
+
+int mmw_import_scenes(mmw_ctx* x, const int32_t* scenes, int n, const void* host_blob, size_t bytes) {
+    if (!x || !host_blob || (!scenes && n > 0)) return fail(MMW_ERR_INVALID, "ctx/scenes/host_blob is NULL");
+    if (n < 0) return fail(MMW_ERR_INVALID, "n must not be negative");
+    mmw_scene_blob_header hd;
+    if (bytes < sizeof(hd)) return fail(MMW_ERR_INVALID, "scene blob is truncated");
+    std::memcpy(&hd, host_blob, sizeof(hd));
+    if (hd.magic != MMW_SCENE_BLOB_MAGIC || hd.abi_version != MMW_ABI_VERSION)
+        return fail(MMW_ERR_INVALID, "not a scene blob of this library version");
+    if (hd.max_points_per_frame != x->ncap || hd.max_tracks != x->tcap || hd.frames_batch != x->cfg.frames_batch)
+        return fail(MMW_ERR_INVALID, "scene blob was exported from a context of another shape "
+                                     "(max_points_per_frame / max_tracks / frames_batch)");
+    if (hd.n != n) return fail(MMW_ERR_INVALID, "n differs from the scene blob's");
+    const SceneLayout L = scene_layout(x);
+    const size_t need = mmw_scene_state_size(x, n);
+    if (hd.record_bytes != L.rec || hd.total_bytes != need || bytes < need)
+        return fail(MMW_ERR_INVALID, "scene blob is truncated or its sizes are inconsistent");
+    int rc = check_scene_list(x, scenes, n);
+    if (rc != MMW_OK) return rc;
+    const size_t head = scene_head_bytes(n);
+    const unsigned char* rec0 = static_cast<const unsigned char*>(host_blob) + head;
+    std::vector<mmw_scene_sensor> sensors(n);
+    for (int i = 0; i < n; ++i) {
+        if (const char* e = scene_record_error(x, L, rec0 + L.rec * i))
+            return fail(MMW_ERR_INVALID, "scene blob record " + std::to_string(i) + ": " + e);
+        std::memcpy(&sensors[i], rec0 + L.rec * i, sizeof(mmw_scene_sensor));
+    }
+    if (n == 0) return MMW_OK;
+    // behind the blob: the destination list, then each scene's SensorRec and Doppler threshold, built on the host
+    const size_t idx_bytes = align16(sizeof(int32_t) * n);
+    std::vector<SensorRec> recs(n);
+    std::vector<double> wrap(n);
+    for (int i = 0; i < n; ++i) {
+        recs[i] = sensor_rec(sensors[i]);
+        wrap[i] = doppler_wrap(sensors[i]);
+    }
+    std::vector<unsigned char> aux(idx_bytes + (sizeof(SensorRec) + sizeof(double)) * n, 0);
+    std::memcpy(aux.data(), scenes, sizeof(int32_t) * n);
+    std::memcpy(aux.data() + idx_bytes, recs.data(), sizeof(SensorRec) * n);
+    std::memcpy(aux.data() + idx_bytes + sizeof(SensorRec) * n, wrap.data(), sizeof(double) * n);
+    CK(cudaSetDevice(x->device));
+    CK(join_pose(x));
+    if ((rc = grow_move(x, need + aux.size())) != MMW_OK) return rc;
+    unsigned char* a = x->d_move + need;
+    CK(cudaMemcpyAsync(x->d_move, host_blob, need, cudaMemcpyHostToDevice, x->stream));
+    CK(cudaMemcpyAsync(a, aux.data(), aux.size(), cudaMemcpyHostToDevice, x->stream));
+    MoveParts m = scene_move_parts(x, L, n);
+    m.p[m.n++] = MovePart{reinterpret_cast<unsigned char*>(x->d_sensors), a + idx_bytes, sizeof(SensorRec),
+                          sizeof(SensorRec), (unsigned)sizeof(SensorRec), 0};
+    m.p[m.n++] = MovePart{reinterpret_cast<unsigned char*>(x->d_doppler_wrap), a + idx_bytes + sizeof(SensorRec) * n,
+                          sizeof(double), sizeof(double), (unsigned)sizeof(double), 0};
+    // the per-scene counters of the last step are cleared, as mmw_reset_scenes clears them
+    m.p[m.n++] = MovePart{reinterpret_cast<unsigned char*>(x->d_scene_stats), nullptr, sizeof(int32_t) * 8, 0,
+                          (unsigned)(sizeof(int32_t) * 8), 0};
+    scene_move_kernel<false><<<n, 256, 0, x->stream>>>(m, reinterpret_cast<const int32_t*>(a), x->S);
+    CK(cudaGetLastError());
+    x->launches++;
+    for (int i = 0; i < n; ++i) x->sensors[scenes[i]] = sensors[i];
+    CK(sync_main(x));
     return MMW_OK;
 }
 

@@ -38,6 +38,25 @@ def gather_results(local, n_scenes: int, per_scene: int, group=None):
     return torch.cat(parts)
 
 
+def move_scenes(src, src_scenes, dst, dst_scenes=None, reset_source=True):
+    """Moves live scenes from BatchedTracker ``src`` to ``dst`` (e.g. to drain a GPU or rebalance ranks): exports
+    ``src_scenes``, imports them into ``dst_scenes`` (default: the same indices) with their tracks, rings, id counters
+    and sensor-table entries, then, with ``reset_source``, frees the source slots (``src.reset_scenes``).  The contexts
+    must have the same max_points, max_tracks and frames_batch; they may sit on different GPUs.  Returns the blob."""
+    import numpy as np
+    src_idx = np.ascontiguousarray(np.atleast_1d(src_scenes), dtype=np.int32).reshape(-1)
+    dst_idx = src_idx if dst_scenes is None else np.ascontiguousarray(np.atleast_1d(dst_scenes), dtype=np.int32).reshape(-1)
+    if dst_idx.size != src_idx.size:
+        raise ValueError("move_scenes: %d source scenes but %d destination slots" % (src_idx.size, dst_idx.size))
+    if reset_source and src is dst and np.intersect1d(src_idx, dst_idx).size:
+        raise ValueError("move_scenes: resetting the source would clear scenes just moved into the same context")
+    blob = src.export_scenes(src_idx)
+    dst.import_scenes(blob, dst_idx)
+    if reset_source:
+        src.reset_scenes(src_idx)
+    return blob
+
+
 class NcclGather:
     """The result gather through the C ABI (mmw_gather_nccl): one ncclAllGather on the context's stream, this rank's
     records packed straight into its block of the output.  The communicator is formed with the library's own helpers;
