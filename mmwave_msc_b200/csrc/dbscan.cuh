@@ -10,6 +10,7 @@
 //
 // which is exactly what dbscan_inner's ascending outer loop + DFS produces.
 #pragma once
+#include <cmath>
 #include "mmw_internal.cuh"
 
 namespace mmw {
@@ -74,6 +75,57 @@ struct NbExact {
 // guard band around eps -- wider than any fp32 rounding could move it -- are re-evaluated exactly in float64 from
 // the raw ring rows.  Decisions are therefore identical to the exact predicate, at a fraction of the FP64 work
 // (the FP64/XU pipe is what bounds this kernel, profiles/).
+//
+// The band only covers the fp32 error where that error is bounded, so the screen has a domain: |y'|, |z'| <= R.
+// A point outside it gets Xf = NaN (screen_domain_mark), which makes the fp32 distance of every pair it is in NaN:
+// such a pair is neither above hi nor below lo and goes to float64.  Derivation (u = 2^-24, first order in u; rw, zw
+// >= 0; both points inside the domain, so w = 1 - rw (y1 + y2) / 2 lies in [w_min, 2] with w_min = 1 - rw R):
+//   inputs   x exact, Yf = y (1 + d), |d| <= u, same for Zf; rw and zw rounded to fp32 (relative u)
+//   w        |w_f - w| <= 4 u rw R + u |w_f| <= 6 u
+//   q        dx^2 + dy^2 + zw dz^2: 7 u q from the roundings of the products and sums (all terms >= 0), plus the
+//            rounding of the inputs, |dy_f - dy| <= 2 u R + u |dy|, which adds 4 u R |dy| <= 4 u R sqrt(q), and
+//            4 u R zw |dz| <= 4 u R sqrt(zw q) for the z term
+//   d = w q  |d_f - d| <= |w_f - w| q + |w| |q_f - q| + u |d_f| <= 22 u q + 8 u R sqrt(q) (1 + sqrt(zw))
+// Fused multiply-adds only remove roundings, so the bound holds for any contraction.  A pair decided wrongly has
+// d <= eps < hi < d_f or d_f < lo < eps < d, so q <= (eps + band) / w_min (1 + O(u)) =: Q / 2.  R is chosen
+// (screen_config) so that the bound at Q is at most half the band; the other half covers the fp32 rounding of eps,
+// lo and hi (~u eps, the band is >= 1e-3 eps) and the float64 rounding of the exact predicate.  w_min is 0.25
+// (R <= 0.75 / rw): the band would need to grow as 1 / w near w = 0, where the fp32 error does.
+// tests/dbscan_screen_model.py restates this function and screen_config.
+__device__ __forceinline__ float screen_d(float xb, float yb, float zb, float xq, float yq, float zq, float rw,
+                                          float zw) {
+    const float w = 1.f - 0.5f * (yb + yq) * rw;
+    const float dx = xb - xq, dy = yb - yq, dz = zb - zq;
+    return w * (dx * dx + dy * dy + zw * (dz * dz));
+}
+
+// The fp32 x of a point as the screen stores it: NaN outside the screen's domain (every pair of the point goes to
+// float64, see screen_d).  yw, zw: the point's float64 world coordinates.
+__device__ __forceinline__ float screen_domain_mark(float x, double yw, double zw, float rmax) {
+    return fabs(yw) <= (double)rmax && fabs(zw) <= (double)rmax ? x : __int_as_float(0x7fc00000);
+}
+
+// Host side: guard band and domain radius for a configuration (mmw_create).  rmax = -1 (every pair exact): eps not
+// positive and finite, a negative or non-finite weight, or no radius at which the bound holds.
+inline void screen_config(double eps, double range_weight, double z_weight, float* lo, float* hi, float* rmax) {
+    const float band = 1e-3f * (float)eps + 1e-4f;
+    *lo = (float)eps - band;
+    *hi = (float)eps + band;
+    *rmax = -1.f;
+    if (!(eps > 0.0 && eps < 1e30) || !(range_weight >= 0.0 && range_weight < 1e30) ||
+        !(z_weight >= 0.0 && z_weight < 1e30))
+        return;
+    const double u = 0x1p-24, wmin = 0.25;
+    const double Q = 2.0 * (eps + (double)band) / wmin;
+    double R = (0.5 * (double)band - 22.0 * u * Q) / (8.0 * u * std::sqrt(Q) * (1.0 + std::sqrt(z_weight)));
+    if (range_weight > 0.0) R = std::fmin(R, (1.0 - wmin) / range_weight);
+    if (!(R > 0.0)) return;
+    R = std::fmin(R, 1e30);
+    float r = (float)R;
+    if ((double)r > R) r = std::nextafter(r, 0.f);                   // round down
+    *rmax = r;
+}
+
 struct NbScreened {
     const DevConfig& c;
     const SensorRec& sr;              // the scene's mounting (shared memory)
@@ -104,13 +156,10 @@ struct NbScreened {
         float lo, hi, rw, zw;
         const NbScreened* full;
         __device__ __forceinline__ bool operator()(int b, int q) const {
-            const float yb = Y[b], yq = Y[q];
-            const float w = 1.f - 0.5f * (yb + yq) * rw;
-            const float dx = X[b] - X[q], dy = yb - yq, dz = Z[b] - Z[q];
-            const float d = w * (dx * dx + dy * dy + zw * (dz * dz));
+            const float d = screen_d(X[b], Y[b], Z[b], X[q], Y[q], Z[q], rw, zw);
             if (d > hi) return false;
             if (d < lo) return true;
-            return full->exact(b, q);                   // inside the guard band (or not finite): decide exactly
+            return full->exact(b, q);                   // inside the guard band or outside the domain: decide exactly
         }
     };
     __device__ __forceinline__ Hot hot() const { return Hot{Xf, Yf, Zf, lo, hi, rw, zw, this}; }
@@ -350,14 +399,11 @@ __device__ inline int dbscan_bits_block(const NbScreened& nbf, int B, int min_sa
             // two rows per step: their dependent chains (broadcast loads -> distance -> ballot) overlap
             for (int r = 0; r < bn; r += 2) {
                 const int ba = b0 + r, bb = r + 1 < bn ? ba + 1 : ba;
-                const float ya = Y[ba], yb = Y[bb];
-                const float wa = 1.f - 0.5f * (ya + yq) * rw, wb = 1.f - 0.5f * (yb + yq) * rw;
-                const float dxa = X[ba] - xq, dya = ya - yq, dza = Z[ba] - zq;
-                const float dxb = X[bb] - xq, dyb = yb - yq, dzb = Z[bb] - zq;
-                const float da = wa * (dxa * dxa + dya * dya + zw * (dza * dza));
-                const float db = wb * (dxb * dxb + dyb * dyb + zw * (dzb * dzb));
+                const float da = screen_d(X[ba], Y[ba], Z[ba], xq, yq, zq, rw, zw);
+                const float db = screen_d(X[bb], Y[bb], Z[bb], xq, yq, zq, rw, zw);
                 bool hita = qlive && (da < lo || q == ba), hitb = qlive && (db < lo || q == bb);
-                const bool unsa = qlive && !(da > hi) && !hita, unsb = qlive && !(db > hi) && !hitb;   // in the band / not finite
+                // in the band or outside the screen's domain (NaN)
+                const bool unsa = qlive && !(da > hi) && !hita, unsb = qlive && !(db > hi) && !hitb;
                 if (__any_sync(kFullMask, unsa || unsb)) {
                     if (unsa) hita = nbf.exact(ba, q);
                     if (unsb) hitb = nbf.exact(bb, q);

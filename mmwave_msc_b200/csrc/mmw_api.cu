@@ -210,6 +210,7 @@ static void fill_devconfig(const mmw_config& c, int ncap, int tcap, DevConfig* d
     d->tcap = tcap;
     grid_screen_config(c.db_eps, c.db_range_weight, c.db_z_weight, c.db_min_samples, &d->grid_inv_h, &d->grid_ybound,
                        &d->grid_ok);
+    screen_config(c.db_eps, c.db_range_weight, c.db_z_weight, &d->screen_lo, &d->screen_hi, &d->screen_rmax);
 }
 
 static const float kDefaultPosture[57] = {

@@ -50,6 +50,9 @@ struct DevConfig {
     // for every pair of points with y' <= grid_ybound; grid_ok = 0: degenerate configuration, the screen always passes
     float grid_inv_h, grid_ybound;
     int grid_ok;
+    // fp32 screen of the eps predicate (dbscan.cuh, screen_d): guard band [lo, hi] around eps, and the domain |y'|, |z'|
+    // <= rmax in which the band covers the fp32 error (rmax = -1: every pair is decided in float64)
+    float screen_lo, screen_hi, screen_rmax;
 };
 
 // One element of a scene's effective_tracks list (ClusterTrack + KalmanState + PointCluster).

@@ -336,11 +336,8 @@ __device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, const S
     const DevConfig& c = a.cfg;
     float* Yf = Xf + stride;
     float* Zf = Yf + stride;
-    NbScreened nb{c, sr, Xf, Yf, Zf, {nullptr, nullptr, nullptr}, {0, 0, 0, 0}, c.db_eps, 0.f, 0.f,
+    NbScreened nb{c, sr, Xf, Yf, Zf, {nullptr, nullptr, nullptr}, {0, 0, 0, 0}, c.db_eps, c.screen_lo, c.screen_hi,
                   (float)c.db_range_weight, (float)c.db_z_weight, rawc};
-    const float band = 1e-3f * (float)c.db_eps + 1e-4f;
-    nb.lo = (float)c.db_eps - band;
-    nb.hi = (float)c.db_eps + band;
     static_assert(kRing == 3, "the flattened ring load below is written for three frames");
     int b0 = 0;
     for (int f = 0; f < kRing; ++f) {
@@ -358,7 +355,7 @@ __device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, const S
         const float x = src[i * kRawCols + 0], y = src[i * kRawCols + 1], z = src[i * kRawCols + 2];
         double yw, zw;
         world_yz(sr, (double)y, (double)z, yw, zw);
-        Xf[b] = x; Yf[b] = (float)yw; Zf[b] = (float)zw;
+        Xf[b] = screen_domain_mark(x, yw, zw, c.screen_rmax); Yf[b] = (float)yw; Zf[b] = (float)zw;
         if (rawc != nullptr) {
             float* r = rawc + (size_t)b * kRawCols;
             r[0] = x; r[1] = y; r[2] = z; r[3] = src[i * kRawCols + 3]; r[4] = src[i * kRawCols + 4];
