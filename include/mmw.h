@@ -39,7 +39,8 @@ typedef enum mmw_status {
 } mmw_status;
 
 /* Mirror of the reference's constants.py (file:line = constants.py).  s_height, s_tilt_deg, z_max, xyz_q_format and
- * doppler_res are the defaults of every scene's entry in the sensor table (mmw_scene_sensor). */
+ * doppler_res are the defaults of every scene's entry in the sensor table (mmw_scene_sensor); the db_*, tr_*, kf_* and
+ * x_nudge_* fields are the defaults of every scene's entry in the tracker table (mmw_scene_tracker). */
 typedef struct mmw_config {
     double s_height;               /* S_HEIGHT :41 */
     double s_tilt_deg;             /* S_TILT :42 */
@@ -124,7 +125,7 @@ const char* mmw_last_error(void);
 int mmw_abi_version(void);
 
 /* Resets every scene to the state of a fresh TrackBuffer() + BatchedData() (Tracking.py:504-511, 38-41).  The sensor
- * table (mmw_scene_sensor) is configuration and stays as it is. */
+ * and tracker tables (mmw_scene_sensor, mmw_scene_tracker) are configuration and stay as they are. */
 int mmw_reset(mmw_ctx* ctx);
 
 /* Changes mmw_config::doppler_res of a live context, the context's unit, and sets it as every scene's doppler_res
@@ -160,18 +161,67 @@ int mmw_set_scene_sensors(mmw_ctx* ctx, int first_scene, int n, const mmw_scene_
 /* Reads the entries of scenes first_scene .. first_scene + n - 1 into out[0 .. n-1]. */
 int mmw_get_scene_sensors(mmw_ctx* ctx, int first_scene, int n, mmw_scene_sensor* out);
 
+/* ---- per-scene tracker table ----
+ * Each scene's tracker and DBSCAN constants: a dense room, a corridor and a ward of mostly still people want other
+ * values, in one context and one pose batch.  Fields have the meanings of the mmw_config fields of the same names
+ * (constants.py lines as there).  Context-wide and not in this table: frames_batch, the pose model's
+ * intensity_mu / intensity_std and default_posture, the fade-square geometry, and the sensor table's fields.
+ * mmw_create fills every scene's entry from the mmw_config; a context that never changes the table behaves as if it
+ * had none.  A change takes effect with the next mmw_step, mmw_step_packets or mmw_run_frames*: it is queued on the
+ * context's stream behind all work already queued there.  Live scenes keep their tracks: ids, state, rings and
+ * lifetimes continue under the new constants from the next frame on -- kf_p_init and kf_group_disp_init only affect
+ * tracks spawned afterwards, the lifetime limits are compared against the lifetime a track has already accumulated, and
+ * tr_max_tracks gates the next DBSCAN.
+ * DBSCAN screen: each ring frame's cell histogram was binned under the db_eps / db_range_weight / db_z_weight of the
+ * frame's push, so when a scene's db_eps, db_z_weight, db_range_weight or db_min_samples change, the update raises the
+ * flag of every ring histogram of that scene (bitwise comparison of the old and new values): the screen passes until
+ * those frames have left the ring and DBSCAN decides exactly.  Scenes whose DBSCAN fields did not change keep their
+ * flags.
+ * The table is configuration, like the sensor table: it is not part of the state blob or the scene blob, and
+ * mmw_reset, mmw_reset_scenes, mmw_state_restore and mmw_import_scenes leave it as it is.  The stateless stage entry
+ * points (mmw_preprocess, mmw_dbscan, mmw_gate, mmw_kalman_*) keep using the values of the mmw_config. */
+typedef struct mmw_scene_tracker {
+    double db_eps;                 /* DB_EPS constants.py:72 */
+    double db_z_weight;            /* DB_Z_WEIGHT :70 */
+    double db_range_weight;        /* DB_RANGE_WEIGHT :71 */
+    double tr_lifetime_dynamic;    /* TR_LIFETIME_DYNAMIC :86 [s] */
+    double tr_lifetime_static;     /* TR_LIFETIME_STATIC :87 [s] */
+    double tr_vel_thres;           /* TR_VEL_THRES :88 */
+    double tr_gate;                /* TR_GATE :89 */
+    double kf_q_var;               /* KF_Q_STD :93, passed as a variance (:212) */
+    double kf_p_init;              /* KF_P_INIT :96 */
+    double kf_group_disp_init;     /* KF_GROUP_DISP_EST_INIT :97 */
+    double kf_a_n;                 /* KF_A_N :101 */
+    double kf_a_spr;               /* KF_A_SPR :104 */
+    double kf_spread_lim[6];       /* KF_SPREAD_LIM :103 */
+    double x_nudge_thres;          /* 0.6, Tracking.py:397 */
+    double x_nudge_gain;           /* 0.4, Tracking.py:398 */
+    int32_t db_min_samples;        /* DB_MIN_SAMPLES_MIN :73, >= 1 */
+    int32_t tr_max_tracks;         /* TR_MAX_TRACKS :85 (only gates whether DBSCAN runs, Tracking.py:693-696), >= 0 */
+    int32_t kf_enable_est;         /* KF_ENABLE_EST :100 */
+    int32_t kf_est_pointnum;       /* KF_EST_POINTNUM :102 */
+} mmw_scene_tracker;
+
+/* Sets the entries of scenes first_scene .. first_scene + n - 1 from params[0 .. n-1].  All or nothing: a range out of
+ * bounds, a NULL pointer, a non-finite value, db_min_samples < 1 or tr_max_tracks < 0 give MMW_ERR_INVALID, change no
+ * entry and queue nothing. */
+int mmw_set_scene_trackers(mmw_ctx* ctx, int first_scene, int n, const mmw_scene_tracker* params);
+/* Reads the entries of scenes first_scene .. first_scene + n - 1 into out[0 .. n-1]. */
+int mmw_get_scene_trackers(mmw_ctx* ctx, int first_scene, int n, mmw_scene_tracker* out);
+
 /* mmw_reset restricted to the n listed scenes (e.g. a sensor slot handed to a new sensor): their scene record, track
  * records, ring histograms, per-scene counters of the last step and pose-row count are cleared, so they continue like
- * fresh scenes (track ids restart at 0).  Other scenes, the sensor table, the accumulated counters and results already
- * packed for earlier frames are left alone.  Duplicate or out-of-range indices give MMW_ERR_INVALID and reset nothing. */
+ * fresh scenes (track ids restart at 0).  Other scenes, the sensor and tracker tables, the accumulated counters and
+ * results already packed for earlier frames are left alone.  Duplicate or out-of-range indices give MMW_ERR_INVALID
+ * and reset nothing. */
 int mmw_reset_scenes(mmw_ctx* ctx, const int32_t* scenes, int n);
 
 /* Checkpoint / resume of the tracker state of all scenes (track records, rings, keypoints, id counters): what a
  * replay needs to continue bit-identically in this or another context created with the same n_scenes,
  * max_points_per_frame, max_tracks and frames_batch (e.g. on another GPU).  mmw_state_size() = bytes of the blob;
  * dump / restore take a HOST buffer of at least that size and are synchronous.  The reference has no equivalent
- * (its state lives in Python objects for the length of the process); pose weights and the sensor table are not part
- * of the blob, and a blob of another ABI version is refused. */
+ * (its state lives in Python objects for the length of the process); pose weights and the sensor and tracker tables
+ * are not part of the blob, and a blob of another ABI version is refused. */
 size_t mmw_state_size(mmw_ctx* ctx);
 int mmw_state_dump(mmw_ctx* ctx, void* host_blob, size_t bytes);
 int mmw_state_restore(mmw_ctx* ctx, const void* host_blob, size_t bytes);
@@ -183,7 +233,12 @@ int mmw_state_restore(mmw_ctx* ctx, const void* host_blob, size_t bytes);
  * the slot they sit in.  Layout: this 64-byte header, the n source scene indices (int32, padded to 16 bytes), then n
  * records of record_bytes each, in list order.  The record's layout is private to the library and versioned by
  * MMW_ABI_VERSION.  Not carried: the outputs of the scene's last frame (point associations, labels, pose rows, packed
- * records), the accumulated counters, and the mmw_config (the tracker constants are the destination's). */
+ * records), the accumulated counters, the mmw_config and the scene's tracker-table entry (mmw_scene_tracker): an
+ * imported scene runs under its destination slot's entry.  To keep a tuned scene's tuning, copy its entry with
+ * mmw_get_scene_trackers on the source and mmw_set_scene_trackers on the destination slot, before or after the import.
+ * The ring histograms travel as they are, binned under the source's DBSCAN constants: to run a scene under other
+ * db_eps / db_z_weight / db_range_weight / db_min_samples than its source's, set the source's entry on the slot first
+ * and the new one after the import, so that the second change raises the histogram flags. */
 #define MMW_SCENE_BLOB_MAGIC 0x4d4d574du   /* "MMWM"; the state blob's is "MMWS" */
 typedef struct mmw_scene_blob_header {
     uint32_t magic;                /* MMW_SCENE_BLOB_MAGIC */

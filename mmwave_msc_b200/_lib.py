@@ -58,6 +58,30 @@ SCENE_SENSOR_DTYPE = np.dtype([
 assert SCENE_SENSOR_DTYPE.itemsize == C.sizeof(SceneSensor), (SCENE_SENSOR_DTYPE.itemsize, C.sizeof(SceneSensor))
 
 
+class SceneTracker(C.Structure):
+    """mmw_scene_tracker: one scene's tracker and DBSCAN constants (see include/mmw.h)."""
+    _fields_ = [
+        ("db_eps", C.c_double), ("db_z_weight", C.c_double), ("db_range_weight", C.c_double),
+        ("tr_lifetime_dynamic", C.c_double), ("tr_lifetime_static", C.c_double), ("tr_vel_thres", C.c_double),
+        ("tr_gate", C.c_double), ("kf_q_var", C.c_double), ("kf_p_init", C.c_double),
+        ("kf_group_disp_init", C.c_double), ("kf_a_n", C.c_double), ("kf_a_spr", C.c_double),
+        ("kf_spread_lim", C.c_double * 6), ("x_nudge_thres", C.c_double), ("x_nudge_gain", C.c_double),
+        ("db_min_samples", C.c_int32), ("tr_max_tracks", C.c_int32), ("kf_enable_est", C.c_int32),
+        ("kf_est_pointnum", C.c_int32),
+    ]
+
+
+SCENE_TRACKER_DTYPE = np.dtype([
+    ("db_eps", "<f8"), ("db_z_weight", "<f8"), ("db_range_weight", "<f8"),
+    ("tr_lifetime_dynamic", "<f8"), ("tr_lifetime_static", "<f8"), ("tr_vel_thres", "<f8"),
+    ("tr_gate", "<f8"), ("kf_q_var", "<f8"), ("kf_p_init", "<f8"),
+    ("kf_group_disp_init", "<f8"), ("kf_a_n", "<f8"), ("kf_a_spr", "<f8"),
+    ("kf_spread_lim", "<f8", (6,)), ("x_nudge_thres", "<f8"), ("x_nudge_gain", "<f8"),
+    ("db_min_samples", "<i4"), ("tr_max_tracks", "<i4"), ("kf_enable_est", "<i4"), ("kf_est_pointnum", "<i4"),
+], align=False)
+assert SCENE_TRACKER_DTYPE.itemsize == C.sizeof(SceneTracker), (SCENE_TRACKER_DTYPE.itemsize, C.sizeof(SceneTracker))
+
+
 SCENE_BLOB_MAGIC = 0x4D4D574D    # MMW_SCENE_BLOB_MAGIC
 
 
@@ -108,6 +132,8 @@ SIGNATURES = {
     "mmw_set_doppler_resolution": (C.c_int, [_p, C.c_double]),
     "mmw_set_scene_sensors": (C.c_int, [_p, C.c_int, C.c_int, _p]),
     "mmw_get_scene_sensors": (C.c_int, [_p, C.c_int, C.c_int, _p]),
+    "mmw_set_scene_trackers": (C.c_int, [_p, C.c_int, C.c_int, _p]),
+    "mmw_get_scene_trackers": (C.c_int, [_p, C.c_int, C.c_int, _p]),
     "mmw_reset_scenes": (C.c_int, [_p, _p, C.c_int]),
     "mmw_state_size": (C.c_size_t, [_p]),
     "mmw_state_dump": (C.c_int, [_p, _p, C.c_size_t]),

@@ -158,9 +158,40 @@ class BatchedTracker:
             table[name][idx] = v
         _lib.check(self.lib.mmw_set_scene_sensors(self._h, 0, self.S, _lib.ptr(table)))
 
+    # -- per-scene tracker constants -----------------------------------------------------------------
+    def scene_trackers(self) -> np.ndarray:
+        """Every scene's tracker and DBSCAN constants (mmw_scene_tracker): a (S,) structured array
+        (``_lib.SCENE_TRACKER_DTYPE``) with the fields of the same names as in mmw_config."""
+        out = np.zeros(self.S, _lib.SCENE_TRACKER_DTYPE)
+        _lib.check(self.lib.mmw_get_scene_trackers(self._h, 0, self.S, _lib.ptr(out)))
+        return out
+
+    def set_scene_trackers(self, scenes=None, **fields):
+        """Sets tracker and DBSCAN constants of the selected scenes (``scenes``: a slice or index array, default all),
+        by field name of ``_lib.SCENE_TRACKER_DTYPE`` (e.g. ``db_eps=0.45, tr_max_tracks=10``).  Each value is a scalar
+        or an array with one entry per selected scene (``kf_spread_lim``: (6,) or (n, 6)); None keeps the current
+        value.  Takes effect with the next step; live scenes keep their tracks.  All or nothing: invalid values change
+        no scene."""
+        idx = self._scene_index(scenes)
+        table = self.scene_trackers()
+        ints = ("db_min_samples", "tr_max_tracks", "kf_enable_est", "kf_est_pointnum")
+        for name, v in fields.items():
+            if name not in _lib.SCENE_TRACKER_DTYPE.names:
+                raise AttributeError("mmw_scene_tracker has no field %r" % name)
+            if v is None:
+                continue
+            v = np.asarray(v)
+            one = _lib.SCENE_TRACKER_DTYPE[name].shape              # () or (6,)
+            if v.shape not in (one, (idx.size,) + one):
+                raise ValueError("%s: give a value of shape %s or one per selected scene" % (name, one))
+            if name in ints and not np.array_equal(v, np.round(v)):
+                raise ValueError("%s must be an integer" % name)
+            table[name][idx] = v
+        _lib.check(self.lib.mmw_set_scene_trackers(self._h, 0, self.S, _lib.ptr(table)))
+
     def reset_scenes(self, scenes):
         """``reset`` restricted to the selected scenes (a slice or index array): their tracks, rings and id counters
-        start afresh; other scenes and the sensor table are left alone."""
+        start afresh; other scenes and the sensor and tracker tables are left alone."""
         idx = self._scene_index(scenes)
         _lib.check(self.lib.mmw_reset_scenes(self._h, _lib.ptr(idx), idx.size))
 

@@ -61,7 +61,7 @@ __device__ __forceinline__ int block_rank(bool flag, int* total, int* s_scan) {
 // Neighbour predicates ------------------------------------------------------------------------------------
 // Exact: float64 world coordinates in shared memory (stage-level entry point mmw_dbscan).
 struct NbExact {
-    const DevConfig& c;
+    const TrackerRec& c;
     const double *X, *Y, *Z;
     double eps;
     __device__ __forceinline__ bool operator()(int b, int q) const {
@@ -105,7 +105,7 @@ __device__ __forceinline__ float screen_domain_mark(float x, double yw, double z
     return fabs(yw) <= (double)rmax && fabs(zw) <= (double)rmax ? x : __int_as_float(0x7fc00000);
 }
 
-// Host side: guard band and domain radius for a configuration (mmw_create).  rmax = -1 (every pair exact): eps not
+// Host side: guard band and domain radius for a tracker-table entry (tracker_rec).  rmax = -1 (every pair exact): eps not
 // positive and finite, a negative or non-finite weight, or no radius at which the bound holds.
 inline void screen_config(double eps, double range_weight, double z_weight, float* lo, float* hi, float* rmax) {
     const float band = 1e-3f * (float)eps + 1e-4f;
@@ -127,7 +127,7 @@ inline void screen_config(double eps, double range_weight, double z_weight, floa
 }
 
 struct NbScreened {
-    const DevConfig& c;
+    const TrackerRec& c;              // the scene's tracker record (shared memory)
     const SensorRec& sr;              // the scene's mounting (shared memory)
     const float *Xf, *Yf, *Zf;        // shared memory, B floats each
     const float* frame[kRing];        // raw rows of the ring frames, oldest first (global)
@@ -178,7 +178,7 @@ struct NbScreened {
 // touched again.  The flag marks a frame with a point beyond ybound (or not finite): then the screen passes.
 constexpr int kGridDim = 16, kGridCells = kGridDim * kGridDim;
 
-// Host side: cell size and validity for a configuration (mmw_create).  ybound: 12 m covers every radar profile of
+// Host side: cell size and validity for a tracker-table entry (tracker_rec).  ybound: 12 m covers every radar profile of
 // the reference (config_cases/*.cfg: <= 8.5 m) and keeps w_min at 0.64 for the default range weight.
 inline void grid_screen_config(double eps, double range_weight, double z_weight, int min_samples, float* inv_h,
                                float* ybound, int* ok) {
@@ -194,7 +194,7 @@ inline void grid_screen_config(double eps, double range_weight, double z_weight,
     *ok = 1;
 }
 
-__device__ __forceinline__ int grid_cell(const DevConfig& c, float x, float yw) {
+__device__ __forceinline__ int grid_cell(const TrackerRec& c, float x, float yw) {
     const int kx = (int)floorf(x * c.grid_inv_h + 0.5f * kGridDim), ky = (int)floorf(yw * c.grid_inv_h);
     const int cx = kx < 0 ? 0 : (kx >= kGridDim ? kGridDim - 1 : kx);
     const int cy = ky < 0 ? 0 : (ky >= kGridDim ? kGridDim - 1 : ky);

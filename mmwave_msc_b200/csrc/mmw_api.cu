@@ -60,6 +60,10 @@ struct mmw_ctx {
     std::vector<mmw_scene_sensor> sensors;
     SensorRec* d_sensors = nullptr;
     double* d_doppler_wrap = nullptr; // [S] num_doppler_bins / 2 - 1 of each scene: the Doppler threshold of mmw_step_packets
+    // tracker table: each scene's tracker and DBSCAN constants as set (host) and as the kernels read them (device, [S])
+    std::vector<mmw_scene_tracker> trackers;
+    TrackerRec* d_trackers = nullptr;
+    int32_t* d_tracker_list = nullptr; // [S] scenes whose ring histograms mmw_set_scene_trackers flags (raise_hist_flags_kernel)
     // resident state
     TrackRec* d_tracks = nullptr;
     SceneRec* d_scenes = nullptr;
@@ -182,36 +186,80 @@ static mmw_scene_sensor config_sensor(const mmw_config& c) {
     return p;
 }
 
+// The kernels' form of one tracker-table entry, with the grid screen's cells and the fp32 screen's band and domain
+// derived for that entry.  Every entry, the context default included, is built here.
+static TrackerRec tracker_rec(const mmw_scene_tracker& p) {
+    TrackerRec d{};
+    d.db_z_weight = p.db_z_weight;
+    d.db_range_weight = p.db_range_weight;
+    d.db_eps = p.db_eps;
+    d.life_dyn = p.tr_lifetime_dynamic;
+    d.life_sta = p.tr_lifetime_static;
+    d.vel_thres = p.tr_vel_thres;
+    d.gate = p.tr_gate;
+    d.q_var = p.kf_q_var;
+    d.p_init = p.kf_p_init;
+    d.g_init = p.kf_group_disp_init;
+    d.a_n = p.kf_a_n;
+    d.a_spr = p.kf_a_spr;
+    for (int i = 0; i < 6; ++i) d.spread_lim[i] = p.kf_spread_lim[i];
+    d.nudge_thres = p.x_nudge_thres;
+    d.nudge_gain = p.x_nudge_gain;
+    d.db_min_samples = p.db_min_samples;
+    d.tr_max_tracks = p.tr_max_tracks;
+    d.enable_est = p.kf_enable_est;
+    d.est_pointnum = p.kf_est_pointnum;
+    grid_screen_config(p.db_eps, p.db_range_weight, p.db_z_weight, p.db_min_samples, &d.grid_inv_h, &d.grid_ybound,
+                       &d.grid_ok);
+    screen_config(p.db_eps, p.db_range_weight, p.db_z_weight, &d.screen_lo, &d.screen_hi, &d.screen_rmax);
+    return d;
+}
+
+// The tracker-table entry every scene starts with: the mmw_config's values.
+static mmw_scene_tracker config_tracker(const mmw_config& c) {
+    mmw_scene_tracker p{};
+    p.db_eps = c.db_eps;
+    p.db_z_weight = c.db_z_weight;
+    p.db_range_weight = c.db_range_weight;
+    p.tr_lifetime_dynamic = c.tr_lifetime_dynamic;
+    p.tr_lifetime_static = c.tr_lifetime_static;
+    p.tr_vel_thres = c.tr_vel_thres;
+    p.tr_gate = c.tr_gate;
+    p.kf_q_var = c.kf_q_var;
+    p.kf_p_init = c.kf_p_init;
+    p.kf_group_disp_init = c.kf_group_disp_init;
+    p.kf_a_n = c.kf_a_n;
+    p.kf_a_spr = c.kf_a_spr;
+    for (int i = 0; i < 6; ++i) p.kf_spread_lim[i] = c.kf_spread_lim[i];
+    p.x_nudge_thres = c.x_nudge_thres;
+    p.x_nudge_gain = c.x_nudge_gain;
+    p.db_min_samples = c.db_min_samples;
+    p.tr_max_tracks = c.tr_max_tracks;
+    p.kf_enable_est = c.kf_enable_est;
+    p.kf_est_pointnum = c.kf_est_pointnum;
+    return p;
+}
+
 static void fill_devconfig(const mmw_config& c, int ncap, int tcap, DevConfig* d) {
     d->sensor = sensor_rec(config_sensor(c));
-    d->db_z_weight = c.db_z_weight;
-    d->db_range_weight = c.db_range_weight;
-    d->db_eps = c.db_eps;
-    d->life_dyn = c.tr_lifetime_dynamic;
-    d->life_sta = c.tr_lifetime_static;
-    d->vel_thres = c.tr_vel_thres;
-    d->gate = c.tr_gate;
-    d->q_var = c.kf_q_var;
-    d->p_init = c.kf_p_init;
-    d->g_init = c.kf_group_disp_init;
-    d->a_n = c.kf_a_n;
-    d->a_spr = c.kf_a_spr;
-    for (int i = 0; i < 6; ++i) d->spread_lim[i] = c.kf_spread_lim[i];
+    d->tracker = tracker_rec(config_tracker(c));
     d->int_mu = c.intensity_mu;
     d->int_std = c.intensity_std;
-    d->nudge_thres = c.x_nudge_thres;
-    d->nudge_gain = c.x_nudge_gain;
-    d->db_min_samples = c.db_min_samples;
     d->ring_size = c.frames_batch + 1;
-    d->tr_max_tracks = c.tr_max_tracks;
-    d->enable_est = c.kf_enable_est;
-    d->est_pointnum = c.kf_est_pointnum;
     d->ncap = ncap;
     d->tcap = tcap;
-    grid_screen_config(c.db_eps, c.db_range_weight, c.db_z_weight, c.db_min_samples, &d->grid_inv_h, &d->grid_ybound,
-                       &d->grid_ok);
-    screen_config(c.db_eps, c.db_range_weight, c.db_z_weight, &d->screen_lo, &d->screen_hi, &d->screen_rmax);
 }
+
+namespace mmw {
+// Raises the flag word of every ring-frame histogram of the n listed scenes: the grid screen then passes for them until
+// those frames have left the ring (their counts were binned under cells the scene's DBSCAN constants no longer give).
+__global__ void raise_hist_flags_kernel(uint8_t* ring_hist, const int32_t* scenes, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n * kRing) return;
+    const size_t frame = (size_t)scenes[i / kRing] * kRing + i % kRing;
+    reinterpret_cast<uint32_t*>(ring_hist + frame * kHistBytes)[kGridCells / 4] = 1u;
+}
+}  // namespace mmw
 
 static const float kDefaultPosture[57] = {
     0.0000f, -0.0007f, -0.0006f, -0.0038f, -0.1820f, -0.2540f, -0.2579f, 0.1830f, 0.2957f, 0.2940f,
@@ -252,7 +300,7 @@ int mmw_destroy(mmw_ctx* x) {
     if (!x) return MMW_OK;
     cudaSetDevice(x->device);
     if (x->stream) cudaStreamSynchronize(x->stream);
-    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_export, x->d_export_valid, x->d_move, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
+    void* ptrs[] = {x->d_sensors, x->d_doppler_wrap, x->d_trackers, x->d_tracker_list, x->d_export, x->d_export_valid, x->d_move, x->d_tracks, x->d_scenes, x->d_track_ring, x->d_uring, x->d_keypoints, x->d_default_posture,
                     x->d_assoc, x->d_labels, x->d_counters, x->d_phase, x->d_defer, x->d_scene_stats, x->d_ring_hist,
                     x->d_results[0], x->d_results[1], x->d_blob, x->d_bn1s,
                     x->d_bn1t, x->d_bn2s, x->d_bn2t, x->d_feats, x->d_row_scene, x->d_row_track, x->d_row_slot,
@@ -474,6 +522,8 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
     ALLOC(x->d_pose_out, sizeof(float) * (size_t)x->pose_cap * kKp);
     ALLOC(x->d_sensors, sizeof(SensorRec) * S);
     ALLOC(x->d_doppler_wrap, sizeof(double) * S);
+    ALLOC(x->d_trackers, sizeof(TrackerRec) * S);
+    ALLOC(x->d_tracker_list, sizeof(int32_t) * S);
 #undef ALLOC
     cudaMemcpy(x->d_default_posture, cfg->default_posture, sizeof(float) * kKp, cudaMemcpyHostToDevice);
     x->sensors.assign(S, config_sensor(*cfg));
@@ -484,6 +534,14 @@ int mmw_create(const mmw_config* cfg, int device, int n_scenes, int max_points, 
             cudaMemcpy(x->d_doppler_wrap, wrap.data(), sizeof(double) * S, cudaMemcpyHostToDevice) != cudaSuccess) {
             mmw_destroy(x);
             return fail(MMW_ERR_CUDA, "upload of the sensor table failed");
+        }
+    }
+    x->trackers.assign(S, config_tracker(*cfg));
+    {
+        const std::vector<TrackerRec> recs(S, x->dc.tracker);
+        if (cudaMemcpy(x->d_trackers, recs.data(), sizeof(TrackerRec) * S, cudaMemcpyHostToDevice) != cudaSuccess) {
+            mmw_destroy(x);
+            return fail(MMW_ERR_CUDA, "upload of the tracker table failed");
         }
     }
     cudaMemset(x->d_keypoints, 0, sizeof(float) * S * max_tracks * kKp);
@@ -545,6 +603,62 @@ int mmw_get_scene_sensors(mmw_ctx* x, int first, int n, mmw_scene_sensor* out) {
     if (!x || !out) return fail(MMW_ERR_INVALID, "ctx/out is NULL");
     if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
     for (int i = 0; i < n; ++i) out[i] = x->sensors[first + i];
+    return MMW_OK;
+}
+
+// What is wrong with a tracker-table entry, or nullptr: the rules of mmw_set_scene_trackers, which are mmw_create's for
+// these fields.
+static const char* tracker_error(const mmw_scene_tracker& p) {
+    const double v[] = {p.db_eps, p.db_z_weight, p.db_range_weight, p.tr_lifetime_dynamic, p.tr_lifetime_static,
+                        p.tr_vel_thres, p.tr_gate, p.kf_q_var, p.kf_p_init, p.kf_group_disp_init, p.kf_a_n, p.kf_a_spr,
+                        p.kf_spread_lim[0], p.kf_spread_lim[1], p.kf_spread_lim[2], p.kf_spread_lim[3],
+                        p.kf_spread_lim[4], p.kf_spread_lim[5], p.x_nudge_thres, p.x_nudge_gain};
+    for (double d : v)
+        if (!std::isfinite(d)) return "tracker parameters must be finite";
+    if (p.db_min_samples < 1 || p.tr_max_tracks < 0) return "db_min_samples >= 1 and tr_max_tracks >= 0 required";
+    return nullptr;
+}
+
+// True when a and b bin the grid screen differently or judge its counts against another min_samples.
+static bool dbscan_fields_differ(const mmw_scene_tracker& a, const mmw_scene_tracker& b) {
+    return std::memcmp(&a.db_eps, &b.db_eps, sizeof(double)) != 0 ||
+           std::memcmp(&a.db_z_weight, &b.db_z_weight, sizeof(double)) != 0 ||
+           std::memcmp(&a.db_range_weight, &b.db_range_weight, sizeof(double)) != 0 || a.db_min_samples != b.db_min_samples;
+}
+
+// Queued on the context's stream behind all work queued there, as upload_sensors is: the records of scenes first ..
+// first + n - 1 in one copy, then the histogram flags of the scenes whose DBSCAN constants changed.  Nothing on the pose
+// stream reads the table (the feature kernel needs only the context-wide intensity normalisation and ring size), and
+// nothing on it touches the ring histograms.
+int mmw_set_scene_trackers(mmw_ctx* x, int first, int n, const mmw_scene_tracker* params) {
+    if (!x || !params) return fail(MMW_ERR_INVALID, "ctx/params is NULL");
+    if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
+    for (int i = 0; i < n; ++i)
+        if (const char* e = tracker_error(params[i])) return fail(MMW_ERR_INVALID, e);
+    if (n == 0) return MMW_OK;
+    std::vector<TrackerRec> recs(n);
+    std::vector<int32_t> flag;
+    for (int i = 0; i < n; ++i) {
+        recs[i] = tracker_rec(params[i]);
+        if (dbscan_fields_differ(x->trackers[first + i], params[i])) flag.push_back(first + i);
+    }
+    CK(cudaSetDevice(x->device));
+    CK(cudaMemcpyAsync(x->d_trackers + first, recs.data(), sizeof(TrackerRec) * n, cudaMemcpyHostToDevice, x->stream));
+    if (!flag.empty()) {
+        const int nf = (int)flag.size();
+        CK(cudaMemcpyAsync(x->d_tracker_list, flag.data(), sizeof(int32_t) * nf, cudaMemcpyHostToDevice, x->stream));
+        raise_hist_flags_kernel<<<(nf * kRing + 255) / 256, 256, 0, x->stream>>>(x->d_ring_hist, x->d_tracker_list, nf);
+        CK(cudaGetLastError());
+        x->launches++;
+    }
+    for (int i = 0; i < n; ++i) x->trackers[first + i] = params[i];
+    return MMW_OK;
+}
+
+int mmw_get_scene_trackers(mmw_ctx* x, int first, int n, mmw_scene_tracker* out) {
+    if (!x || !out) return fail(MMW_ERR_INVALID, "ctx/out is NULL");
+    if (first < 0 || n < 0 || n > x->S - first) return fail(MMW_ERR_INVALID, "scene range out of bounds");
+    for (int i = 0; i < n; ++i) out[i] = x->trackers[first + i];
     return MMW_OK;
 }
 
@@ -826,6 +940,7 @@ int mmw_step(mmw_ctx* x, const float* pts, const int32_t* offsets, const double*
 static int step_queue(mmw_ctx* x, StepArgs& a, uint32_t flags) {
     a.cfg = x->dc;
     a.sensors = x->d_sensors;
+    a.trackers = x->d_trackers;
     a.tracks = x->d_tracks; a.scenes = x->d_scenes; a.track_ring = x->d_track_ring; a.uring = x->d_uring;
     a.keypoints = x->d_keypoints; a.default_posture = x->d_default_posture; a.assoc_out = x->d_assoc;
     a.labels_out = (flags & MMW_STEP_RECORD_LABELS) ? x->d_labels : nullptr;
@@ -1108,7 +1223,7 @@ __global__ void __launch_bounds__(kStepThreads) dbscan_stage_kernel(DevConfig c,
         Z[b] = xyz[(size_t)(off + b) * 3 + 2];
     }
     __syncthreads();
-    dbscan_block(NbExact{c, X, Y, Z, eps}, B, min_samples, par, cl, scan);
+    dbscan_block(NbExact{c.tracker, X, Y, Z, eps}, B, min_samples, par, cl, scan);
     for (int b = threadIdx.x; b < B; b += blockDim.x) labels[off + b] = cl[b];
 }
 
@@ -2153,7 +2268,7 @@ int mmw_kalman_predict(mmw_ctx* x, double* hx, double* hP, const double* dt, int
     CK(cudaMemcpyAsync(dx, hx, (size_t)n * 9 * 8, cudaMemcpyHostToDevice, x->stream));
     CK(cudaMemcpyAsync(dP, hP, (size_t)n * 81 * 8, cudaMemcpyHostToDevice, x->stream));
     CK(cudaMemcpyAsync(ddt, dt, (size_t)n * 8, cudaMemcpyHostToDevice, x->stream));
-    kalman_predict_kernel<<<n, 128, 0, x->stream>>>(dx, dP, ddt, n, x->dc.q_var);
+    kalman_predict_kernel<<<n, 128, 0, x->stream>>>(dx, dP, ddt, n, x->dc.tracker.q_var);
     CK(cudaGetLastError());
     x->launches++;
     CK(cudaMemcpyAsync(hx, dx, (size_t)n * 9 * 8, cudaMemcpyDeviceToHost, x->stream));
@@ -2179,8 +2294,8 @@ int mmw_kalman_update(mmw_ctx* x, double* hx, double* hP, const double* z, const
     CK(cudaMemcpyAsync(dz, z, (size_t)n * 6 * 8, cudaMemcpyHostToDevice, x->stream));
     CK(cudaMemcpyAsync(dR, R, (size_t)n * 36 * 8, cudaMemcpyHostToDevice, x->stream));
     CK(cudaMemcpyAsync(dl, life0, (size_t)n, cudaMemcpyHostToDevice, x->stream));
-    kalman_update_kernel<<<n, 128, 0, x->stream>>>(dx, dP, dz, dR, dl, n, x->dc.nudge_thres,
-                                                             x->dc.nudge_gain);
+    kalman_update_kernel<<<n, 128, 0, x->stream>>>(dx, dP, dz, dR, dl, n, x->dc.tracker.nudge_thres,
+                                                             x->dc.tracker.nudge_gain);
     CK(cudaGetLastError());
     x->launches++;
     CK(cudaMemcpyAsync(hx, dx, (size_t)n * 9 * 8, cudaMemcpyDeviceToHost, x->stream));
@@ -2210,7 +2325,7 @@ int mmw_gate(mmw_ctx* x, const double* points, int M, const double* hxv, const d
     }
     const size_t smem = ((size_t)(T ? T : 1) * (kGateWords + 36)) * 8;
     CK(cudaFuncSetAttribute(gate_stage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gate_stage_kernel<<<1, 128, smem, x->stream>>>(dp, M, dh, dC, T, x->dc.gate, dd, da);
+    gate_stage_kernel<<<1, 128, smem, x->stream>>>(dp, M, dh, dC, T, x->dc.tracker.gate, dd, da);
     CK(cudaGetLastError());
     x->launches++;
     if (T) CK(cudaMemcpyAsync(d2, dd, (size_t)M * T * 8, cudaMemcpyDeviceToHost, x->stream));

@@ -36,23 +36,33 @@ __device__ __forceinline__ SensorRec sensor_at_use(const SensorRec& r) {
     return o;
 }
 
-// Derived constants handed to kernels by value.
-struct DevConfig {
-    SensorRec sensor;          // the mmw_config's mounting: the stateless stage entry points use it
+// One scene's tracker and DBSCAN constants (mmw_scene_tracker) as the kernels use it, with what is derived from them
+// per entry on the host: one record per scene in HBM (mmw_ctx::d_trackers), read by step_kernel and dbscan_big_kernel.
+struct TrackerRec {
     double db_z_weight, db_range_weight, db_eps;
     double life_dyn, life_sta, vel_thres, gate;
     double q_var, p_init, g_init, a_n, a_spr;
     double spread_lim[6];
-    double int_mu, int_std, nudge_thres, nudge_gain;
-    int db_min_samples, ring_size, tr_max_tracks, enable_est, est_pointnum;
-    int ncap, tcap;
+    double nudge_thres, nudge_gain;
+    int32_t db_min_samples, tr_max_tracks, enable_est, est_pointnum;
     // grid screen in front of DBSCAN (dbscan.cuh): fixed 16 x 16 cells over world (x, y'), at least one eps reach wide
     // for every pair of points with y' <= grid_ybound; grid_ok = 0: degenerate configuration, the screen always passes
     float grid_inv_h, grid_ybound;
-    int grid_ok;
+    int32_t grid_ok;
     // fp32 screen of the eps predicate (dbscan.cuh, screen_d): guard band [lo, hi] around eps, and the domain |y'|, |z'|
     // <= rmax in which the band covers the fp32 error (rmax = -1: every pair is decided in float64)
     float screen_lo, screen_hi, screen_rmax;
+    int32_t pad[2];
+};
+static_assert(sizeof(TrackerRec) == 208, "TrackerRec is thirteen 16-byte chunks (moved with one bulk copy)");
+
+// Derived constants handed to kernels by value.
+struct DevConfig {
+    SensorRec sensor;          // the mmw_config's mounting: the stateless stage entry points use it
+    TrackerRec tracker;        // the mmw_config's tracker constants: the stateless stage entry points use them
+    double int_mu, int_std;
+    int ring_size;
+    int ncap, tcap;
 };
 
 // One element of a scene's effective_tracks list (ClusterTrack + KalmanState + PointCluster).
@@ -100,6 +110,7 @@ static_assert(sizeof(SceneRec) == 64, "SceneRec is one 64-byte record");
 struct StepArgs {
     DevConfig cfg;
     const SensorRec* sensors;  // [S] each scene's mounting and radar profile
+    const TrackerRec* trackers;  // [S] each scene's tracker and DBSCAN constants
     const float* pts;          // [sum N, 5] fp32 rows; int16 rows when flags has MMW_STEP_INPUT_I16
     const int32_t* offsets;    // [S+1]
     const double* dt;          // [S]
@@ -255,7 +266,7 @@ __device__ __forceinline__ void write_fade_square(const FadeCfg& fade, double x0
 }
 
 // altered_EuclideanDist(p, q) <= eps (Utils.py:242-247, compared as sklearn's radius query does)
-__device__ __forceinline__ bool eps_neighbour(const DevConfig& c, double x1, double y1, double z1, double x2,
+__device__ __forceinline__ bool eps_neighbour(const TrackerRec& c, double x1, double y1, double z1, double x2,
                                               double y2, double z2, double eps) {
     const double w = __dsub_rn(1.0, __dmul_rn(__dmul_rn(__dadd_rn(y1, y2), 0.5), c.db_range_weight));
     const double dx = __dsub_rn(x1, x2), dy = __dsub_rn(y1, y2), dz = __dsub_rn(z1, z2);

@@ -7,9 +7,10 @@
 // ring rows written and three 272-byte cell histograms for the screen.
 //
 // How the work is laid out (round 2; profiles/r02_*.md):
-//   * inputs arrive by four bulk copies (cp.async.bulk, 1-D TMA) behind one mbarrier: the scene's contiguous block
-//     of raw points (as the 16-byte aligned window around it), its track records, the ring's cell histograms and the
-//     scene's sensor record (mounting, Doppler unit, Q format; read from shared memory where it is used);
+//   * inputs arrive by five bulk copies (cp.async.bulk, 1-D TMA) behind one mbarrier: the scene's contiguous block
+//     of raw points (as the 16-byte aligned window around it), its track records, the ring's cell histograms, the
+//     scene's sensor record (mounting, Doppler unit, Q format) and its tracker record (tracker and DBSCAN constants,
+//     grid-screen cells); both records are read from shared memory where they are used;
 //   * point phases are thread-per-point, two points per thread per tile of 256, both in flight at once (straight-
 //     line code, two independent float64 chains) -- transform, filter, gate, list positions, ring pushes all work
 //     from registers;
@@ -41,6 +42,7 @@ static_assert(kStepThreads == 128, "the element-parallel track phases are writte
 
 // Dynamic shared memory of step_kernel.
 //   sensor  the scene's SensorRec (48 bytes; first, so that its address is a constant)
+//   tracker the scene's TrackerRec (208 bytes; right behind, at a constant address too)
 //   tracks  TrackRec [tcap]
 //   B       double [tcap][72]   gate..association: see above;  update: S -> S^-1 (0..35) | Rc (36..71)
 //   A       double [tcap][81]   F P (predict), C (gate matrix, first 36), (I - K H) P (update)
@@ -50,7 +52,7 @@ static_assert(kStepThreads == 128, "the element-parallel track phases are writte
 //   and the update; the staged raw points lie over KK when a frame is a single tile, in their own space otherwise
 //   (they must survive the tile loop).
 struct SmemLayout {
-    int sensor, tracks, B, A, KK, stage, hist, hnew, misc, total;
+    int sensor, tracker, tracks, B, A, KK, stage, hist, hnew, misc, total;
 };
 constexpr int kMiscInts = 192;
 // misc int slots (slot 0-1: the mbarrier)
@@ -62,6 +64,7 @@ __host__ __device__ inline SmemLayout make_layout(int ncap, int tcap) {
     SmemLayout L;
     int o = 0;
     L.sensor = o;  o += (int)sizeof(SensorRec);
+    L.tracker = o; o += (int)sizeof(TrackerRec);
     L.tracks = o;  o += tcap * (int)sizeof(TrackRec);
     L.B = o;       o += tcap * kBw * 8;
     L.A = o;
@@ -140,16 +143,23 @@ __device__ __forceinline__ const float* uring_frame(const StepArgs& a, int s, in
     return a.uring + ((size_t)s * kRing + phys) * (size_t)a.cfg.ncap * kRawCols;
 }
 
+// _estimate_point_num (Tracking.py:232-244) for a track that got n points.  With KF_ENABLE_EST the smoothing is rounded
+// like numpy's, product by product: contracted into a fused multiply-add it missed the reference's N_est in the last bit.
+__device__ __forceinline__ double n_est_next(const TrackerRec& c, double n_est, int n) {
+    const double dn = (double)n;
+    if (!c.enable_est) return (double)(n > c.est_pointnum ? n : c.est_pointnum);
+    return dn > n_est ? dn : __dadd_rn(__dmul_rn(__dsub_rn(1.0, c.a_n), n_est), __dmul_rn(c.a_n, dn));
+}
+
 // One warp turns DBSCAN cluster q of the fused ring into a fresh track (ClusterTrack.__init__, Tracking.py:210-230
 // over PointCluster(cluster), :120-136): statistics over the 6 world columns recomputed from the ring's raw rows,
 // state x = [centroid, 0, 0, 0], P = KF_P_INIT*I, group dispersion = KF_GROUP_DISP_EST_INIT*I, ring = [first 64
 // cluster rows in fused order], keypoints = MODEL_DEFAULT_POSTURE.  `t` may live in shared or global memory.
-__device__ __forceinline__ void spawn_track(const StepArgs& a, const SensorRec& sr, int s, TrackRec& t, int q, int slot,
-                                            int track_id, const int* cl, const int* fcnt, const int* fphys, int lane,
-                                            const float* rawc = nullptr /* fused raw rows in shared memory */,
+__device__ __forceinline__ void spawn_track(const StepArgs& a, const SensorRec& sr, const TrackerRec& c, int s, TrackRec& t,
+                                            int q, int slot, int track_id, const int* cl, const int* fcnt, const int* fphys,
+                                            int lane, const float* rawc = nullptr /* fused raw rows in shared memory */,
                                             const double* w6 = nullptr /* their world 6-vectors, precomputed */) {
-    const DevConfig& c = a.cfg;
-    const int tcap = c.tcap;
+    const int tcap = a.cfg.tcap;
     int n = 0;
     double sacc[6], mn[6], mx[6];
 #pragma unroll
@@ -232,10 +242,10 @@ __device__ __forceinline__ void spawn_track(const StepArgs& a, const SensorRec& 
 // maxima are reduced per warp by shuffles and across warps in warp order (fixed order: deterministic), the first 64
 // cluster rows in fused order get their ring positions from per-chunk ballot counts, and the record's fields are
 // written by different threads at once.  `red` is shared scratch of at least 16 * 20 + 32 + 20 doubles.
-__device__ __forceinline__ void spawn_track_block(const StepArgs& a, int s, TrackRec& t, int q, int slot, int track_id,
-                                                  const int* cl, int B, const float* rawc, const double* w6, double* red) {
-    const DevConfig& c = a.cfg;
-    const int tcap = c.tcap, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
+__device__ __forceinline__ void spawn_track_block(const StepArgs& a, const TrackerRec& c, int s, TrackRec& t, int q, int slot,
+                                                  int track_id, const int* cl, int B, const float* rawc, const double* w6,
+                                                  double* red) {
+    const int tcap = a.cfg.tcap, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
     const unsigned ltmask = (1u << lane) - 1u;
     double* wred = red;                                   // [nwarps][20]: n, sums (6), minima (6), maxima (6)
     int* ccnt = reinterpret_cast<int*>(red + nwarps * 20);   // [<= 32] in-cluster points per chunk of 32
@@ -331,9 +341,9 @@ __device__ __forceinline__ void spawn_track_block(const StepArgs& a, int s, Trac
 
 // fp32 world coordinates of the fused ring (oldest frame first) into shared memory + the screened predicate over
 // them (dbscan.cuh).  Block-cooperative; ends with __syncthreads().
-__device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, const SensorRec& sr, int s, const int* fcnt,
-                                                      const int* fphys, float* Xf, int stride, float* rawc = nullptr) {
-    const DevConfig& c = a.cfg;
+__device__ __forceinline__ NbScreened load_fused_ring(const StepArgs& a, const SensorRec& sr, const TrackerRec& c, int s,
+                                                      const int* fcnt, const int* fphys, float* Xf, int stride,
+                                                      float* rawc = nullptr) {
     float* Yf = Xf + stride;
     float* Zf = Yf + stride;
     NbScreened nb{c, sr, Xf, Yf, Zf, {nullptr, nullptr, nullptr}, {0, 0, 0, 0}, c.db_eps, c.screen_lo, c.screen_hi,
@@ -388,8 +398,8 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
         a.phase_cycles[16 + gridDim.x + blockIdx.x] = ns;
     }
     extern __shared__ __align__(16) unsigned char smem[];
-    const DevConfig& c = a.cfg;
-    const int ncap = c.ncap, tcap = c.tcap;
+    const DevConfig& cfg = a.cfg;
+    const int ncap = cfg.ncap, tcap = cfg.tcap;
     const SmemLayout L = make_layout(ncap, tcap);
     TrackRec* tr = reinterpret_cast<TrackRec*>(smem + L.tracks);
     double* Bm = reinterpret_cast<double*>(smem + L.B);
@@ -402,6 +412,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     uint8_t* cntG = reinterpret_cast<uint8_t*>(misc + kCntG);   // [kChunks][32] points per chunk and track
     uint64_t* mbar = reinterpret_cast<uint64_t*>(smem + L.misc);
     const SensorRec& sr = *reinterpret_cast<const SensorRec*>(smem);   // this scene's mounting (L.sensor = 0)
+    const TrackerRec& c = *reinterpret_cast<const TrackerRec*>(smem + sizeof(SensorRec));   // its constants (L.tracker)
 
     const int s = blockIdx.x;
     if (s >= a.n_scenes) return;
@@ -410,7 +421,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     const Elem el(tid);
     const unsigned ltmask = (1u << lane) - 1u;
 
-    // ---- 0. round trip one: scene record, offsets, dt; then the four bulk copies -----------------------------
+    // ---- 0. round trip one: scene record, offsets, dt; then the five bulk copies -----------------------------
     if (tid == 0) sk_mbar_init(mbar, 1);
     SceneRec sc = a.scenes[s];           // every thread keeps a copy; thread 0 writes it back
     const int off = a.offsets[s];
@@ -431,12 +442,14 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     const int16_t* stageh = reinterpret_cast<const int16_t*>(stageb);
     if (tid == 0) {
         const uint32_t tr_bytes = (uint32_t)T0 * (uint32_t)sizeof(TrackRec);
-        sk_mbar_expect_tx(mbar, tr_bytes + (bulk_pts ? win_bytes : 0u) + (uint32_t)(kRing * kHistBytes + sizeof(SensorRec)));
+        sk_mbar_expect_tx(mbar, tr_bytes + (bulk_pts ? win_bytes : 0u) +
+                                    (uint32_t)(kRing * kHistBytes + sizeof(SensorRec) + sizeof(TrackerRec)));
         if (tr_bytes) sk_bulk_g2s(tr, a.tracks + (size_t)s * tcap, tr_bytes, mbar);
         if (bulk_pts && win_bytes)
             sk_bulk_g2s(smem + L.stage, reinterpret_cast<const unsigned char*>(a.pts) + win0, win_bytes, mbar);
         sk_bulk_g2s(hist, a.ring_hist + (size_t)s * (kRing * kHistBytes), kRing * kHistBytes, mbar);
         sk_bulk_g2s(smem + L.sensor, a.sensors + s, (uint32_t)sizeof(SensorRec), mbar);
+        sk_bulk_g2s(smem + L.tracker, a.trackers + s, (uint32_t)sizeof(TrackerRec), mbar);
     }
     if (!bulk_pts) {
         if (i16) {
@@ -499,7 +512,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
 
     // ---- 2. tiles of 256 points: transform + filter + compaction (Utils.py:379-432), gating + association
     //         (Tracking.py:553-572, Q14), list positions, ring pushes (Tracking.py:691, 338), statistics ------------
-    const int uphys = sc.ring_n >= c.ring_size ? sc.ring_head : ring_wrap(sc.ring_head + sc.ring_n, c.ring_size);
+    const int uphys = sc.ring_n >= cfg.ring_size ? sc.ring_head : ring_wrap(sc.ring_head + sc.ring_n, cfg.ring_size);
     float* udst = const_cast<float*>(uring_frame(a, s, uphys));
     int M = 0;
     const int ntiles = (N + kTile - 1) / kTile;
@@ -633,7 +646,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
                 if (lp < kFeatPts) {
                     // first 64 associated rows in input order are what format_single_frame can see
                     const TrackRec& t = tr[g];
-                    const int phys = t.ring_n >= c.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, c.ring_size);
+                    const int phys = t.ring_n >= cfg.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, cfg.ring_size);
                     float* dst = a.track_ring + (((size_t)s * tcap + t.slot) * kRing + phys) * (kFeatPts * kRawCols) +
                                  (size_t)lp * kRawCols;
 #pragma unroll
@@ -751,9 +764,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
         const double dn = (double)n;
         double v0 = 0.0, v1 = 0.0, v2 = 0.0, v3 = 0.0;
         if (tid < 36) {
-            double n_est;
-            if (c.enable_est) n_est = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
-            else n_est = (double)(n > c.est_pointnum ? n : c.est_pointnum);
+            const double n_est = n_est_next(c, t.n_est, n);
             int r = el.i6, q = el.a6;
             if (r > q) { const int tmp = r; r = q; q = tmp; }
             const int p = r * 6 - (r * (r - 1)) / 2 + (q - r);
@@ -775,8 +786,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
             spread = fmax(c.spread_lim[m], spread);
             v3 = spread > t.spread[m] ? spread : (1.0 - c.a_spr) * t.spread[m] + c.a_spr * spread;
         } else if (tid == 96) {
-            if (c.enable_est) v0 = dn > t.n_est ? dn : (1 - c.a_n) * t.n_est + c.a_n * dn;
-            else v0 = (double)(n > c.est_pointnum ? n : c.est_pointnum);
+            v0 = n_est_next(c, t.n_est, n);
             const double c3 = tv[kHx + 3] + tv[kSum + 3] / dn, c4 = tv[kHx + 4] + tv[kSum + 4] / dn,
                          c5 = tv[kHx + 5] + tv[kSum + 5] / dn;
             v1 = sqrt(c3 * c3 + c4 * c4 + c5 * c5) < c.vel_thres ? 1.0 : 0.0;
@@ -787,8 +797,8 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
             const int m = tid - 64;
             t.centroid[m] = v0; t.minv[m] = v1; t.maxv[m] = v2; t.spread[m] = v3;
         } else if (tid == 96) {
-            const int phys = t.ring_n >= c.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, c.ring_size);
-            if (t.ring_n >= c.ring_size) t.ring_head = ring_wrap(t.ring_head + 1, c.ring_size);
+            const int phys = t.ring_n >= cfg.ring_size ? t.ring_head : ring_wrap(t.ring_head + t.ring_n, cfg.ring_size);
+            if (t.ring_n >= cfg.ring_size) t.ring_head = ring_wrap(t.ring_head + 1, cfg.ring_size);
             else t.ring_n += 1;
             t.ring_cnt[phys] = n < kFeatPts ? n : kFeatPts;
             t.lifetime = 0.0;
@@ -798,8 +808,8 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
         }
     }
     {
-        if (!sc.ring_ph_gone && sc.ring_n + 1 >= c.ring_size) sc.ring_ph_gone = 1;   // the deque's initial empty frame
-        if (sc.ring_n >= c.ring_size) sc.ring_head = ring_wrap(sc.ring_head + 1, c.ring_size);
+        if (!sc.ring_ph_gone && sc.ring_n + 1 >= cfg.ring_size) sc.ring_ph_gone = 1;   // the deque's initial empty frame
+        if (sc.ring_n >= cfg.ring_size) sc.ring_head = ring_wrap(sc.ring_head + 1, cfg.ring_size);
         else sc.ring_n += 1;
         sc.ring_cnt[uphys] = U;
     }
@@ -905,7 +915,7 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinBlocks) step_kernel(cons
     int fphys[kRing];
     bool fl = false;
     for (int f = 0; f < kRing; ++f) {
-        fphys[f] = ring_wrap(sc.ring_head + f, c.ring_size);
+        fphys[f] = ring_wrap(sc.ring_head + f, cfg.ring_size);
         if (f < sc.ring_n) {
             Bf += sc.ring_cnt[fphys[f]];
             fl = fl || hist[fphys[f] * kHistBytes + kGridCells] != 0;
@@ -980,8 +990,8 @@ __host__ __device__ inline int big_w6_offset(int ncap) {
 }
 __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid_constant__ StepArgs a) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const DevConfig& c = a.cfg;
-    const int ncap = c.ncap, tcap = c.tcap;
+    const DevConfig& cfg = a.cfg;
+    const int ncap = cfg.ncap, tcap = cfg.tcap;
     float* Xf = reinterpret_cast<float*>(smem);
     int* par = reinterpret_cast<int*>(smem + 36 * ncap);
     int* cl = par + 3 * ncap;
@@ -1009,22 +1019,27 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
         }
     };
     __shared__ SensorRec s_sr;            // the scene's mounting
+    __shared__ TrackerRec s_tk;           // and its tracker constants
+    const TrackerRec& c = s_tk;
     for (int it = blockIdx.x; it < n_defer; it += gridDim.x) {
         const int s = a.defer_list[it];
         SceneRec sc = a.scenes[s];
         if (tid < (int)(sizeof(SensorRec) / 8))
             reinterpret_cast<double*>(&s_sr)[tid] = reinterpret_cast<const double*>(a.sensors + s)[tid];
+        else if (tid < (int)((sizeof(SensorRec) + sizeof(TrackerRec)) / 8))
+            reinterpret_cast<double*>(&s_tk)[tid - sizeof(SensorRec) / 8] =
+                reinterpret_cast<const double*>(a.trackers + s)[tid - sizeof(SensorRec) / 8];
         __syncthreads();
         const int T1 = sc.n_tracks;
         int B = 0;
         int fcnt[kRing], fphys[kRing];
         for (int f = 0; f < kRing; ++f) {
-            fphys[f] = ring_wrap(sc.ring_head + f, c.ring_size);
+            fphys[f] = ring_wrap(sc.ring_head + f, cfg.ring_size);
             fcnt[f] = f < sc.ring_n ? sc.ring_cnt[fphys[f]] : 0;
             B += fcnt[f];
         }
         const bool bits = B <= bits_cap;
-        NbScreened nb = load_fused_ring(a, s_sr, s, fcnt, fphys, Xf, 3 * ncap, bits ? rawc : nullptr);
+        NbScreened nb = load_fused_ring(a, s_sr, c, s, fcnt, fphys, Xf, 3 * ncap, bits ? rawc : nullptr);
         stamp(0);
         int ncl = bits ? dbscan_bits_block(nb, B, c.db_min_samples, adj, cm, bws, par, cl, dbg != nullptr ? dbg - 10 : nullptr)
                        : dbscan_block(nb, B, c.db_min_samples, par, cl, scan, dbg != nullptr ? dbg - 10 : nullptr, false,
@@ -1058,11 +1073,11 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                 // the adjacency matrix is dead by now: its first bytes serve as the reduction scratch
                 double* red = reinterpret_cast<double*>(adj);
                 for (int q = 0; q < ncl; ++q)
-                    spawn_track_block(a, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, B, rawc,
+                    spawn_track_block(a, c, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, B, rawc,
                                       w6, red);
             } else {
                 for (int q = warp; q < ncl; q += kBigThreads / 32)
-                    spawn_track(a, s_sr, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, fcnt,
+                    spawn_track(a, s_sr, c, s, a.tracks[(size_t)s * tcap + T1 + q], q, newslot[q], sc.next_id + q, cl, fcnt,
                                 fphys, lane, nullptr, nullptr);
             }
             if (a.nr_extra != nullptr) {
@@ -1081,7 +1096,7 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                     s_row0 = r0 + atomicAdd(a.nr_extra, ncl);
                 }
                 __syncthreads();
-                const int nfr = c.ring_size;
+                const int nfr = cfg.ring_size;
                 unsigned char* scratch = smem + ((big_adj_offset(ncap) + 15) & ~15) + warp * kFeatItemBytes;
                 long long* fkeys = reinterpret_cast<long long*>(scratch);
                 float* fso = reinterpret_cast<float*>(scratch + kFeatPts * 8);
@@ -1099,7 +1114,7 @@ __global__ void __launch_bounds__(kBigThreads, 1) dbscan_big_kernel(const __grid
                     uint4* pk = a.nr_packed != nullptr
                                     ? reinterpret_cast<uint4*>(static_cast<unsigned char*>(a.nr_packed) + (size_t)row * nfr * kFeatPts * 32)
                                     : nullptr;
-                    pose_feature_item<false>(c, s_sr, src, cnt, __ldcg(&t->centroid[0]), __ldcg(&t->centroid[1]), f, out, pk,
+                    pose_feature_item<false>(cfg, s_sr, src, cnt, __ldcg(&t->centroid[0]), __ldcg(&t->centroid[1]), f, out, pk,
                                              fkeys, fso, fsp, lane, 0);
                 }
             }
